@@ -10,7 +10,7 @@ One STEP = one pass of the post-backbone hot path over one batch of 16 synthetic
 Every rank of an N-GPU run processes its own batch of 16 images (images are independent: weak scaling,
 no data-path collective).  `value` = ROIs pooled by all ranks / max-over-ranks step time.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 """
 import argparse
 import json
@@ -102,6 +102,44 @@ def to_torch(host, dev=None, pin=False):
             return t.pin_memory() if pin else t
         out[k] = [conv(a) for a in v] if isinstance(v, list) else conv(v)
     return out
+
+
+# ROI feature rows written by --dump-outputs: 512 of 16,000 box rows (50 KB each) and 128 of 1,600 mask rows
+# (200 KB each) keep the files at about 52 MB in all
+DUMP_ROWS = {"box_feats": 512, "mask_feats": 128}
+
+
+def dump_rows(name, n):
+    """The rows of output `name` (of n rows) that --dump-outputs writes: all of them, or the same seeded sample."""
+    if name not in DUMP_ROWS:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS[name], replace=False))
+
+
+def dump_outputs(path, outs):
+    """Write what one step returned -- a list of per-image-block output dicts (torch tensors of a graphed step, or
+    numpy arrays of the CPU arm), concatenated in image order -- as `path`/<name>.npy: float64 for 8-byte types,
+    float32 otherwise.  The pooled ROI features are written as the same seeded sample of rows on every run, taken
+    block by block, so that two builds can be compared output for output."""
+    import torch
+    os.makedirs(path, exist_ok=True)
+    for k in outs[0]:
+        rows = dump_rows(k, sum(o[k].shape[0] for o in outs))
+        parts, b = [], 0
+        for o in outs:
+            x, n = o[k], o[k].shape[0]
+            sel = rows[(rows >= b) & (rows < b + n)] - b
+            parts.append(x[torch.from_numpy(sel).to(x.device)].cpu().numpy() if isinstance(x, torch.Tensor) else x[sel])
+            b += n
+        a = np.concatenate(parts)
+        np.save(os.path.join(path, k + ".npy"), a.astype(np.float64 if a.dtype.itemsize == 8 else np.float32))
+
+
+def oracle_outputs(o):
+    """cpu_step's result under the output names of the graphed step (MaskRCNNPostBackbone.flatten_outputs)."""
+    (pb, pl, pv), (db, ds, dc, dv) = o["proposals"], o["dets"]
+    return {"proposal_boxes": pb, "proposal_logits": pl, "proposal_valid": pv, "box_feats": o["box_feats"],
+            "det_boxes": db, "det_scores": ds, "det_classes": dc, "det_valid": dv, "mask_feats": o["mask_feats"]}
 
 
 def nbytes(obj):
@@ -221,7 +259,7 @@ def cpu_step(host, n_images, stage_s=None):
 
 def time_cpu(host, n_images, steps, warmup, threads=None):
     """Returns dict: ROIs/s (from the median step), seconds per step (median, mean), threads, per-stage seconds per
-    step, NMS boxes entering per step."""
+    step, NMS boxes entering per step, the outputs of the last step."""
     import oracle
     oracle.build()
     # all the host threads this process may use -- explicitly, because torchrun exports OMP_NUM_THREADS=1
@@ -231,7 +269,7 @@ def time_cpu(host, n_images, steps, warmup, threads=None):
     stage = [0.0, 0.0, 0.0, 0.0]
     for i in range(warmup + steps):
         t0 = time.perf_counter()
-        cpu_step(host, n_images, stage if i >= warmup else None)
+        out = cpu_step(host, n_images, stage if i >= warmup else None)
         dt = time.perf_counter() - t0
         if i >= warmup:
             ts.append(dt)
@@ -241,14 +279,15 @@ def time_cpu(host, n_images, steps, warmup, threads=None):
         int((host["scores"][:n_images * ROIS_PER_IMAGE, :-1] > SCORE_THR).sum())
     med = float(np.median(ts))
     r = {"rois_per_s": rois / med, "sec_median": med, "sec_mean": float(np.mean(ts)), "threads": oracle.max_threads(),
-         "stage_sec": [x / steps for x in stage], "nms_in": nms_in, "rois": rois}
+         "stage_sec": [x / steps for x in stage], "nms_in": nms_in, "rois": rois, "outputs": out}
     oracle.set_num_threads(avail)
     return r
 
 
 def cpu_baseline_dict(host, n_images, steps, warmup, sample, one_thread_images=2):
     """The CPU oracle (port of the reference's TF-CPU path) on `n_images` of the workload with every host thread
-    (median of `steps` after `warmup`), plus a 1-thread leg on a smaller sample (BASELINE.md section 3)."""
+    (median of `steps` after `warmup`), plus a 1-thread leg on a smaller sample (BASELINE.md section 3).
+    Returns the cpu_baseline object and time_cpu's result for all threads."""
     r = time_cpu(host, n_images, steps, warmup)
     st = r["stage_sec"]
     cb = {"value": r["rois_per_s"], "unit": "ROIs/s", "cores": r["threads"], "kind": "port", "sample": sample,
@@ -268,7 +307,7 @@ def cpu_baseline_dict(host, n_images, steps, warmup, sample, one_thread_images=2
                             "ms_per_image": r1["sec_median"] * 1e3 / k,
                             "roi_align_rois_per_s": r1["rois"] / (s1[1] + s1[3]),
                             "nms_boxes_per_s": r1["nms_in"] / (s1[0] + s1[2])}
-    return cb, r["rois_per_s"], r["sec_median"]
+    return cb, r
 
 
 def run_reference(args):
@@ -279,9 +318,12 @@ def run_reference(args):
         return
     n_img = IMAGES_PER_RANK
     host = make_host_inputs(n_img)
-    steps, warmup = max(min(args.steps, 150), 1), max(args.warmup, 3)  # ~0.7 s of CPU per step
-    cb, v, sec = cpu_baseline_dict(host, n_img, steps, warmup,
-                                   f"{n_img} of {n_img} images per step, median of {steps} steps after {warmup} warm-ups")
+    steps, warmup = args.steps, max(args.warmup, 3)  # ~0.7 s of CPU per step
+    cb, r = cpu_baseline_dict(host, n_img, steps, warmup,
+                              f"{n_img} of {n_img} images per step, median of {steps} steps after {warmup} warm-ups")
+    v, sec = r["rois_per_s"], r["sec_median"]
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, [oracle_outputs(r["outputs"])])
     line = {
         "impl": "reference", "metric": METRIC, "value": v, "unit": "ROIs/s", "n_gpus": args.gpus, "steps": steps,
         "warmup": warmup, "ms_per_step": sec * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
@@ -432,13 +474,15 @@ def run_gpu(args):
     barrier()
     t0 = time.perf_counter()
     e0.record()
-    pipe.run(K)
+    last = pipe.run(K)
     e1.record()
     barrier()
     wall = time.perf_counter() - t0
     launches = gstep.kernels_per_replay * K
     clocks = sampler.summary()
     dev_ms = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
     if world > 1:
         t = torch.tensor([dev_ms, wall * 1e3, eager_ms, step_latency_ms], device=dev, dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -578,7 +622,7 @@ def run_gpu(args):
 
     # ---- CPU baseline beside it (rank 0, N=1 only): bounded sample of the same workload
     if world == 1 and not args.no_cpu:
-        cb, _, _ = cpu_baseline_dict(host, n, 10, 2, f"{n} of {n} images per step, median of 10 steps after 2 warm-ups")
+        cb, _ = cpu_baseline_dict(host, n, 10, 2, f"{n} of {n} images per step, median of 10 steps after 2 warm-ups")
         line["cpu_baseline"] = cb
     if rank == 0:
         EMIT(json.dumps(line))
@@ -1064,7 +1108,12 @@ def main():
     ap.add_argument("--no-extras", action="store_true", dest="no_extras",
                     help="skip the device timings of the other BASELINE.json configs (other_configs key)")
     ap.add_argument("--no-e2e", action="store_true", help="skip the host-buffer end-to-end leg (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", dest="dump_outputs",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32 / float64, about 52 MB; "
+                         "a fixed sample of the pooled ROI feature rows); both arms write the same names")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -7,7 +7,9 @@ not exist on the GPU box, nothing at test time reads it).
 The reference modules are imported unmodified from /root/reference/lib (under the package name
 ``reflib``; its ``__init__`` files are replaced by empty stub packages because they import the
 backbones, data pipeline, ...).  ``tensorflow`` resolves to tests/golden/tf_numpy_shim.py -- see its
-docstring for what that does and does not pin.
+docstring for what that does and does not pin.  The FPN maps of case 4 and the SOLOv2 logits of case 14 are
+regenerated at load time instead of stored, and case 4's pooled outputs are kept for a sample of rows
+(reference_golden.py), so that the file stays under 1 MB.
 """
 import importlib
 import os
@@ -22,6 +24,7 @@ sys.path.insert(0, ROOT)
 sys.path.insert(0, HERE)
 REF = "/root/reference/lib"
 
+import reference_golden as golden  # noqa: E402
 import tf_numpy_shim as shim  # noqa: E402
 
 t = shim.t
@@ -125,24 +128,24 @@ def main(out_path=None):
 
     # ---- 4. assign_boxes_to_levels + ROIAlign + ROIPooler (poolers.py, roi_align.py, functional.py)
     Nimg, C = 2, 8
-    feats = [rng.standard_normal((Nimg, h, w, C)).astype(np.float32) for h, w in ((50, 84), (25, 42), (13, 21), (7, 11))]
+    feat_state = golden.pack_state(rng)  # stored instead of the maps: golden.rp_feats(feat_state) draws them again
+    feats = [rng.standard_normal((Nimg, h, w, C)).astype(np.float32) for h, w in golden.FEAT_HW]
     boxes, idx = syn.rois(Nimg, 60, seed=501, image_hw=(200, 333))
     boxes[:4] += 40
-    out["rp_boxes"], out["rp_idx"] = boxes, idx
-    for l, f in enumerate(feats):
-        out[f"rp_feat{l}"] = f
+    out["rp_boxes"], out["rp_idx"], out["rp_feat_state"] = boxes, idx, feat_state
     out["rp_levels"] = np.asarray(R.poolers.assign_boxes_to_levels(BoxList(t(boxes)), 2, 5, 224, 4))
+    out["rp_levels56"] = np.asarray(R.poolers.assign_boxes_to_levels(BoxList(t(boxes)), 2, 5, 56, 4))
+    rows = out["rp_rows"] = golden.roi_rows(out["rp_levels56"])
     sparse = SparseBoxList(t(idx), BoxList(t(boxes)), [Nimg, 60])
     for ptype, sr, osz in (("ROIAlignV2", 0, 7), ("ROIAlignV2", 2, 7), ("ROIAlign", 0, 14)):
         pooler = R.poolers.ROIPooler((osz, osz), [1 / 4., 1 / 8., 1 / 16., 1 / 32.], sr, ptype,
                                      canonical_box_size=56)  # small canonical size: all 4 levels populated
-        out[f"rp_out_{ptype}_{sr}_{osz}"] = np.asarray(pooler([t(f) for f in feats], sparse))
-    out["rp_levels56"] = np.asarray(R.poolers.assign_boxes_to_levels(BoxList(t(boxes)), 2, 5, 56, 4))
+        out[f"rp_out_{ptype}_{sr}_{osz}"] = np.asarray(pooler([t(f) for f in feats], sparse))[rows]
     bi = idx[:, 0].astype(np.int32)
     ra = R.roi_align.ROIAlign((7, 7), 1 / 8., 0, aligned=True)
-    out["ra_single"] = np.asarray(ra(t(feats[1]), t(boxes), t(bi)))
+    out["ra_single"] = np.asarray(ra(t(feats[1]), t(boxes), t(bi)))[rows]
     out["cr_nopad"] = np.asarray(R.functional.crop_and_resize(t(feats[0]), t(boxes * 0.25), t(bi), [5, 6], aligned=True,
-                                                              pad_border=False))
+                                                              pad_border=False))[rows]
 
     # ---- 5. find_top_rpn_proposals (rpn_outputs.py:29-132)
     Nimg = 2
@@ -264,7 +267,8 @@ def main(out_path=None):
 
     # ---- 14. MaskKernelBranch.inference (solo_v2.py:476-612) with image_shape == mask-feature size (resize = identity).
     # The op under test starts after the dynamic conv, so the generator repeats the candidate selection (:481-497)
-    # and the 1x1 conv (:499-511) in numpy to record the op's inputs; everything after is the reference's code.
+    # and the 1x1 conv (:499-511, golden.so_logits at load time) to record the op's inputs; everything after is the
+    # reference's code.
     Nimg, K, E, Hm, Wm = 2, 3, 8, 24, 32
     grids, sstr = [6, 4], [8, 16]
     shead = types.SimpleNamespace(score_threshold=0.3, num_grids=grids, strides=sstr, mask_kernel_size=1,
@@ -282,7 +286,6 @@ def main(out_path=None):
     flat_k = np.concatenate([k_.reshape(Nimg, -1, E) for k_ in kerns], 1)
     cell_stride = np.concatenate([np.full(g_ * g_, s_, np.float32) for g_, s_ in zip(grids, sstr)])
     ncap = int(max((flat_p[i] > 0.3).sum() for i in range(Nimg)))
-    so_logits = np.zeros((Nimg, ncap, Hm, Wm), np.float32)
     so_sc, so_cl, so_st = np.zeros((Nimg, ncap), np.float32), np.zeros((Nimg, ncap), np.int64), np.ones((Nimg, ncap), np.float32)
     so_cnt = np.zeros(Nimg, np.int32)
     so_kern = np.zeros((Nimg, ncap, E), np.float32)  # the gathered pred_kernels (:486): input of the fused dynamic conv
@@ -294,10 +297,9 @@ def main(out_path=None):
         so_cl[i, :c_] = keep[:, 1]
         so_st[i, :c_] = cell_stride[keep[:, 0]]
         so_kern[i, :c_] = flat_k[i][keep[:, 0]]
-        so_logits[i, :c_] = np.einsum("nhwc,co->nhwo", mfeat[i:i + 1], flat_k[i][keep[:, 0]].T.copy())[0].transpose(2, 0, 1)
     for li, (p_, k_) in enumerate(zip(probs, kerns)):  # the raw arguments of MaskKernelBranch.inference
         out[f"so_raw_probs_{li}"], out[f"so_raw_kernels_{li}"] = p_, k_
-    out.update(so_in_logits=so_logits, so_in_scores=so_sc, so_in_classes=so_cl, so_in_strides=so_st, so_in_counts=so_cnt,
+    out.update(so_in_scores=so_sc, so_in_classes=so_cl, so_in_strides=so_st, so_in_counts=so_cnt,
                so_in_mask_features=mfeat, so_in_kernels=so_kern)
 
     # ---- 15. the same inference with image_shape != mask-feature size: resize_images (functional.py:9-36 takes the

@@ -7,16 +7,18 @@ Exact (np.array_equal) wherever the path contains only +,-,*,/,min,max,compare,f
 where numpy's exp/log stand in for Eigen's (apply_deltas/get_deltas/matrix_nms), per north_star.
 """
 import os
+import sys
 
 import numpy as np
 import pytest
 
-G = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
+import reference_golden  # noqa: E402
 
 
 @pytest.fixture(scope="module")
 def z():
-    return np.load(os.path.join(G, "reference_python.npz"))
+    return reference_golden.load()
 
 
 def test_pairwise_iou(oracle_lib, z):
@@ -52,14 +54,16 @@ def test_roi_pooler(oracle_lib, z, ptype, sr, osz):
     feats = [z[f"rp_feat{l}"] for l in range(4)]
     got, _ = oracle_lib.roi_pooler(feats, [1 / 4., 1 / 8., 1 / 16., 1 / 32.], z["rp_boxes"], z["rp_idx"][:, 0],
                                    (osz, osz), sr, aligned=(ptype == "ROIAlignV2"), canonical_box_size=56)
-    assert np.array_equal(got, z[f"rp_out_{ptype}_{sr}_{osz}"])
+    assert np.array_equal(got[z["rp_rows"]], z[f"rp_out_{ptype}_{sr}_{osz}"])
 
 
 def test_roi_align_and_crop(oracle_lib, z):
     bi = z["rp_idx"][:, 0].astype(np.int32)
-    assert np.array_equal(oracle_lib.roi_align(z["rp_feat1"], z["rp_boxes"], bi, (7, 7), 1 / 8., 0, True), z["ra_single"])
+    rows = z["rp_rows"]
+    got = oracle_lib.roi_align(z["rp_feat1"], z["rp_boxes"], bi, (7, 7), 1 / 8., 0, True)
+    assert np.array_equal(got[rows], z["ra_single"])
     got = oracle_lib.crop_and_resize(z["rp_feat0"], z["rp_boxes"] * np.float32(0.25), bi, (5, 6), True, False)
-    assert np.array_equal(got, z["cr_nopad"])
+    assert np.array_equal(got[rows], z["cr_nopad"])
 
 
 def test_find_top_rpn_proposals(oracle_lib, z):

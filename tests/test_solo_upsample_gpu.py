@@ -2,12 +2,16 @@
 solo_v2.py:599-627: bilinear resize of the kept masks to the image size, threshold, boxes from masks -- against the
 CPU oracle and the reference-python golden.  Integer / byte work: masks, packed words and boxes are compared exactly."""
 import os
+import sys
 
 import numpy as np
 import pytest
 import torch
 
 from detectron2_tensorflow_b200.modeling import solo_upsample_masks
+
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
+import reference_golden  # noqa: E402
 
 pytestmark = pytest.mark.gpu
 
@@ -75,7 +79,7 @@ def test_reference_python_golden(cuda):
     """MaskKernelBranch.inference of the reference with image_shape != mask size (tests/golden/make_reference_golden.py
     case 15): the image-size masks and the boxes, bit-exact, from the packed masks of the CUDA tail."""
     from detectron2_tensorflow_b200.modeling import SOLOv2Inference
-    z = np.load(os.path.join(os.path.dirname(__file__), "golden", "reference_python.npz"))
+    z = reference_golden.load()
     head = SOLOv2Inference(0.5, 30, "gaussian", 2.0, 0.05, 12)
     tail = head.postprocess(T(z["so_in_logits"], cuda), T(z["so_in_scores"], cuda), T(z["so_in_classes"], cuda),
                             T(z["so_in_strides"], cuda), T(z["so_in_counts"], cuda), return_masks=False)

@@ -1,5 +1,5 @@
 import sys, os
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
 from detectron2_tensorflow_b200.modeling import solo_upsample_masks
 from detectron2_tensorflow_b200.utils import synthetic as syn
