@@ -1,6 +1,5 @@
 // api.cu -- version, status strings and the thread-local error detail.
 #include <stdarg.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 
@@ -13,11 +12,6 @@ void set_last_error(const char* fmt, ...) {
   va_end(ap);
 }
 bool pdl_enabled(cudaStream_t st) {
-  static const int mode = [] {  // 0 = never, 1 = always, 2 = eager launches only (default)
-    const char* e = getenv("D2B_PDL");
-    return !e ? 2 : (e[0] == '0' ? 0 : (e[0] == '1' ? 1 : 2));
-  }();
-  if (mode != 2) return mode == 1;
   cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
   if (cudaStreamIsCapturing(st, &cs) != cudaSuccess) {
     cudaGetLastError();

@@ -76,9 +76,9 @@ __device__ __forceinline__ void d2b_prof_stamp(int slot) {
 // profiles/r02aj_step_probe_*.jsonl): eager chains gain (Fast R-CNN post 87 -> 68 us at 2 images), but the step the
 // bench replays is a captured multi-stream graph and there the programmatic edges cost time (2 image blocks: 0.209 ->
 // 0.257 ms; 4 blocks of 16 images: 0.648 -> 0.701 ms).  Hence: the attribute is set on EAGER launches only -- never
-// while the stream is being captured -- unless D2B_PDL=0 (never) or D2B_PDL=1 (always) says otherwise.  The RetinaNet
-// top-k chain does not use it at all: there it measured slower even eagerly (0.572 -> 0.645 ms at N = 32: the early
-// CTAs of the dependents take slots from the HBM-bound scan); Matrix-NMS gains a little (0.418 -> 0.4135 ms).
+// while the stream is being captured.  The RetinaNet top-k chain does not use it at all: there it measured slower
+// even eagerly (0.572 -> 0.645 ms at N = 32: the early CTAs of the dependents take slots from the HBM-bound scan);
+// Matrix-NMS gains a little (0.418 -> 0.4135 ms).
 bool pdl_enabled(cudaStream_t st);
 __device__ __forceinline__ void grid_dep_sync() {
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");

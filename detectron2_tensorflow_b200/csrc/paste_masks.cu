@@ -4,28 +4,25 @@
 // The reference crops every box mask to the FULL image with tf.image.crop_and_resize on inverted boxes,
 // materialising [M, H, W, 1] fp32 (430 MB per 100 detections at 800x1344), then thresholds to uint8.
 // Here the bilinear sample and the threshold are fused and only the uint8 plane is written: the op is
-// bound by that write (1 B/pixel).  Pixels outside the box are zeros by the extrapolation rule, so a CTA
-// whose rows miss the box stores zeros without touching the mask.
-#include <stdlib.h>
-
+// bound by that write (1 B/pixel).  Pixels outside the box are zeros by the extrapolation rule, so the
+// planes are zero-filled by a memset, and paste_boxes_kernel then visits only a conservative bounding
+// rectangle of each box -- the index range the inverse of the affine crop_and_resize map gives, widened
+// by 2 -- and applies the exact per-pixel rule there, storing the ones.  A one-pass kernel that computed
+// every pixel wrote 2.3-2.5 TB/s on a B200 against 7.3 TB/s for the memset.
 #include "kernels.cuh"
 
 namespace d2b {
 namespace {
 
 constexpr int kPasteThreads = 256;
-constexpr int kPx = 16;      // output pixels (bytes) per thread per iteration: one 16-byte store
-constexpr int kIters = 8;    // iterations per CTA
 constexpr int kMaxMaskSmem = 16384;  // floats
 
 struct PasteArgs {
   const float* masks;  // [M, mh, mw]
   const float* boxes;  // [M, 4] absolute yxyx in output-image pixels
-  long long M;
   int mh, mw, H, W;
   float thr;
   uint8_t* out;  // [M, H, W]
-  int vec;       // 16-byte stores allowed
   int smem_mask;
 };
 
@@ -33,9 +30,6 @@ struct Axis {  // tf.image.crop_and_resize coordinate rule along one axis
   float n1, step, mid;
   int crop, dim;
   __device__ __forceinline__ float at(int i) const { return crop > 1 ? n1 * (float)(dim - 1) + (float)i * step : mid; }
-  // the same value from the index held as a float (exact below 2^24): the int -> float conversion per pixel ran on the
-  // quarter-rate XU pipe, which was the kernel's limiter
-  __device__ __forceinline__ float at_f(float fi) const { return crop > 1 ? n1 * (float)(dim - 1) + fi * step : mid; }
 };
 __device__ __forceinline__ Axis make_axis(float lo, float hi, int crop, int dim) {
   Axis a;
@@ -49,101 +43,6 @@ __device__ __forceinline__ Axis make_axis(float lo, float hi, int crop, int dim)
   return a;
 }
 
-__global__ void __launch_bounds__(kPasteThreads) paste_masks_kernel(PasteArgs a) {
-  extern __shared__ float s_mask[];
-  const long long m = blockIdx.y;
-  const unsigned plane = (unsigned)a.H * (unsigned)a.W;  // < 2^31 (checked on the host): 32-bit index math
-  const unsigned cta_first = blockIdx.x * (unsigned)(kPasteThreads * kPx * kIters);
-  if (cta_first >= plane) return;
-  const unsigned cta_last = min(plane, cta_first + (unsigned)(kPasteThreads * kPx * kIters)) - 1u;
-  const float4 bx = __ldg(reinterpret_cast<const float4*>(a.boxes) + m);
-  // to_normalized_coordinates: scale by 1/height, 1/width (box_list_ops.py:829-839)
-  const float ys = 1.0f / (float)a.H, xs = 1.0f / (float)a.W;
-  const Axis ay = make_axis(ys * bx.x, ys * bx.z, a.H, a.mh);
-  const Axis ax = make_axis(xs * bx.y, xs * bx.w, a.W, a.mw);
-  const float ymax_in = (float)(a.mh - 1), xmax_in = (float)(a.mw - 1);
-  // does any output row of this CTA fall inside the mask?
-  const int yA = (int)(cta_first / (unsigned)a.W), yB = (int)(cta_last / (unsigned)a.W);
-  // at(i) is monotone in i under fp32 rounding (monotone product + monotone sum), so the rows of this
-  // CTA map into [min(at(yA), at(yB)), max(...)]; NaN coordinates compare false -> zeros, as the exact rule.
-  const float e0 = ay.at(yA), e1 = ay.at(yB);
-  const bool any = fminf(e0, e1) <= ymax_in && fmaxf(e0, e1) >= 0.0f && e0 == e0 && e1 == e1;
-  const float* mk = a.masks + (size_t)m * a.mh * a.mw;
-  if (any && a.smem_mask) {  // block-uniform
-    for (int i = threadIdx.x; i < a.mh * a.mw; i += kPasteThreads) s_mask[i] = __ldg(mk + i);
-    __syncthreads();
-    mk = s_mask;
-  }
-  uint8_t* o = a.out + (size_t)m * (size_t)plane;
-  for (int it = 0; it < kIters; ++it) {
-    const unsigned p0 = cta_first + (unsigned)(it * kPasteThreads + threadIdx.x) * kPx;
-    if (p0 >= plane) break;
-    int y = (int)(p0 / (unsigned)a.W), x = (int)(p0 - (unsigned)y * (unsigned)a.W);
-    unsigned pk[4] = {0u, 0u, 0u, 0u};
-    // A run of kPx pixels inside one row whose row, or whose whole column span, misses the mask is zeros by the
-    // extrapolation rule: decided from the row coordinate and the two END columns (at() is monotone in the index, see
-    // above; a NaN coordinate compares false and takes the per-pixel path).  With ~1 % of the pixels inside a box the
-    // per-pixel loop was the bound (84 % issue-active at 2.3 TB/s written); now it only runs where a box is.
-    bool work = any;
-    if (any && x + kPx <= a.W) {
-      const float in_y = ay.at(y);
-      if (in_y < 0.0f || in_y > ymax_in) work = false;
-      else {
-        const float c0 = ax.at(x), c1 = ax.at(x + kPx - 1);
-        if (fmaxf(c0, c1) < 0.0f || fminf(c0, c1) > xmax_in) work = (c0 != c0) || (c1 != c1);
-      }
-    }
-    if (work) {
-      int top = 0, bot = 0;
-      float ly = 0.0f;
-      bool vy = false;
-      int cur_y = -1;
-      float xf = (float)x;
-#pragma unroll
-      for (int j = 0; j < kPx; ++j) {
-        if (p0 + j < plane) {
-          if (y != cur_y) {
-            const float in_y = ay.at(y);
-            vy = in_y >= 0.0f && in_y <= ymax_in;
-            const float f = floorf(in_y);
-            top = (int)f; bot = (int)ceilf(in_y);
-            ly = in_y - f;
-            cur_y = y;
-          }
-          if (vy) {
-            const float in_x = ax.at_f(xf);
-            if (in_x >= 0.0f && in_x <= xmax_in) {
-              // floor / ceil of a value in [0, mw - 1]: truncation, and floor + 1 unless the value is an integer
-              const int left = (int)in_x;
-              const float f = (float)left;
-              const float lx = in_x - f;
-              const int right = left + (lx > 0.0f ? 1 : 0);
-              const float tl = mk[top * a.mw + left], tr = mk[top * a.mw + right];
-              const float bl = mk[bot * a.mw + left], br = mk[bot * a.mw + right];
-              float t = tr - tl; t = t * lx; t = tl + t;
-              float bb = br - bl; bb = bb * lx; bb = bl + bb;
-              float r = bb - t; r = r * ly; r = t + r;
-              if (r > a.thr) pk[j >> 2] |= 1u << (8 * (j & 3));
-            }
-          }
-          if (++x == a.W) { x = 0; ++y; xf = 0.0f; } else { xf = xf + 1.0f; }
-        }
-      }
-    }
-    if (a.vec && p0 + kPx <= plane) {
-      __stcs(reinterpret_cast<uint4*>(o + p0), make_uint4(pk[0], pk[1], pk[2], pk[3]));
-    } else {
-#pragma unroll
-      for (int j = 0; j < kPx; ++j)  // (static indices: a run-time index would push pk[] to local memory)
-        if (p0 + j < plane) o[p0 + j] = (uint8_t)((pk[j >> 2] >> (8 * (j & 3))) & 0xffu);
-    }
-  }
-}
-
-// ---- two-phase variant (the default): the output is zero-filled at memset speed (7.3 TB/s on a B200; the fused kernel
-// above wrote 2.3-2.5 TB/s because the warps that straddle a box run the 16-pixel body with most lanes idle), then
-// this kernel visits only a conservative bounding rectangle of each box -- the index range the inverse of the affine
-// crop_and_resize map gives, widened by 2 -- and applies the SAME exact per-pixel rule there, storing the ones.
 #ifndef D2B_PASTE_RECT_CTAS
 #define D2B_PASTE_RECT_CTAS 8  // A/B at 1,600 masks: 32 -> 0.515 ms, 16 -> 0.452, 8 -> 0.431, 4 -> 0.441, 2 -> 0.476
 #endif
@@ -168,6 +67,7 @@ __global__ void __launch_bounds__(kPasteThreads) paste_boxes_kernel(PasteArgs a)
   extern __shared__ float s_mask[];
   const long long m = blockIdx.y;
   const float4 bx = __ldg(reinterpret_cast<const float4*>(a.boxes) + m);
+  // to_normalized_coordinates: scale by 1/height, 1/width (box_list_ops.py:829-839)
   const float ys = 1.0f / (float)a.H, xs = 1.0f / (float)a.W;
   const Axis ay = make_axis(ys * bx.x, ys * bx.z, a.H, a.mh);
   const Axis ax = make_axis(xs * bx.y, xs * bx.w, a.W, a.mw);
@@ -225,26 +125,18 @@ extern "C" int d2b_paste_masks(const d2b_paste_masks_params* p, void*, size_t, d
   a.masks = p->box_masks; a.boxes = p->boxes; a.mh = p->mask_h; a.mw = p->mask_w;
   a.H = p->image_h; a.W = p->image_w; a.thr = p->mask_threshold;
   const long long plane = (long long)a.H * a.W;
-  a.vec = (plane % 16 == 0) && ((reinterpret_cast<uintptr_t>(p->out) & 15) == 0);
   a.smem_mask = (a.mh * a.mw <= kMaxMaskSmem);
   const size_t smem = a.smem_mask ? sizeof(float) * a.mh * a.mw : 0;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
+  D2B_CUDA(cudaMemsetAsync(p->out, 0, (size_t)p->num_masks * (size_t)plane, st));
   if (smem > 48 * 1024)
-    D2B_CUDA(cudaFuncSetAttribute(paste_masks_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  const unsigned gx = (unsigned)((plane + kPasteThreads * kPx * kIters - 1) / (kPasteThreads * kPx * kIters));
-  const char* fused_env = getenv("D2B_PASTE_FUSED");  // tests / A-B: the one-pass kernel
-  const bool two_phase = !(fused_env && fused_env[0] == '1');
-  if (two_phase) D2B_CUDA(cudaMemsetAsync(p->out, 0, (size_t)p->num_masks * (size_t)plane, st));
-  if (two_phase && smem > 48 * 1024)
     D2B_CUDA(cudaFuncSetAttribute(paste_boxes_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   for (long long m0 = 0; m0 < p->num_masks; m0 += 65535) {  // grid.y limit
     const long long cnt = p->num_masks - m0 < 65535 ? p->num_masks - m0 : 65535;
     a.masks = p->box_masks + (size_t)m0 * a.mh * a.mw;
     a.boxes = p->boxes + 4 * m0;
     a.out = p->out + (size_t)m0 * plane;
-    a.M = cnt;
-    if (two_phase) paste_boxes_kernel<<<dim3(kRectCtas, (unsigned)cnt), kPasteThreads, smem, st>>>(a);
-    else paste_masks_kernel<<<dim3(gx, (unsigned)cnt), kPasteThreads, smem, st>>>(a);
+    paste_boxes_kernel<<<dim3(kRectCtas, (unsigned)cnt), kPasteThreads, smem, st>>>(a);
     D2B_LAUNCH_CHECK();
   }
   return D2B_OK;

@@ -5,9 +5,9 @@
 // one contraction on the path, so it runs on the 5th-generation tensor cores:
 //   * tcgen05.mma kind::tf32, M=128 (mask kernels) x N=256 (pixels) x K=8, accumulators in TMEM (2 x 256 columns,
 //     double buffered), operands staged by TMA (cp.async.bulk.tensor, 128-byte swizzle) through an mbarrier ring;
-//     by default two CTAs of a cluster form a cta_group::2 pair (M=256): each CTA owns one 128-row block of D in its
-//     own TMEM and stages / converts only HALF of the feature tile, the leader CTA issues the MMAs for both and
-//     tcgen05.commit multicasts the completion to the barriers of both CTAs;
+//     with more than 128 mask kernels two CTAs of a cluster form a cta_group::2 pair (M=256): each CTA owns one
+//     128-row block of D in its own TMEM and stages / converts only HALF of the feature tile, the leader CTA issues
+//     the MMAs for both and tcgen05.commit multicasts the completion to the barriers of both CTAs;
 //   * fp32 accuracy from three tf32 products per k-step (3xTF32: a = a_hi + a_lo, D += a_lo.b_hi + a_hi.b_hi +
 //     a_hi.b_lo; the dropped a_lo.b_lo is O(2^-22)): the kernels are split once by a tiny prologue kernel (both halves
 //     rounded to tf32); for the feature tile the raw fp32 tile IS the hi half (the tensor core ignores the low 13
@@ -23,7 +23,6 @@
 // Warp roles: 0 = TMA producer, 1 = MMA issuer (+ TMEM owner), 2-5 = converters, 6-13 = epilogue.
 #include <cuda.h>
 #include <math.h>
-#include <stdlib.h>
 
 #include "kernels.cuh"
 
@@ -523,28 +522,11 @@ int make_map(CUtensorMap* m, const void* ptr, int E, long long rows, int batch, 
   return D2B_OK;
 }
 
-// Variants (all four are built and parity-tested; measured at 16 x 500 x 200x336, E=256):
-//   pair, BK=32 (128-byte swizzle, 3 stages of 64 KB)  1.19 ms   <- default when n > 128
-//   one CTA, BK=16 (64-byte swizzle, 4 stages of 48 KB) 1.23 ms   <- default when n <= 128 (a pair would idle one SM)
+// Variants measured at 16 x 500 x 200x336, E=256 (the two slower ones were removed):
+//   pair, BK=32 (128-byte swizzle, 3 stages of 64 KB)  1.19 ms   <- used when n > 128
+//   one CTA, BK=16 (64-byte swizzle, 4 stages of 48 KB) 1.23 ms   <- used when n <= 128 (a pair would idle one SM)
 //   one CTA, BK=32 (2 stages of 96 KB)                  1.29 ms
 //   pair, BK=16 (6 stages of 32 KB)                     1.74 ms
-// D2B_DYNCONV_CTAS=1 / D2B_DYNCONV_BK=16|32 override the choice (measurement only).
-int dyn_block_k(int ctas) {
-  static const int forced = []() {
-    const char* e = getenv("D2B_DYNCONV_BK");
-    const int v = e ? atoi(e) : 0;
-    return (v == 16 || v == 32) ? v : 0;
-  }();
-  return forced ? forced : (ctas == 2 ? 32 : 16);
-}
-int dyn_ctas() {
-  static const int c = []() {
-    const char* e = getenv("D2B_DYNCONV_CTAS");
-    return (e && atoi(e) == 1) ? 1 : 2;
-  }();
-  return c;
-}
-
 template <int BK, int CTAS>
 int launch_dyn(const CUtensorMap& tm_ahi, const CUtensorMap& tm_alo, const CUtensorMap& tm_feat, const DynArgs& a, int sms,
                int dev, cudaStream_t st) {
@@ -628,8 +610,8 @@ extern "C" int d2b_solo_dynamic_masks(const d2b_solo_dynamic_masks_params* p, vo
   a.RB = (p->n + kBM - 1) / kBM;
   a.PT = (int)((p->hw + kBN - 1) / kBN);
   // a cta_group::2 pair works on two row blocks at once; with a single row block (n <= 128) it would idle one SM
-  const int ctas = (dyn_ctas() == 2 && p->n > kBM) ? 2 : 1;
-  const int bk = dyn_block_k(ctas);
+  const int ctas = p->n > kBM ? 2 : 1;
+  const int bk = ctas == 2 ? 32 : 16;
   a.KB = (E + bk - 1) / bk;
   a.Wd = (int)((p->hw + 63) / 64);
   a.thr = p->mask_threshold;
@@ -671,8 +653,6 @@ extern "C" int d2b_solo_dynamic_masks(const d2b_solo_dynamic_masks_params* p, vo
     sm_count[dev] = v > 0 ? v : 148;
   }
   const int sms = (dev >= 0 && dev < 64) ? sm_count[dev] : 148;
-  if (ctas == 2) return bk == 32 ? launch_dyn<32, 2>(tm_ahi, tm_alo, tm_feat, a, sms, dev, st)
-                                 : launch_dyn<16, 2>(tm_ahi, tm_alo, tm_feat, a, sms, dev, st);
-  return bk == 32 ? launch_dyn<32, 1>(tm_ahi, tm_alo, tm_feat, a, sms, dev, st)
-                  : launch_dyn<16, 1>(tm_ahi, tm_alo, tm_feat, a, sms, dev, st);
+  if (ctas == 2) return launch_dyn<32, 2>(tm_ahi, tm_alo, tm_feat, a, sms, dev, st);
+  return launch_dyn<16, 1>(tm_ahi, tm_alo, tm_feat, a, sms, dev, st);
 }

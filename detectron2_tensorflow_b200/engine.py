@@ -148,7 +148,7 @@ class MaskRCNNPostBackbone(object):
             st["mask_feats"] = self.mask_pooler(x["feats"], dinst)
 
     # ------------------------------------------------------------------ CUDA-graphed, chunk-concurrent step
-    def capture(self, x, chunks=4, epilogue=None, epilogue_warmup=True, hbm_lane=False):
+    def capture(self, x, chunks=4, epilogue=None, epilogue_warmup=True):
         """Capture the device-resident step as ONE CUDA graph in which the batch is cut into `chunks` image blocks
         that run on their own streams (forked from / joined to the capturing stream).  Images are independent, so
         the latency-bound proposal / post-processing kernels of one block overlap the HBM-bound ROIAlign of
@@ -178,38 +178,10 @@ class MaskRCNNPostBackbone(object):
             start = torch.cuda.Event()
             start.record(cur)
             outs = []
-            if not hbm_lane or chunks == 1:
-                for s, (b, e) in zip(streams, bounds):
-                    s.wait_event(start)
-                    with torch.cuda.stream(s):
-                        outs.append(self.flatten_outputs(self(cut(b, e))))
-            else:
-                xs = [cut(b, e) for b, e in bounds]
-                sts = [None] * chunks
-                lane = [None]  # the event of the last pooler in the lane
-
-                def in_lane(c, fn):
-                    with torch.cuda.stream(streams[c]):
-                        if lane[0] is not None:
-                            streams[c].wait_event(lane[0])
-                        fn(xs[c], sts[c])
-                        ev = torch.cuda.Event()
-                        ev.record(streams[c])
-                        lane[0] = ev
-                lag = 2  # a detection stage lasts about two box poolers of a block
-                for i in range(chunks + lag):
-                    if i < chunks:
-                        streams[i].wait_event(start)
-                        with torch.cuda.stream(streams[i]):
-                            sts[i] = self.stage_proposals(xs[i])
-                        in_lane(i, self.stage_box_pool)
-                        with torch.cuda.stream(streams[i]):
-                            self.stage_detections(xs[i], sts[i])
-                    if i >= lag:
-                        in_lane(i - lag, self.stage_mask_pool)
-                for st in sts:
-                    outs.append(self.flatten_outputs(dict(proposals=st["props"], box_feats=st["box_feats"],
-                                                          dets=st["dets"], mask_feats=st["mask_feats"])))
+            for s, (b, e) in zip(streams, bounds):
+                s.wait_event(start)
+                with torch.cuda.stream(s):
+                    outs.append(self.flatten_outputs(self(cut(b, e))))
             for s in streams:
                 cur.wait_stream(s)
             if epilogue is not None and with_epilogue:
@@ -229,11 +201,11 @@ class MaskRCNNPostBackbone(object):
             outs = step()
         return GraphedStep(graph, outs, bounds, nv.kernel_launch_count() - l0)
 
-    def pipeline(self, x, chunks=4, depth=2, epilogues=None, epilogue_warmup=True, hbm_lane=False):
+    def pipeline(self, x, chunks=4, depth=2, epilogues=None, epilogue_warmup=True):
         """`depth` independent captures of the step over the same static inputs `x` -> StepPipeline
         (`epilogues[i]`: the capture epilogue of step i)."""
         depth = max(1, int(depth))
-        return StepPipeline([self.capture(x, chunks, epilogues[i] if epilogues else None, epilogue_warmup, hbm_lane)
+        return StepPipeline([self.capture(x, chunks, epilogues[i] if epilogues else None, epilogue_warmup)
                              for i in range(depth)],
                             x["shapes"].device)
 

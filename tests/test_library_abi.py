@@ -143,3 +143,18 @@ def test_no_cpu_fallback_in_product():
         from detectron2_tensorflow_b200.layers import ROIAlign
         with pytest.raises(nv.D2BError):
             ROIAlign((7, 7), 0.25, 0)(torch.zeros(1, 8, 8, 4), torch.zeros(1, 4), torch.zeros(1, dtype=torch.int32))
+
+
+def test_product_env_switches():
+    """The environment variables the product reads.  A run-time switch that selects a slower variant lets a user step
+    off the measured path; variants that lost their A/B are deleted, not left behind a switch.  D2B_RPN_GENERIC runs
+    the generic proposal chain (the only one for k > 4096) on inputs the specialised chain would take, so that tests
+    compare the two; D2B_LIB, NVCC and D2B_EXTRA_NVCC choose the library and the build."""
+    pkg = os.path.join(ROOT, "detectron2_tensorflow_b200")
+    read = re.compile(r"""(?:getenv|os\.environ\.get|os\.environ)\s*[(\[]\s*["']([A-Za-z0-9_]+)["']""")
+    names = set()
+    for dp, _, fs in os.walk(pkg):
+        for f in fs:
+            if f.endswith((".py", ".cu", ".cuh", ".cc")):
+                names.update(read.findall(open(os.path.join(dp, f)).read()))
+    assert names == {"D2B_RPN_GENERIC", "D2B_LIB", "NVCC", "D2B_EXTRA_NVCC"}

@@ -12,8 +12,8 @@ dev = torch.device("cuda", 0)
 x = bench.to_torch(bench.make_host_inputs(16), dev=dev)
 eng = bench.make_engine()
 res = {}
-for chunks, depth, lane in ((1, 3, False), (1, 4, False), (2, 2, False), (2, 3, False), (2, 4, False), (4, 1, False), (4, 2, False), (4, 3, False), (4, 4, False), (4, 6, False), (8, 2, False), (8, 3, False), (4, 3, True)):
-    pipe = eng.pipeline(x, chunks=chunks, depth=depth, hbm_lane=lane)
+for chunks, depth in ((1, 3), (1, 4), (2, 2), (2, 3), (2, 4), (4, 1), (4, 2), (4, 3), (4, 4), (4, 6), (8, 2), (8, 3)):
+    pipe = eng.pipeline(x, chunks=chunks, depth=depth)
     pipe.run(2 * depth)
     torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -21,7 +21,7 @@ for chunks, depth, lane in ((1, 3, False), (1, 4, False), (2, 2, False), (2, 3, 
     pipe.run(60)
     e1.record()
     torch.cuda.synchronize()
-    res[f"chunks{chunks}_inflight{depth}" + ("_hbm_lane" if lane else "")] = round(e0.elapsed_time(e1) / 60, 4)
+    res[f"chunks{chunks}_inflight{depth}"] = round(e0.elapsed_time(e1) / 60, 4)
     del pipe
     torch.cuda.empty_cache()
 print(json.dumps(res))
