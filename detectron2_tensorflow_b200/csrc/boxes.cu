@@ -104,6 +104,8 @@ extern "C" int d2b_batched_nms(const d2b_batched_nms_params* p, void* workspace,
   const int S = p->num_segments, n = p->n, mo = p->max_output_size;
   if (n == 0 || mo == 0) return nms_sorted(nullptr, nullptr, S, n, mo, p->iou_threshold, p->keep, p->num_keep, nullptr, st);
   D2B_REQUIRE(p->boxes && p->scores, "batched_nms: boxes/scores must be non-NULL");
+  const int size_rc = nms_check_sizes(n, mo);  // before the ordering launches below
+  if (size_rc != D2B_OK) return size_rc;
   if (nms_small_applies(n))  // the latency regime: the whole chain in one launch, no workspace
     return nms_small(p->boxes, p->scores, p->counts, S, n, mo, p->iou_threshold, p->keep, p->num_keep, st);
   if (workspace == nullptr || workspace_bytes < d2b_batched_nms_workspace_bytes(p)) {

@@ -117,6 +117,17 @@ static inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 b
   return cudaLaunchKernelEx(&L.cfg, kernel, static_cast<KArgs>(args)...);
 }
 
+// Raises `kernel`'s dynamic shared-memory limit to `smem` bytes when it is below that.  For a kernel with static
+// shared memory the default limit is 48 KB MINUS the static size, so a fixed "smem > 48 KB" test misses the sizes just
+// below 48 KB.  The limit is per kernel and per device, and is only ever raised.
+template <typename... KArgs>
+static inline cudaError_t allow_dynamic_smem(void (*kernel)(KArgs...), size_t smem) {
+  cudaFuncAttributes fa;
+  const cudaError_t e = cudaFuncGetAttributes(&fa, kernel);
+  if (e != cudaSuccess || smem <= (size_t)fa.maxDynamicSharedSizeBytes) return e;
+  return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+}
+
 static inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
 // Bump allocator over the caller's workspace (256-byte aligned slices).

@@ -43,6 +43,9 @@ int nms_sorted(const float* boxes, const int32_t* counts, int S, int n, int max_
                int32_t* num_keep, void* ws, cudaStream_t st, bool sweep = true);
 bool nms_uses_bitmask(int n, int max_out);
 bool nms_lazy_applies(int n, int max_out);  // the capped lazy sweep would be chosen (cap << n)
+// D2B_OK when nms_sorted accepts (n, max_out), else D2B_EINVAL with the last error set; callers that launch work of
+// their own before nms_sorted check it first, so that a rejected call launches nothing.
+int nms_check_sizes(int n, int max_out);
 // Small segments with UNSORTED scores (n <= 512): order, mask, sweep and index un-mapping in ONE launch, one CTA per
 // segment; keep holds input indices (selection order, -1 padded).  No workspace.
 bool nms_small_applies(int n);

@@ -400,8 +400,7 @@ extern "C" int d2b_matrix_nms(const d2b_matrix_nms_params* p, void* workspace, s
   size_t iou_smem = (size_t)a.Wd * sizeof(u64);
   const int stage = iou_smem <= 160 * 1024;  // (larger masks: the row is re-read from L2 per pair)
   if (!stage) iou_smem = 0;
-  if (iou_smem > 48 * 1024)
-    D2B_CUDA(cudaFuncSetAttribute(mnms_iou_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)iou_smem));
+  if (iou_smem > 0) D2B_CUDA(allow_dynamic_smem(mnms_iou_kernel, iou_smem));
   D2B_CUDA(launch_pdl(mnms_iou_kernel, dim3(a.n, a.B), dim3(256), iou_smem, st, 0, a, stage));
   D2B_LAUNCH_CHECK();
   if (a.n <= kDecayStageMax) {

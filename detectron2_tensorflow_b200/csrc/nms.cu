@@ -377,8 +377,15 @@ bool use_lazy(int n, int max_out) {
 
 }  // namespace
 
+int nms_check_sizes(int n, int max_out) {
+  D2B_REQUIRE(use_lazy(n, max_out) || n <= kBitmaskMaxN,
+              "nms: n=%d with max_output_size=%d is not supported (n <= %d or cap <= %d)", n, max_out, kBitmaskMaxN,
+              kLazyMaxOut);
+  return D2B_OK;
+}
+
 size_t nms_sorted_workspace_bytes(int S, int n, int max_out) {
-  if (S <= 0 || n <= 0 || use_lazy(n, max_out)) return 0;
+  if (S <= 0 || n <= 0 || use_lazy(n, max_out) || n > kBitmaskMaxN) return 0;
   const size_t W = (n + 63) / 64;
   return ws_slice((size_t)S * W * 64 * W * sizeof(u64));
 }
@@ -394,8 +401,7 @@ int nms_small(const float* boxes, const float* scores, const int32_t* counts, in
   while (P < n) P <<= 1;
   const int W = (n + 63) / 64;
   const size_t smem = nms_small_smem(n, P);
-  if (smem > 48 * 1024)
-    D2B_CUDA(cudaFuncSetAttribute(nms_small_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  D2B_CUDA(allow_dynamic_smem(nms_small_kernel, smem));
   nms_small_kernel<<<S, kColSweepThreads, smem, st>>>(reinterpret_cast<const float4*>(boxes), scores, counts, n, P, W,
                                                       max_out, thr, keep, num_keep);
   D2B_LAUNCH_CHECK();
@@ -421,14 +427,13 @@ int nms_sorted(const float* boxes, const int32_t* counts, int S, int n, int max_
   const float4* b4 = reinterpret_cast<const float4*>(boxes);
   if (use_lazy(n, max_out)) {
     const size_t smem = (size_t)max_out * sizeof(float4);
-    if (smem > 48 * 1024)
-      D2B_CUDA(cudaFuncSetAttribute(nms_lazy_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    D2B_CUDA(allow_dynamic_smem(nms_lazy_kernel, smem));
     nms_lazy_kernel<<<S, kLazyThreads, smem, st>>>(b4, counts, n, max_out, thr, keep, num_keep);
     D2B_LAUNCH_CHECK();
     return D2B_OK;
   }
-  D2B_REQUIRE(n <= kBitmaskMaxN, "nms: n=%d with max_output_size=%d is not supported (n <= %d or cap <= %d)", n,
-              max_out, kBitmaskMaxN, kLazyMaxOut);
+  const int rc = nms_check_sizes(n, max_out);
+  if (rc != D2B_OK) return rc;
   const int W = (n + 63) / 64;
   u64* mask = static_cast<u64*>(ws);
   // few segments: spread a row block's column blocks over up to 4 CTAs so that the grid still fills the SMs

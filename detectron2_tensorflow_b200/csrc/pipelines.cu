@@ -675,8 +675,7 @@ extern "C" int d2b_rpn_proposals(const d2b_rpn_proposals_params* p, void* worksp
   if (rc != D2B_OK) return rc;
   const size_t merge_smem = (size_t)a.P2 * sizeof(uint32_t);
   const int merge_in_smem = merge_smem <= 160 * 1024;
-  if (merge_in_smem && merge_smem > 48 * 1024)
-    D2B_CUDA(cudaFuncSetAttribute(rpn_merge_rank_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)merge_smem));
+  if (merge_in_smem) D2B_CUDA(allow_dynamic_smem(rpn_merge_rank_kernel, merge_smem));
   rpn_merge_rank_kernel<<<a.N, kMergeThreads, merge_in_smem ? merge_smem : 0, st>>>(
       a, seg_boxes, seg_scores, keep, nkeep, keys2, merge_in_smem, reinterpret_cast<float4*>(p->out_boxes),
       p->out_logits, p->out_valid, p->out_num_valid);  // :101-114
@@ -901,8 +900,7 @@ extern "C" int d2b_retinanet_postprocess(const d2b_retinanet_params* p, void* wo
   D2B_LAUNCH_CHECK();
   const size_t merge_smem = (size_t)a.stride * sizeof(u64);
   if (merge_smem <= 96 * 1024) {  // the per-level runs are sorted already: merge by rank instead of sorting
-    if (merge_smem > 48 * 1024)  // per device / context: set on every call (cheap), as nms.cu and sort.cu do
-      D2B_CUDA(cudaFuncSetAttribute(retina_merge_rank_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)merge_smem));
+    D2B_CUDA(allow_dynamic_smem(retina_merge_rank_kernel, merge_smem));
     u64* keys3b = reinterpret_cast<u64*>(ws + pl.o_keys3b);
     retina_merge_rank_kernel<<<N, 1024, merge_smem, st>>>(keys3, lvl_off, a.L, a.P3, keys3b);
     D2B_LAUNCH_CHECK();

@@ -788,8 +788,7 @@ int rpn_sweep_merge_fused(const RpnArgs& a, const int32_t* seg_count, const unsi
   const int cap = a.post < a.k ? a.post : a.k;  // survivors per segment
   const size_t smem = (size_t)a.L * cap * sizeof(uint32_t) + align_up((size_t)cap * sizeof(uint16_t), 16);
   D2B_REQUIRE(smem <= 200 * 1024, "fused sweep: %d levels x %d survivors do not fit shared memory", a.L, cap);
-  if (smem > 48 * 1024)
-    D2B_CUDA(cudaFuncSetAttribute(rpn_sweep_merge_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  D2B_CUDA(allow_dynamic_smem(rpn_sweep_merge_kernel, smem));
   // one cluster per image (L <= D2B_MAX_LEVELS = 8: portable size)
   D2B_CUDA(launch_pdl(rpn_sweep_merge_kernel, dim3((unsigned)rows, 1, 1), dim3(kColSweepThreads, 1, 1), smem, st,
                       (unsigned)a.L, a, seg_count, W, cap, reinterpret_cast<const u64*>(mask), seg_boxes, seg_scores,
