@@ -39,8 +39,10 @@ int sort_segments_desc(unsigned long long* keys, int S, int P, const int32_t* se
 size_t nms_sorted_workspace_bytes(int S, int n, int max_out);
 // sweep = false (bitmask formulation only, see nms_uses_bitmask): only the suppression mask is built in `ws`
 // ([S][64 W][W] u64, W = ceil(n / 64)); the caller sweeps it itself (rpn_fused.cu fuses the sweep with the merge).
+// skip (device, optional, mask-only calls): no mask is built for segment s when skip[s / skip_group] != 0.
 int nms_sorted(const float* boxes, const int32_t* counts, int S, int n, int max_out, float thr, int32_t* keep,
-               int32_t* num_keep, void* ws, cudaStream_t st, bool sweep = true);
+               int32_t* num_keep, void* ws, cudaStream_t st, bool sweep = true, const int32_t* skip = nullptr,
+               int skip_group = 1);
 bool nms_uses_bitmask(int n, int max_out);
 bool nms_lazy_applies(int n, int max_out);  // the capped lazy sweep would be chosen (cap << n)
 // D2B_OK when nms_sorted accepts (n, max_out), else D2B_EINVAL with the last error set; callers that launch work of

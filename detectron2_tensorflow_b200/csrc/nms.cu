@@ -84,6 +84,7 @@ __device__ __forceinline__ FBox filter_box(const CBox c, float kf) {
 // grid (ceil(W/2), S, csplit).  mask word (i, w) of a segment (column-word major, nms_mask_index), bit c: box (w*64+c)
 // is suppressed by box i (only j > i).
 // csplit > 1 (few segments: the latency regime) deals the column blocks of a row block to csplit CTAs.
+// skip (optional): segment s is left alone when skip[s / skip_group] != 0 (its CTAs return at entry).
 // A CTA handles the 64-row blocks x and nb-1-x of its segment, so every CTA walks nb+1 column blocks (the upper
 // triangle is balanced).  8 independent warps per CTA: warp = (column group q, row half); it owns 32 rows of the
 // 64-row block and walks column blocks rb+q, rb+q+4, ...  The 64 column boxes of a block are staged in a
@@ -92,8 +93,10 @@ __device__ __forceinline__ FBox filter_box(const CBox c, float kf) {
 #define D2B_MASK_MINB 4  // 64 registers; 1 (98 registers), 5 (48) and 6 (40) measured the same or slower
 #endif
 __global__ void __launch_bounds__(kMaskThreads, D2B_MASK_MINB) nms_mask_kernel(const float4* boxes, const int32_t* counts, int n,
-                                                                 int W, float thr, u64* mask) {
+                                                                 int W, float thr, u64* mask, const int32_t* skip,
+                                                                 int skip_group) {
   grid_dep_sync();
+  if (skip && skip[blockIdx.y / skip_group]) return;
   __shared__ float4 s_flt[kMaskThreads / 32][64];  // (ylo, xlo, yhi, xhi) of the shrunk box
   __shared__ float4 s_box[kMaskThreads / 32][64];
   __shared__ float s_area[kMaskThreads / 32][64];
@@ -411,7 +414,7 @@ int nms_small(const float* boxes, const float* scores, const int32_t* counts, in
 bool nms_uses_bitmask(int n, int max_out) { return n > 0 && max_out > 0 && !use_lazy(n, max_out); }
 
 int nms_sorted(const float* boxes, const int32_t* counts, int S, int n, int max_out, float thr, int32_t* keep,
-               int32_t* num_keep, void* ws, cudaStream_t st, bool sweep) {
+               int32_t* num_keep, void* ws, cudaStream_t st, bool sweep, const int32_t* skip, int skip_group) {
   if (S <= 0) return D2B_OK;
   D2B_REQUIRE(max_out >= 0 && n >= 0, "nms: negative sizes");
   D2B_REQUIRE(thr >= 0.0f && thr <= 1.0f, "iou_threshold must be in [0, 1]");  // as tf.image.non_max_suppression
@@ -424,6 +427,7 @@ int nms_sorted(const float* boxes, const int32_t* counts, int S, int n, int max_
     D2B_CUDA(cudaMemsetAsync(keep, 0xff, sizeof(int32_t) * (size_t)S * max_out, st));
     return D2B_OK;
   }
+  D2B_REQUIRE(skip == nullptr || (!sweep && skip_group >= 1), "nms: skip flags apply to mask-only calls");
   const float4* b4 = reinterpret_cast<const float4*>(boxes);
   if (use_lazy(n, max_out)) {
     const size_t smem = (size_t)max_out * sizeof(float4);
@@ -440,7 +444,7 @@ int nms_sorted(const float* boxes, const int32_t* counts, int S, int n, int max_
   int csplit = 1;
   while (csplit < 4 && (long long)((W + 1) / 2) * S * csplit * 2 <= 2 * 148 && csplit * 8 < W) csplit *= 2;
   D2B_CUDA(launch_pdl(nms_mask_kernel, dim3((W + 1) / 2, S, csplit), dim3(kMaskThreads), 0, st, 0, b4, counts, n, W, thr,
-                      mask));
+                      mask, skip, skip_group));
   D2B_LAUNCH_CHECK();
   if (!sweep) return D2B_OK;  // the caller runs its own sweep over the mask (fused with the proposal merge)
   D2B_REQUIRE(W <= kColSweepMaxW, "nms: n=%d too large for the bitmask sweep", n);

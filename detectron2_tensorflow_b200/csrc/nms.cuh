@@ -12,6 +12,33 @@ __device__ __forceinline__ unsigned long long warp_or64(unsigned long long v) {
   return ((unsigned long long)hi << 32) | lo;
 }
 
+// Greedy resolve of one 64-candidate tile by a full warp, as a fixpoint (same result as the serial scan).  Lane l
+// holds the suppression rows of candidates l and l + 32 (dA, dB: bit c set = the row's candidate suppresses candidate
+// c, c > row); `rem` marks candidates already removed (suppressed from outside the tile, or absent).  Returns the
+// kept candidates, of which at most `left` (the first ones) remain when the cap is reached inside the tile.
+// Shared by the bitmask sweep (nms_sweep_columns), det_tail_kernel and rpn_lazy_merge_kernel.
+__device__ __forceinline__ unsigned long long nms_tile_resolve(unsigned long long dA, unsigned long long dB,
+                                                               unsigned long long rem, int left) {
+  typedef unsigned long long u64;
+  const int lane = threadIdx.x & 31;
+  const u64 bitA = 1ull << lane, bitB = 1ull << (lane + 32);
+  u64 U = ~rem, K = 0;
+  while (U) {  // warp-uniform
+    const u64 blocked = warp_or64(((U & bitA) ? dA : 0ull) | ((U & bitB) ? dB : 0ull));
+    const u64 nk = U & ~blocked;  // never empty: the first undecided candidate cannot be blocked
+    K |= nk;
+    U &= ~nk;
+    if (!U) break;  // (the usual sparse tile: nothing undecided is blocked, one round)
+    U &= ~warp_or64(((nk & bitA) ? dA : 0ull) | ((nk & bitB) ? dB : 0ull));
+  }
+  int c = __popcll(K);
+  while (c > left) {  // cap reached inside this tile: keep only the first `left`
+    K &= ~(1ull << (63 - __clzll((long long)K)));
+    --c;
+  }
+  return K;
+}
+
 // Greedy sweep over the suppression bitmask of ONE segment by a CTA of kColSweepThreads threads (32 warps).
 // mask word (row i, column word w), bit c: box i suppresses box 64w+c (only c > i is set / read).  In global memory
 // the mask is stored COLUMN-WORD MAJOR -- word (i, w) at w * (64 W) + i -- so that the 64 rows of a block's column
@@ -116,21 +143,7 @@ __device__ __forceinline__ int nms_sweep_columns(int cnt, int W, int max_out, co
     if (!capped) {
       u64 rem = warp_or64(acc);
       if (rows < 64) rem |= ~0ull << rows;
-      u64 U = ~rem;
-      while (U) {  // warp-uniform
-        const u64 blocked = warp_or64(((U & bitA) ? dA : 0ull) | ((U & bitB) ? dB : 0ull));
-        const u64 nk = U & ~blocked;  // never empty: the first undecided row cannot be blocked
-        K |= nk;
-        U &= ~nk;
-        if (!U) break;  // (the usual sparse tile: nothing undecided is blocked, one round)
-        U &= ~warp_or64(((nk & bitA) ? dA : 0ull) | ((nk & bitB) ? dB : 0ull));
-      }
-      int c = __popcll(K);
-      const int left = max_out - kept_before;
-      while (c > left) {  // cap reached inside this block: keep only the first `left`
-        K &= ~(1ull << (63 - __clzll((long long)K)));
-        --c;
-      }
+      K = nms_tile_resolve(dA, dB, rem, max_out - kept_before);
       D2B_BOUND(word, W);
       if (K & bitA) {
         const int slot = kept_before + __popcll(K & (bitA - 1ull));

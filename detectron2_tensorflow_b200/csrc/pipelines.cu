@@ -6,6 +6,7 @@
 // The reference runs them as tf.map_fn over images with a CPU NMS per segment.
 #include <stdlib.h>
 
+#include "nms.cuh"
 #include "rpn.cuh"
 
 namespace d2b {
@@ -68,9 +69,11 @@ struct RpnPlan {
   int rows;
   size_t bytes;
   // offsets
-  size_t o_topk, o_keys, o_kr, o_boxes, o_scores, o_count, o_keep, o_nkeep, o_nms, o_keys2;
+  size_t o_topk, o_keys, o_kr, o_boxes, o_scores, o_count, o_keep, o_nkeep, o_nms, o_keys2, o_done;
   bool fused_select;  // k small enough for the cluster-fused select / sort / decode kernel (rpn_fused.cu)
   bool fused_sweep;   // ... and the NMS is the bitmask formulation: column sweep fused with the per-image merge
+  bool lazy_merge;    // ... and the capped walk in merge order fits shared memory: masks + sweep only for the images
+                      // it does not finish
 };
 
 int rpn_plan(const d2b_rpn_proposals_params* p, RpnPlan& pl) {
@@ -79,6 +82,8 @@ int rpn_plan(const d2b_rpn_proposals_params* p, RpnPlan& pl) {
   D2B_REQUIRE(p->num_images >= 0, "num_images must be >= 0");
   D2B_REQUIRE(p->pre_nms_topk >= 1 && p->pre_nms_topk <= kTopkMaxK, "pre_nms_topk=%d out of [1,%d]", p->pre_nms_topk, kTopkMaxK);
   D2B_REQUIRE(p->post_nms_topk >= 1 && p->post_nms_topk <= kTopkMaxK, "post_nms_topk=%d out of [1,%d]", p->post_nms_topk, kTopkMaxK);
+  // as tf.image.non_max_suppression; checked here, before the first launch (the walk writes outputs)
+  D2B_REQUIRE(p->nms_thresh >= 0.0f && p->nms_thresh <= 1.0f, "nms_thresh must be in [0, 1]");
   RpnArgs& a = pl.a;
   TopkDesc& td = pl.td;
   long long maxlen = 0;
@@ -132,12 +137,14 @@ int rpn_plan(const d2b_rpn_proposals_params* p, RpnPlan& pl) {
   pl.o_nkeep = o; o += ws_slice(rows * sizeof(int32_t));
   pl.o_nms = o; o += nms_sorted_workspace_bytes(pl.rows, a.k, a.post);
   pl.o_keys2 = o; o += ws_slice(N * a.P2 * sizeof(uint32_t));
+  pl.o_done = o; o += ws_slice(N * sizeof(int32_t));  // the last slice: per-image "finished by the walk" flags
   pl.bytes = o;
   // D2B_RPN_GENERIC=1 forces the generic multi-launch chain (tests exercise both paths on the same inputs)
   const char* force_generic = getenv("D2B_RPN_GENERIC");
   pl.fused_select = a.k <= kRpnFusedMaxK && !(force_generic && force_generic[0] == '1');
   pl.fused_sweep = pl.fused_select && nms_uses_bitmask(a.k, a.post) &&
                    ((size_t)a.L * 4 + 2) * (a.post < a.k ? a.post : a.k) + 16 <= 200 * 1024;
+  pl.lazy_merge = pl.fused_sweep && a.N >= kRpnLazyMinImages && rpn_lazy_merge_smem(a) <= kRpnLazyMaxSmem;
   return D2B_OK;
 }
 
@@ -296,30 +303,12 @@ __global__ void __launch_bounds__(kTailThreads) det_tail_kernel(F f, const u64* 
         if (d2b_iou(bi, s_blk[c]) > thr) bits |= 1ull << c;
     if (bits) atomicOr(&s_diag[r], bits);
     __syncthreads();
-    if (tid < 32) {  // warp 0: greedy resolve of the 64 candidates as a fixpoint (same result as the serial scan)
-      const u64 dA = s_diag[lane], dB = s_diag[lane + 32];
+    if (tid < 32) {  // warp 0: greedy resolve of the 64 candidates (nms.cuh)
       u64 rem = ((u64)s_dead[1] << 32) | (u64)s_dead[0];
       if (rows < 64) rem |= ~0ull << rows;
+      const u64 K = nms_tile_resolve(s_diag[lane], s_diag[lane + 32], rem, max_out - kept);
+      const int c = __popcll(K);
       const u64 bitA = 1ull << lane, bitB = 1ull << (lane + 32);
-      u64 U = ~rem, K = 0;
-      while (U) {  // warp-uniform
-        const u64 sel = ((U & bitA) ? dA : 0ull) | ((U & bitB) ? dB : 0ull);
-        const u64 blocked = ((u64)__reduce_or_sync(0xffffffffu, (unsigned)(sel >> 32)) << 32) |
-                            __reduce_or_sync(0xffffffffu, (unsigned)sel);
-        const u64 nk = U & ~blocked;  // never empty: the first undecided candidate cannot be blocked
-        K |= nk;
-        U &= ~nk;
-        if (!U) break;
-        const u64 s2 = ((nk & bitA) ? dA : 0ull) | ((nk & bitB) ? dB : 0ull);
-        U &= ~(((u64)__reduce_or_sync(0xffffffffu, (unsigned)(s2 >> 32)) << 32) |
-               __reduce_or_sync(0xffffffffu, (unsigned)s2));
-      }
-      int c = __popcll(K);
-      const int left = max_out - kept;
-      while (c > left) {  // cap reached inside this block: keep only the first `left`
-        K &= ~(1ull << (63 - __clzll((long long)K)));
-        --c;
-      }
       if (K & bitA) { const int s = kept + __popcll(K & (bitA - 1ull)); s_kept[s] = s_blk[lane]; s_keptj[s] = b0 + lane; }
       if (K & bitB) { const int s = kept + __popcll(K & (bitB - 1ull)); s_kept[s] = s_blk[lane + 32]; s_keptj[s] = b0 + lane + 32; }
       if (lane == 0) s_kept_n = kept + c;
@@ -656,13 +645,23 @@ extern "C" int d2b_rpn_proposals(const d2b_rpn_proposals_params* p, void* worksp
     if (rc != D2B_OK) return rc;
   }
   if (pl.fused_sweep) {
+    int32_t* done = nullptr;
+    if (pl.lazy_merge) {
+      // NMS (:90-94) and merge (:101-114) as one capped walk per image in merge order; the images it does not finish
+      // within kRpnLazyMaxBlocks blocks are left to the launches below, which skip the finished ones
+      done = reinterpret_cast<int32_t*>(ws + pl.o_done);
+      rc = rpn_lazy_merge_fused(a, seg_count, seg_boxes, seg_scores, p->nms_thresh,
+                                reinterpret_cast<float4*>(p->out_boxes), p->out_logits, p->out_valid,
+                                p->out_num_valid, done, st);
+      if (rc != D2B_OK) return rc;
+    }
     // suppression masks (:90-94), then ONE launch sweeps every segment and merges each image's levels (:101-114)
     rc = nms_sorted(reinterpret_cast<const float*>(seg_boxes), seg_count, pl.rows, a.k, a.post, p->nms_thresh, keep,
-                    nkeep, ws + pl.o_nms, st, /*sweep=*/false);
+                    nkeep, ws + pl.o_nms, st, /*sweep=*/false, done, a.L);
     if (rc != D2B_OK) return rc;
     return rpn_sweep_merge_fused(a, seg_count, reinterpret_cast<const u64*>(ws + pl.o_nms), seg_boxes, seg_scores,
                                  reinterpret_cast<float4*>(p->out_boxes), p->out_logits, p->out_valid,
-                                 p->out_num_valid, st);
+                                 p->out_num_valid, done, st);
   }
   if (!pl.fused_select) {
     rc = topk_run(pl.td, keys, nullptr, nullptr, kr, ws + pl.o_topk, st);  // rpn_outputs.py:70

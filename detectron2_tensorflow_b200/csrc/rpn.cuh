@@ -69,6 +69,14 @@ struct RpnArgs {
   int k, P, post, P2;
 };
 
+// Shared-memory layout of rpn_lazy_merge_kernel (rpn_fused.cu), from sizes the host knows: a level holds at most
+// kcap = min(k, row length) candidates and keeps at most min(post, kcap) of them.  Scalars only: the kernel keeps
+// the per-level offsets in shared memory (an array here would put the struct in local memory).
+struct LazyLayout {
+  int R;  // merge-order entries: min(kRpnLazyMaxBlocks * 64, all candidates)
+  size_t o_cbox, o_keys, o_order, o_ids, bytes;
+};
+
 
 // One CTA per image: the final per-image top-k (rpn_outputs.py:101-114) as a rank computation.
 // Each level's NMS survivors are already ordered (score desc, index asc), so the position of a
@@ -201,9 +209,32 @@ constexpr int kRpnFusedMaxK = 4096;
 int rpn_select_fused(const RpnArgs& a, float4* seg_boxes, float* seg_scores, int32_t* seg_count,
                      unsigned long long* nms_in_total, cudaStream_t st);
 // ... and ONE cluster launch (one cluster per image, one CTA per level) sweeps every segment's suppression mask and
-// merges each image's levels (top `post`, zero padded).
+// merges each image's levels (top `post`, zero padded).  skip (device [N], optional): images with skip[n] != 0 are
+// left alone (their clusters return before the first cluster barrier).
 int rpn_sweep_merge_fused(const RpnArgs& a, const int32_t* seg_count, const unsigned long long* mask,
                           const float4* seg_boxes, const float* seg_scores, float4* out_boxes, float* out_logits,
-                          uint8_t* out_valid, int32_t* out_num, cudaStream_t st);
+                          uint8_t* out_valid, int32_t* out_num, const int32_t* skip, cudaStream_t st);
+
+// Capped walk in merge order (rpn_fused.cu): one CTA per image visits the image's candidates 64 at a time in the order
+// of the final merge (score desc, level asc, position asc), tests each only against the kept boxes of its own level,
+// and stops at `post` kept.  Same result as per-level NMS + merge: a box's fate depends only on the higher-ranked
+// boxes of its level, and a level's survivors past the image's first `post` are never output.
+// An image that finishes within kRpnLazyMaxBlocks blocks writes its outputs and done[n] = 1; one that does not writes
+// done[n] = 0 and nothing else, and the mask + sweep-merge launches (which skip the finished images) produce it.
+// 64 blocks = 4,096 candidates; the bench's inputs need 16 per image, the clustered ones 21-22 (tools/rpn_lazy_visits.py).
+constexpr int kRpnLazyMaxBlocks = 64;
+// Dynamic shared memory of the walk (keys, merge order, per-level kept boxes); the walk runs when it is at most
+// kRpnLazyMaxSmem bytes, else the image goes straight to masks + sweep-merge.
+constexpr size_t kRpnLazyMaxSmem = 200 * 1024;
+// The walk keeps one SM busy per image for about 140 us (B200, bench inputs; DESIGN.md section 6 breaks it down), longer
+// than masks + sweep-merge take for one image on the whole machine (about 40 us), so it only pays when other work
+// fills the other SMs: batches of at least kRpnLazyMinImages images (bench.py's 4-image blocks, 4 graphs in flight:
+// 0.505 -> 0.451 ms per step).  Smaller batches (a single image: 0.139 -> 0.255 ms for configs[0] with the walk) keep
+// masks + sweep-merge.
+constexpr int kRpnLazyMinImages = 4;
+size_t rpn_lazy_merge_smem(const RpnArgs& a);
+int rpn_lazy_merge_fused(const RpnArgs& a, const int32_t* seg_count, const float4* seg_boxes, const float* seg_scores,
+                         float thr, float4* out_boxes, float* out_logits, uint8_t* out_valid, int32_t* out_num,
+                         int32_t* done, cudaStream_t st);
 
 }  // namespace d2b

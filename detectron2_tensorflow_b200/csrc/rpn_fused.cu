@@ -687,8 +687,10 @@ __global__ void __launch_bounds__(kSelThreads, D2B_SEL_MINB) rpn_select_kernel(R
 // straight to their output slots.  No sort, no intermediate buffers, no last-block hand-off.
 __global__ void __launch_bounds__(kColSweepThreads) rpn_sweep_merge_kernel(
     RpnArgs a, const int32_t* seg_count, int W, int cap, const u64* mask, const float4* seg_boxes,
-    const float* seg_scores, float4* out_boxes, float* out_logits, uint8_t* out_valid, int32_t* out_num) {
+    const float* seg_scores, float4* out_boxes, float* out_logits, uint8_t* out_valid, int32_t* out_num,
+    const int32_t* skip) {
   grid_dep_sync();
+  if (skip && skip[blockIdx.x / a.L]) return;  // the whole cluster (= image), before its first barrier
   extern __shared__ uint32_t s_keys[];  // [L][cap] score keys of every level's survivors, then [cap] u16 positions
   __shared__ int s_cnt;
   __shared__ int s_off[D2B_MAX_LEVELS + 1];
@@ -761,7 +763,284 @@ __global__ void __launch_bounds__(kColSweepThreads) rpn_sweep_merge_kernel(
 
 size_t select_smem_bytes(int P) { return kSelOffRaw + 2 * (size_t)P * sizeof(u64); }
 
+// ------------------------------------------------------------------ capped walk in merge order (rpn.cuh)
+constexpr int kLazyThreads = 1024;  // 16 threads per candidate of a 64-candidate block
+constexpr int kLazyChunk = 1024;    // merge ranks are computed for this many positions of every level at a time
+
+// Candidates (kcap) and kept boxes (vcap) level l can hold.
+__host__ __device__ __forceinline__ void lazy_level(const RpnArgs& a, int l, int& kcap, int& vcap) {
+  kcap = (int)(a.hwa[l] < (long long)a.k ? a.hwa[l] : (long long)a.k);
+  vcap = a.post < kcap ? a.post : kcap;
+}
+
+__host__ __device__ __forceinline__ LazyLayout lazy_layout(const RpnArgs& a) {
+  int KT = 0, VT = 0;
+  for (int l = 0; l < a.L; ++l) {
+    int kc, vc;
+    lazy_level(a, l, kc, vc);
+    KT += kc;
+    VT += vc;
+  }
+  LazyLayout g;
+  g.R = KT < kRpnLazyMaxBlocks * 64 ? KT : kRpnLazyMaxBlocks * 64;
+  const int ids = a.post < KT ? a.post : KT;
+  // [kept canonical boxes VT float4][chunk canonical boxes kLazyChunk float4][keys KT u32][order R u32][ids u32]
+  g.o_cbox = (size_t)VT * 16;
+  g.o_keys = g.o_cbox + (size_t)kLazyChunk * 16;
+  g.o_order = g.o_keys + (size_t)KT * 4;
+  g.o_ids = g.o_order + (size_t)g.R * 4;
+  g.bytes = g.o_ids + (size_t)ids * 4;
+  return g;
+}
+
+// One CTA per image.  The merge order is built in chunks: ranks (exactly as rpn_sweep_merge_kernel ranks survivors:
+// own position + per other level a binary search, ties to the lower level) of the positions [plo, plo + kLazyChunk)
+// of every level; since a rank is never below the position, the order is then complete up to plo + kLazyChunk.  A
+// block of 64 candidates in that order is tested against the kept boxes of each candidate's own level (16 threads per
+// candidate; a pre-test that the kept box covers a (1 - thr) shrunk span of the candidate in y and x -- implied by
+// IoU > thr, with slack for rounding -- then the exact TF rule d2b_iou > thr), the same-level pairs of the diagonal tile
+// are tested exactly, and warp 0 resolves the tile (nms_tile_resolve) and appends the kept boxes to their level lists.
+// Coordinates carry no level offset: the reference runs NMS per level on the raw boxes.
+__global__ void __launch_bounds__(kLazyThreads) rpn_lazy_merge_kernel(
+    RpnArgs a, const int32_t* seg_count, const float4* seg_boxes, const float* seg_scores, float thr,
+    float4* out_boxes, float* out_logits, uint8_t* out_valid, int32_t* out_num, int32_t* done) {
+  grid_dep_sync();
+  extern __shared__ __align__(16) unsigned char s_lz[];
+  __shared__ float4 s_can[64];  // canonical (ymin, xmin, ymax, xmax) of the block's candidates
+  __shared__ float4 s_flt[64];  // (ylo, yhi, xlo, xhi): a suppressing box must reach ylo and xlo, start by yhi and xhi
+  __shared__ int s_lvl[64];     // level, -1 past the end
+  __shared__ uint32_t s_id[64];  // level << 16 | position
+  __shared__ u64 s_diag[64];
+  __shared__ unsigned s_dead[2];
+  __shared__ int s_cnt[D2B_MAX_LEVELS], s_kc[D2B_MAX_LEVELS], s_koff[D2B_MAX_LEVELS + 1], s_voff[D2B_MAX_LEVELS + 1];
+  __shared__ int s_nk, s_total;
+  const LazyLayout g = lazy_layout(a);
+  const int R = g.R;
+  float4* s_kept = reinterpret_cast<float4*>(s_lz);                   // [voff[L]] per-level kept canonical boxes
+  float4* s_cbox = reinterpret_cast<float4*>(s_lz + g.o_cbox);        // [kLazyChunk] candidates of the current chunk
+  uint32_t* s_keys = reinterpret_cast<uint32_t*>(s_lz + g.o_keys);    // [koff[L]] score keys, per level
+  uint32_t* s_order = reinterpret_cast<uint32_t*>(s_lz + g.o_order);  // [R] merge order: level << 16 | position
+  uint32_t* s_ids = reinterpret_cast<uint32_t*>(s_lz + g.o_ids);      // [min(post, koff[L])] kept, in output order
+  const int n = blockIdx.x, tid = threadIdx.x, lane = tid & 31, L = a.L;
+  const size_t rbase = (size_t)n * L;
+  D2B_PROF(n == 0 && tid == 0, 128);  // phase stamps of image 0 (tools/phase_probe.py): 128-131, 132 + block, 200
+  if (tid == 0) {
+    s_koff[0] = 0; s_voff[0] = 0;
+    for (int l = 0; l < L; ++l) {
+      int kc, vc;
+      lazy_level(a, l, kc, vc);
+      s_cnt[l] = min(seg_count[rbase + l], kc);
+      s_kc[l] = 0;
+      s_koff[l + 1] = s_koff[l] + kc;
+      s_voff[l + 1] = s_voff[l] + vc;
+    }
+    s_nk = 0;
+  }
+  __syncthreads();
+  if (tid == 0) {
+    int t = 0;
+    for (int l = 0; l < L; ++l) t += s_cnt[l];
+    s_total = t;
+  }
+  for (int l = 0; l < L; ++l) {  // the loads of a trip are issued together
+    const int c = s_cnt[l];
+    const float* sc = seg_scores + (rbase + l) * a.k;
+    for (int p0 = 0; p0 < c; p0 += 4 * kLazyThreads) {
+      float v[4];
+#pragma unroll
+      for (int u = 0; u < 4; ++u) {
+        const int p = p0 + u * kLazyThreads + tid;
+        v[u] = p < c ? __ldg(sc + p) : 0.0f;
+      }
+#pragma unroll
+      for (int u = 0; u < 4; ++u) {
+        const int p = p0 + u * kLazyThreads + tid;
+        if (p < c) {
+          D2B_BOUND(s_koff[l] + p, s_koff[L]);
+          s_keys[s_koff[l] + p] = float_to_key(v[u]);
+        }
+      }
+    }
+  }
+  __syncthreads();
+  const bool prof = (n == 0 && tid == 0);
+  D2B_PROF(prof, 129);
+  const int total = s_total;
+  const float kf = thr * 0.999f;
+  int plo = 0, base = 0, ready = 0;  // order complete on [0, ready); s_cbox holds the candidates of [base, ready)
+  bool finished = false;
+  for (int b0 = 0;; b0 += 64) {
+    const int nk = s_nk;
+    if (nk >= a.post || b0 >= total) { finished = true; break; }
+    if (b0 >= R) break;  // visit budget spent: this image goes to masks + sweep-merge
+    if (b0 >= ready) {
+      const int phi = plo + kLazyChunk;
+      for (int l = 0; l < L; ++l) {
+        const uint32_t* kl = s_keys + s_koff[l];
+        for (int p = plo + tid; p < min(phi, s_cnt[l]); p += kLazyThreads) {
+          const uint32_t key = kl[p];
+          int rank = p;
+          for (int l2 = 0; l2 < L && rank < R; ++l2) {
+            if (l2 == l) continue;
+            const uint32_t* k2 = s_keys + s_koff[l2];
+            int lo = 0, hi = s_cnt[l2];
+            while (lo < hi) {  // first position whose element does NOT precede (key, level l)
+              const int mid = (lo + hi) >> 1;
+              const uint32_t ke = k2[mid];
+              const bool before = (l2 < l) ? (ke >= key) : (ke > key);
+              if (before) lo = mid + 1; else hi = mid;
+            }
+            rank += lo;
+          }
+          if (rank < R) s_order[rank] = ((uint32_t)l << 16) | (uint32_t)p;
+        }
+      }
+      __syncthreads();
+      D2B_PROF(prof && plo == 0, 130);
+      base = ready;
+      ready = min(min(phi, total), R);
+      plo = phi;
+      for (int q = base + tid; q < ready; q += kLazyThreads) {
+        const uint32_t id = s_order[q];
+        const int l = (int)(id >> 16), p = (int)(id & 0xffffu);
+        D2B_BOUND(l, L);
+        D2B_BOUND(p, s_cnt[l]);
+        D2B_BOUND(q - base, kLazyChunk);
+        const float4 b = __ldg(seg_boxes + (rbase + l) * a.k + p);
+        s_cbox[q - base] = make_float4(fminf(b.x, b.z), fminf(b.y, b.w), fmaxf(b.x, b.z), fmaxf(b.y, b.w));
+      }
+      __syncthreads();
+      D2B_PROF(prof && base == 0, 131);
+    }
+    const int rows = min(64, ready - b0);
+    if (tid < 64) {
+      int lv = -1;
+      uint32_t id = 0;
+      float4 c = make_float4(0, 0, 0, 0), f = c;
+      if (tid < rows) {
+        D2B_BOUND(b0 + tid, R);
+        id = s_order[b0 + tid];
+        lv = (int)(id >> 16);
+        c = s_cbox[b0 + tid - base];
+        const float h = c.z - c.x, w = c.w - c.y;
+        const float ey = 1e-6f * (fabsf(c.x) + fabsf(c.z)), ex = 1e-6f * (fabsf(c.y) + fabsf(c.w));
+        f = make_float4(c.x + kf * h - ey, c.z - kf * h + ey, c.y + kf * w - ex, c.w - kf * w + ex);
+      }
+      s_can[tid] = c; s_flt[tid] = f; s_lvl[tid] = lv; s_id[tid] = id;
+    }
+    if (tid < 2) s_dead[tid] = 0;
+    __syncthreads();
+    // candidate r against the kept boxes of its level; the two candidates of a warp stop together once both are dead
+    const int r = tid >> 4, sub = tid & 15;
+    const int lv = s_lvl[r];
+    const float4 cr = s_can[r], fr = s_flt[r];
+    const int kc = lv >= 0 ? s_kc[lv] : 0;
+    const float4* kl = s_kept + (lv >= 0 ? s_voff[lv] : 0);
+    const int kmax = max(kc, __shfl_xor_sync(0xffffffffu, kc, 16));
+    const unsigned half = (lane < 16) ? 0x0000ffffu : 0xffff0000u;
+    bool dead = false;
+    for (int j0 = 0; j0 < kmax; j0 += 16) {
+      const int j = j0 + sub;
+      bool hit = false;
+      if (j < kc && !dead) {
+        const float4 kb = kl[j];
+        if (kb.z >= fr.x && kb.x <= fr.y && kb.w >= fr.z && kb.y <= fr.w) hit = d2b_iou(cr, kb) > thr;
+      }
+      const unsigned m = __ballot_sync(0xffffffffu, hit);
+      dead = dead || (m & half) != 0;
+      if (__all_sync(0xffffffffu, dead)) break;
+    }
+    if (dead && sub == 0) atomicOr(&s_dead[r >> 5], 1u << (r & 31));
+    // diagonal tile: bit c of row r = candidate r suppresses candidate c (c > r, same level)
+    u64 bits = 0;
+    if (lv >= 0)
+      for (int c = r + 1 + sub; c < rows; c += 16)
+        if (s_lvl[c] == lv && d2b_iou(cr, s_can[c]) > thr) bits |= 1ull << c;
+#pragma unroll
+    for (int o = 8; o > 0; o >>= 1) bits |= __shfl_xor_sync(0xffffffffu, bits, o);
+    if (sub == 0) s_diag[r] = bits;
+    __syncthreads();
+    if (tid < 32) {
+      u64 rem = ((u64)s_dead[1] << 32) | (u64)s_dead[0];
+      if (rows < 64) rem |= ~0ull << rows;
+      const u64 K = nms_tile_resolve(s_diag[lane], s_diag[lane + 32], rem, a.post - nk);
+      const u64 bitA = 1ull << lane, bitB = 1ull << (lane + 32);
+      const int lA = s_lvl[lane], lB = s_lvl[lane + 32];
+      u64 sameA = 0, sameB = 0;
+      int mine = 0;  // lane l < L: boxes of level l kept in this block
+      for (int l = 0; l < L; ++l) {
+        const u64 m = ((u64)__ballot_sync(0xffffffffu, lB == l) << 32) | __ballot_sync(0xffffffffu, lA == l);
+        if (lA == l) sameA = m;
+        if (lB == l) sameB = m;
+        if (lane == l) mine = __popcll(K & m);
+      }
+      if (K & bitA) {
+        const int slot = s_kc[lA] + __popcll(K & sameA & (bitA - 1ull)), o = nk + __popcll(K & (bitA - 1ull));
+        D2B_BOUND(slot, s_voff[lA + 1] - s_voff[lA]);
+        D2B_BOUND(o, a.post);
+        s_kept[s_voff[lA] + slot] = s_can[lane];
+        s_ids[o] = s_id[lane];
+      }
+      if (K & bitB) {
+        const int slot = s_kc[lB] + __popcll(K & sameB & (bitB - 1ull)), o = nk + __popcll(K & (bitB - 1ull));
+        D2B_BOUND(slot, s_voff[lB + 1] - s_voff[lB]);
+        D2B_BOUND(o, a.post);
+        s_kept[s_voff[lB] + slot] = s_can[lane + 32];
+        s_ids[o] = s_id[lane + 32];
+      }
+      __syncwarp();
+      if (lane < L) s_kc[lane] += mine;
+      if (lane == 0) s_nk = nk + __popcll(K);
+    }
+    __syncthreads();
+    D2B_PROF(prof, 132 + (b0 >> 6));
+  }
+  if (!finished) {
+    if (tid == 0) done[n] = 0;
+    return;
+  }
+  // outputs as rpn_sweep_merge_kernel writes them: the kept boxes in merge order, then zero padding (:101-114)
+  const int nk = s_nk;
+  for (int o = tid; o < a.post; o += kLazyThreads) {
+    float4 box = make_float4(0, 0, 0, 0);
+    float logit = 0.0f;
+    uint8_t valid = 0;
+    if (o < nk) {
+      const uint32_t id = s_ids[o];
+      const size_t src = (rbase + (id >> 16)) * a.k + (id & 0xffffu);
+      box = seg_boxes[src];
+      logit = seg_scores[src];
+      valid = 1;
+    }
+    const size_t dst = (size_t)n * a.post + o;
+    out_boxes[dst] = box;
+    out_logits[dst] = logit;
+    out_valid[dst] = valid;
+  }
+  if (tid == 0) {
+    if (out_num) out_num[n] = nk;
+    done[n] = 1;
+  }
+  D2B_PROF(prof, 200);
+}
+
 }  // namespace
+
+size_t rpn_lazy_merge_smem(const RpnArgs& a) { return lazy_layout(a).bytes; }
+
+int rpn_lazy_merge_fused(const RpnArgs& a, const int32_t* seg_count, const float4* seg_boxes, const float* seg_scores,
+                         float thr, float4* out_boxes, float* out_logits, uint8_t* out_valid, int32_t* out_num,
+                         int32_t* done, cudaStream_t st) {
+  D2B_REQUIRE(a.k <= kRpnFusedMaxK && a.L <= D2B_MAX_LEVELS, "lazy merge: k=%d, L=%d out of range", a.k, a.L);
+  const size_t smem = rpn_lazy_merge_smem(a);
+  D2B_REQUIRE(smem <= kRpnLazyMaxSmem, "lazy merge: %zu bytes of shared memory > %zu", smem, kRpnLazyMaxSmem);
+  if (a.N == 0) return D2B_OK;
+  D2B_CUDA(allow_dynamic_smem(rpn_lazy_merge_kernel, smem));
+  D2B_CUDA(launch_pdl(rpn_lazy_merge_kernel, dim3((unsigned)a.N), dim3(kLazyThreads), smem, st, 0, a, seg_count,
+                      seg_boxes, seg_scores, thr, out_boxes, out_logits, out_valid, out_num, done));
+  D2B_LAUNCH_CHECK();
+  return D2B_OK;
+}
 
 int rpn_select_fused(const RpnArgs& a, float4* seg_boxes, float* seg_scores, int32_t* seg_count,
                      unsigned long long* nms_in_total, cudaStream_t st) {
@@ -780,7 +1059,7 @@ int rpn_select_fused(const RpnArgs& a, float4* seg_boxes, float* seg_scores, int
 
 int rpn_sweep_merge_fused(const RpnArgs& a, const int32_t* seg_count, const unsigned long long* mask,
                           const float4* seg_boxes, const float* seg_scores, float4* out_boxes, float* out_logits,
-                          uint8_t* out_valid, int32_t* out_num, cudaStream_t st) {
+                          uint8_t* out_valid, int32_t* out_num, const int32_t* skip, cudaStream_t st) {
   const int rows = a.L * a.N;
   if (rows == 0) return D2B_OK;
   const int W = (a.k + 63) / 64;
@@ -792,7 +1071,7 @@ int rpn_sweep_merge_fused(const RpnArgs& a, const int32_t* seg_count, const unsi
   // one cluster per image (L <= D2B_MAX_LEVELS = 8: portable size)
   D2B_CUDA(launch_pdl(rpn_sweep_merge_kernel, dim3((unsigned)rows, 1, 1), dim3(kColSweepThreads, 1, 1), smem, st,
                       (unsigned)a.L, a, seg_count, W, cap, reinterpret_cast<const u64*>(mask), seg_boxes, seg_scores,
-                      out_boxes, out_logits, out_valid, out_num));
+                      out_boxes, out_logits, out_valid, out_num, skip));
   D2B_LAUNCH_CHECK();
   return D2B_OK;
 }

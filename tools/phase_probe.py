@@ -1,6 +1,10 @@
 """Phase timeline of the fused RPN kernels (debug build only: D2B_EXTRA_NVCC=-DD2B_PROFILE python -m
 detectron2_tensorflow_b200.build --force).  Prints the %globaltimer deltas (us) recorded by cluster 0 of
-rpn_select_kernel (the P2 row of image 0) and by segment 0 of rpn_sweep_merge_kernel."""
+rpn_select_kernel (the P2 row of image 0), by segment 0 of rpn_sweep_merge_kernel and, with N >= 4 images (the walk
+runs), by image 0 of rpn_lazy_merge_kernel: keys loaded, merge ranks of the first chunk, its boxes gathered, and the
+end of every 64-candidate block.
+
+    python tools/phase_probe.py [N]"""
 import ctypes as C
 import os
 import sys
@@ -40,3 +44,9 @@ for it in range(3):
     print(f"   merge (since sweep start): lists exchanged={(t[20] - t[16]) / 1e3:.1f} written={(t[18] - t[16]) / 1e3:.1f}")
     blk = t[32:64]
     print("   block publish times (us since sweep start): " + " ".join(f"{(b - t[16]) / 1e3:.1f}" for b in blk))
+    if t[128] and t[200] >= t[128]:
+        blocks = [(t[132 + b] - t[128]) / 1e3 for b in range(64) if t[132 + b] >= t[128] and t[132 + b] <= t[200]]
+        steps = np.diff([(t[131] - t[128]) / 1e3] + blocks)
+        print("   walk (image 0), us since start: keys={:.1f} ranks={:.1f} gathered={:.1f} blocks={} end={:.1f}".format(
+            *[(t[i] - t[128]) / 1e3 for i in (129, 130, 131)], len(blocks), (t[200] - t[128]) / 1e3))
+        print("   per block (us): " + " ".join(f"{x:.2f}" for x in steps))

@@ -1,5 +1,11 @@
-"""Timing of the RPN proposal stage alone (d2b_rpn_proposals: select / sort / decode -> NMS masks -> sweep + merge)
-at config-2 sizes (2000 pre / 1000 post), for N = 16, 2 and 1 images; CUDA events, median, L2 flushed or warm."""
+"""Timing of the RPN proposal stage alone (d2b_rpn_proposals: select / sort / decode -> capped walk in merge order ->
+NMS masks + sweep-merge for the images the walk does not finish) at config-2 sizes (2000 pre / 1000 post), for N = 16,
+4 and 1 images (the walk runs from 4 images on); CUDA events, median, L2 flushed or warm.  Variant "whole-image": the
+gaussian logits with every box grown past the image (clamped size deltas), so that all boxes clip to the whole image
+and each level keeps one box: the walk visits every candidate, spends its budget, and every image goes to masks +
+sweep-merge (its worst case).
+
+    python tools/rpn_probe.py [--images 16,4,1] [--variants gaussian,clustered,ties,whole-image]"""
 import argparse
 import json
 import os
@@ -16,8 +22,8 @@ from detectron2_tensorflow_b200.utils import synthetic as syn
 
 ap = argparse.ArgumentParser()
 ap.add_argument("--iters", type=int, default=20)
-ap.add_argument("--images", default="16,2,1")
-ap.add_argument("--variants", default="gaussian,clustered,ties")
+ap.add_argument("--images", default="16,4,1")
+ap.add_argument("--variants", default="gaussian,clustered,ties,whole-image")
 ap.add_argument("--once", action="store_true", help="one call per case, no timing (ncu launch lists)")
 args = ap.parse_args()
 dev = torch.device("cuda", 0)
@@ -44,8 +50,11 @@ def timeit(fn, cold):
 
 
 for variant in args.variants.split(","):
-    seed = {"gaussian": 2, "clustered": 3, "ties": 4}[variant]
-    logits, deltas = syn.rpn_inputs(16, seed=seed, variant=variant, anchors=anchors)
+    seed = {"gaussian": 2, "clustered": 3, "ties": 4, "whole-image": 2}[variant]
+    logits, deltas = syn.rpn_inputs(16, seed=seed, variant=variant.replace("whole-image", "gaussian"), anchors=anchors)
+    if variant == "whole-image":
+        for d in deltas:
+            d[..., 2:] = 8.0  # above the scale clamp: every box 62x its anchor, clipped to the image
     for N in [int(v) for v in args.images.split(",")]:
         tl = [torch.from_numpy(x[:N]).to(dev) for x in logits]
         td = [torch.from_numpy(x[:N]).to(dev) for x in deltas]
