@@ -695,10 +695,14 @@ int frcnn_plan(const d2b_fast_rcnn_params* p, FrcnnPlan& pl) {
   D2B_REQUIRE(p->num_bbox_reg_classes == 1 || p->num_bbox_reg_classes == p->num_classes,
               "fast_rcnn: boxes must be [M,4] or [M,K*4] (Kb=%d, K=%d)", p->num_bbox_reg_classes, p->num_classes);
   D2B_REQUIRE(p->topk_per_image >= 1, "fast_rcnn: topk_per_image must be >= 1");
+  // as tf.image.non_max_suppression; checked here, before the first launch, like the NMS sizes below
+  D2B_REQUIRE(p->nms_thresh >= 0.0f && p->nms_thresh <= 1.0f, "nms_thresh must be in [0, 1]");
   const long long cmax = (long long)p->rmax * p->num_classes;
   D2B_REQUIRE(cmax < (1ll << 30), "fast_rcnn: Rmax*K too large");
   pl.stride = (int)(cmax > 0 ? cmax : 1);
   pl.P = pad_pow2(pl.stride);
+  const int rc = nms_check_sizes(pl.stride, p->topk_per_image);
+  if (rc != D2B_OK) return rc;
   const size_t N = p->num_images;
   size_t o = 0;
   pl.o_keys = o; o += ws_slice(N * pl.P * sizeof(u64));
@@ -796,6 +800,8 @@ int retina_plan(const d2b_retinanet_params* p, RetinaPlan& pl) {
   D2B_REQUIRE(p->topk_candidates >= 1 && p->topk_candidates <= kTopkMaxK, "topk_candidates=%d out of [1,%d]",
               p->topk_candidates, kTopkMaxK);
   D2B_REQUIRE(p->max_detections >= 1, "max_detections must be >= 1");
+  // as tf.image.non_max_suppression; checked here, before the first launch, like the NMS sizes below
+  D2B_REQUIRE(p->nms_thresh >= 0.0f && p->nms_thresh <= 1.0f, "nms_thresh must be in [0, 1]");
   RetinaArgs& a = pl.a;
   TopkDesc& td = pl.td;
   long long maxhwa = 0;
@@ -828,6 +834,8 @@ int retina_plan(const d2b_retinanet_params* p, RetinaPlan& pl) {
   a.P = topk_padded_k(a.k);
   a.stride = a.L * a.k;
   a.P3 = pad_pow2(a.stride);
+  const int rc = nms_check_sizes(a.stride, p->max_detections);
+  if (rc != D2B_OK) return rc;
   td.G = a.L; td.rows_per_group = a.N; td.k = a.k; td.transform = D2B_TOPK_SIGMOID;
   pl.rows = a.L * a.N;
   const size_t rows = pl.rows, N = a.N;
@@ -940,9 +948,13 @@ int yolo_plan(const d2b_yolo_params* p, YoloPlan& pl) {
   D2B_REQUIRE(p->num_images <= 65535, "yolo: too many images");
   D2B_REQUIRE(p->num_classes >= 1, "yolo: num_classes must be >= 1");
   D2B_REQUIRE(p->post_nms_topk >= 1, "yolo: post_nms_topk must be >= 1");
+  // as tf.image.non_max_suppression; checked here, before the first launch, like the NMS sizes below
+  D2B_REQUIRE(p->nms_thresh >= 0.0f && p->nms_thresh <= 1.0f, "nms_thresh must be in [0, 1]");
   D2B_REQUIRE(p->num_boxes < (1 << 30), "yolo: num_boxes too large");
   const size_t N = p->num_images, n = p->num_boxes > 0 ? p->num_boxes : 1;
   pl.P = pad_pow2((long long)n);
+  const int rc = nms_check_sizes((int)n, p->post_nms_topk);
+  if (rc != D2B_OK) return rc;
   size_t o = 0;
   pl.o_keys = o; o += ws_slice(N * pl.P * sizeof(u64));
   pl.o_count = o; o += ws_slice(N * sizeof(int32_t));
