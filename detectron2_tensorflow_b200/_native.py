@@ -190,7 +190,8 @@ class SoloUpsampleParams(C.Structure):
 
 
 class RoiAlignBackwardParams(C.Structure):
-    _fields_ = [("fwd", RoiAlignParams), ("grad_out", _vp), ("grad_features", _vp * MAX_LEVELS)]
+    _fields_ = [("fwd", RoiAlignParams), ("grad_out", _vp), ("grad_features", _vp * MAX_LEVELS),
+                ("deterministic", _i32)]
 
 
 # op name -> params struct; every op exports d2b_<op> and d2b_<op>_workspace_bytes

@@ -18,6 +18,8 @@
 // HBM-bound gather: no contraction, so no tensor cores.
 #include <cuda_bf16.h>
 
+#include <climits>
+
 #include "common.cuh"
 
 namespace d2b {
@@ -87,10 +89,9 @@ __device__ __forceinline__ int level_of(float y1, float x1, float y2, float x2, 
   return lvl - min_level;
 }
 
-// functional.py:128-160 + TF CropAndResize coordinate rule for sample `s` of `cs`
+// functional.py:128-160 + TF CropAndResize coordinate rule: position (in padded pixels) of sample `s` of `cs`
 // along an axis of (padded) extent P; lo/hi are the scaled (+pad) box edges.
-__device__ __forceinline__ Tap make_tap(float lo, float hi, int s, int cs, int P, int pad,
-                                        int dim, int aligned, int stride) {
+__device__ __forceinline__ float sample_coord(float lo, float hi, int s, int cs, int P, int aligned) {
   float n1, n2;
   if (aligned) {
     float sp = (hi - lo) / (float)cs;
@@ -113,6 +114,12 @@ __device__ __forceinline__ Tap make_tap(float lo, float hi, int s, int cs, int P
   } else {
     in = 0.5f * (n1 + n2) * (float)(P - 1);
   }
+  return in;
+}
+
+__device__ __forceinline__ Tap make_tap(float lo, float hi, int s, int cs, int P, int pad,
+                                        int dim, int aligned, int stride) {
+  const float in = sample_coord(lo, hi, s, cs, P, aligned);
   Tap t;
   t.valid = (in >= 0.0f && in <= (float)(P - 1)) ? 1 : 0;
   const float f = floorf(in);
@@ -414,6 +421,230 @@ __global__ void __launch_bounds__(kThreads) roi_align_backward_kernel(const RoiA
   }
 }
 
+// ---------------------------------------------------------------------------------------------
+// Deterministic backward: the CPU kernel's summation order, bit for bit, without floating-point atomics.
+// Per level and image, a zeroed padded gradient receives, ROI by ROI in input order, crop row y by crop row, column
+// x by column, the TL, TR, BL, BR products of each sample; then each padded pixel is added onto clamp(p - pad) in
+// raster order.  Every padded accumulator is owned by one thread, which pulls its contributions in that order:
+//   roi_align_grad_bin_kernel        thread per ROI: (level, image) key, padded footprint, sample taps
+//   roi_align_grad_partition_kernel  CTA per (level, image): its ROI indices in input order (ballot compaction)
+//   roi_align_grad_accum_kernel      CTA per (level, image, 8x8 destination tile, 128 channels): warp per padded
+//                                    row, lane per 16-byte channel group; walks the key's ROI list, then folds
+constexpr int kGradTile = 8;                   // destination tile edge (un-padded pixels)
+constexpr int kGradRows = kGradTile + 2;       // + the border row / column of each side that folds onto an edge tile
+constexpr int kGradThreads = 32 * kGradRows;   // warp w owns padded row w of the tile
+constexpr int kGradChannels = 32 * 4;          // channels per accumulate CTA (one float4 per lane)
+constexpr int kBinThreads = 256;
+constexpr int kPartThreads = 1024;
+
+struct GTap {  // one crop row / column of one ROI, padded coordinates
+  int p;       // floor of the sample position; -1 => outside [0, P-1] (the sample contributes nothing)
+  float w;     // position - p; the ceil neighbour is p + (w != 0)
+};
+
+struct GradDetArgs {
+  RoiAlignGradArgs g;
+  int* key;      // [M] level * N + image, -1 => no contribution
+  int4* rect;    // [M] padded footprint: rows y0..y1, columns x0..x1 (inclusive)
+  int* list;     // [M] ROI indices grouped by key, input order inside a key
+  int2* range;   // [L * N] [begin, end) of each key in `list`
+  GTap* taps;    // [M, ch + cw]
+  long long tile_start[D2B_MAX_LEVELS + 1];  // first accumulate CTA of each level
+  int tiles_x[D2B_MAX_LEVELS], tiles_y[D2B_MAX_LEVELS];
+};
+
+__global__ void __launch_bounds__(kBinThreads) roi_align_grad_bin_kernel(const GradDetArgs d) {
+  const RoiAlignArgs& a = d.g.f;
+  const long long roi = (long long)blockIdx.x * kBinThreads + threadIdx.x;
+  if (roi >= a.M) return;
+  const int s1 = a.sr > 0 ? a.sr : 1;
+  const int ch = a.oh * s1, cw = a.ow * s1;
+  const float4 b = __ldg(reinterpret_cast<const float4*>(a.boxes) + roi);
+  int lvl = 0;
+  if (a.L > 1) lvl = level_of(b.x, b.y, b.z, b.w, a.min_level, a.max_level, a.canon_size, a.canon_level);
+  D2B_BOUND(lvl, a.L);
+  const Level L = a.lv[lvl];
+  const float padf = a.pad ? 1.0f : 0.0f;
+  GTap* tap = d.taps + (size_t)roi * (ch + cw);
+  int lo[2] = {INT_MAX, INT_MAX}, hi[2] = {-1, -1};
+  for (int t = 0; t < ch + cw; ++t) {
+    const int ax = t < ch ? 0 : 1;
+    const float e0 = ax ? b.y : b.x, e1 = ax ? b.w : b.z;
+    const float elo = e0 * L.scale + padf, ehi = e1 * L.scale + padf;
+    const int cs = ax ? cw : ch, P = (ax ? L.W : L.H) + 2 * a.pad;
+    const float in = sample_coord(elo, ehi, ax ? t - ch : t, cs, P, a.aligned);
+    GTap g{-1, 0.0f};
+    if (in >= 0.0f && in <= (float)(P - 1)) {
+      const float f = floorf(in);
+      g.p = (int)f;
+      g.w = in - f;
+      lo[ax] = min(lo[ax], g.p);
+      hi[ax] = max(hi[ax], g.p + (g.w != 0.0f ? 1 : 0));
+    }
+    tap[t] = g;
+  }
+  const long long img = a.bidx64 ? reinterpret_cast<const long long*>(a.bidx)[roi * a.bidx_stride]
+                                 : (long long)reinterpret_cast<const int*>(a.bidx)[roi * a.bidx_stride];
+  const bool live = img >= 0 && img < a.N && hi[0] >= 0 && hi[1] >= 0;  // TF skips out-of-range box_ind
+  d.key[roi] = live ? lvl * a.N + (int)img : -1;
+  d.rect[roi] = make_int4(lo[0], hi[0], lo[1], hi[1]);
+}
+
+__global__ void __launch_bounds__(kPartThreads) roi_align_grad_partition_kernel(const GradDetArgs d) {
+  __shared__ int s_warp[kPartThreads / 32];
+  const int key = blockIdx.x;
+  const int M = (int)d.g.f.M;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  int begin = 0;  // ROIs of smaller keys
+  for (int b0 = 0; b0 < M; b0 += kPartThreads) {
+    const int i = b0 + tid;
+    int k = -1;
+    if (i < M) k = d.key[i];
+    begin += __syncthreads_count(k >= 0 && k < key);
+  }
+  int pos = begin;
+  for (int b0 = 0; b0 < M; b0 += kPartThreads) {
+    const int i = b0 + tid;
+    const bool hit = i < M && d.key[i] == key;
+    const unsigned m = __ballot_sync(0xffffffffu, hit);
+    if (lane == 0) s_warp[warp] = __popc(m);
+    __syncthreads();
+    int before = 0, total = 0;
+    for (int w = 0; w < kPartThreads / 32; ++w) {
+      const int c = s_warp[w];
+      before += w < warp ? c : 0;
+      total += c;
+    }
+    if (hit) {
+      const int o = pos + before + __popc(m & ((1u << lane) - 1u));
+      D2B_BOUND(o, M);
+      d.list[o] = i;
+    }
+    pos += total;
+    __syncthreads();
+  }
+  if (tid == 0) d.range[key] = make_int2(begin, pos);
+}
+
+__device__ __forceinline__ float4 f4_scale(float s, float4 v) { return make_float4(s * v.x, s * v.y, s * v.z, s * v.w); }
+__device__ __forceinline__ void f4_acc(float4& a, float4 v) {
+  a.x = a.x + v.x; a.y = a.y + v.y; a.z = a.z + v.z; a.w = a.w + v.w;
+}
+
+__global__ void __launch_bounds__(kGradThreads) roi_align_grad_accum_kernel(const GradDetArgs d) {
+  const RoiAlignArgs& a = d.g.f;
+  long long t = blockIdx.x;
+  int lvl = 0;
+  while (lvl + 1 < a.L && t >= d.tile_start[lvl + 1]) ++lvl;
+  t -= d.tile_start[lvl];
+  const int tx_n = d.tiles_x[lvl], per_img = tx_n * d.tiles_y[lvl];
+  const int img = (int)(t / per_img);
+  const int tr = (int)(t - (long long)img * per_img);
+  const int ty = tr / tx_n, tx = tr - ty * tx_n;
+  D2B_BOUND(img, a.N);
+  const int2 rg = d.range[lvl * a.N + img];
+  if (rg.x == rg.y) return;  // no ROI on this level and image
+  const Level L = a.lv[lvl];
+  const int pad = a.pad, C = a.C;
+  // padded rows [py0, py1) and columns [px0, px1) whose fold lands in this tile
+  const int sy0 = ty * kGradTile, sy1 = min(sy0 + kGradTile, L.H);
+  const int sx0 = tx * kGradTile, sx1 = min(sx0 + kGradTile, L.W);
+  const int py0 = sy0 == 0 ? 0 : sy0 + pad, py1 = sy1 == L.H ? L.H + 2 * pad : sy1 + pad;
+  const int px0 = sx0 == 0 ? 0 : sx0 + pad, px1 = sx1 == L.W ? L.W + 2 * pad : sx1 + pad;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int py = py0 + warp;
+  const bool row_live = py < py1;
+  const int c = (blockIdx.y * 32 + lane) * 4;  // this lane's channel group
+  const bool grp_live = c < C;
+  const int s1 = a.sr > 0 ? a.sr : 1;
+  const int ch = a.oh * s1, cw = a.ow * s1;
+  const float cnt = (float)(s1 * s1);
+
+  float4 acc[kGradRows];
+#pragma unroll
+  for (int j = 0; j < kGradRows; ++j) acc[j] = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+  int touched = 0;
+  if (row_live) {
+    for (int b0 = rg.x; b0 < rg.y; b0 += 32) {
+      const int i = b0 + lane;
+      int roi = -1;
+      bool hit = false;
+      if (i < rg.y) {
+        D2B_BOUND(i, a.M);
+        roi = d.list[i];
+        D2B_BOUND(roi, a.M);
+        const int4 r = d.rect[roi];
+        hit = r.x <= py && py <= r.y && r.z < px1 && r.w >= px0;
+      }
+      unsigned m = __ballot_sync(0xffffffffu, hit);
+      while (m) {  // ROIs of this chunk, in input order
+        const int src = __ffs(m) - 1;
+        m &= m - 1;
+        const int r = __shfl_sync(0xffffffffu, roi, src);
+        touched = 1;
+        const GTap* tap_y = d.taps + (size_t)r * (ch + cw);
+        const GTap* tap_x = tap_y + ch;
+        const float* gro = d.g.grad_out + (size_t)r * a.oh * a.ow * C + c;
+        for (int y = 0; y < ch; ++y) {
+          const GTap ty_ = tap_y[y];
+          if (ty_.p < 0) continue;
+          const int top = ty_.p, bot = ty_.p + (ty_.w != 0.0f ? 1 : 0);
+          if (top != py && bot != py) continue;
+          const float ly = ty_.w, omy = 1.0f - ly;
+          for (int x = 0; x < cw; ++x) {
+            const GTap tx_ = tap_x[x];
+            if (tx_.p < 0) continue;
+            const int left = tx_.p, right = tx_.p + (tx_.w != 0.0f ? 1 : 0);
+            if (right < px0 || left >= px1) continue;
+            if (!grp_live) continue;
+            const float lx = tx_.w, omx = 1.0f - lx;
+            const size_t bin = (size_t)(y / s1) * a.ow + x / s1;
+            D2B_BOUND(bin, (size_t)a.oh * a.ow);
+            float4 gv = __ldg(reinterpret_cast<const float4*>(gro + bin * C));
+            if (s1 > 1) { gv.x = gv.x / cnt; gv.y = gv.y / cnt; gv.z = gv.z / cnt; gv.w = gv.w / cnt; }
+            const float4 dtop = f4_scale(omy, gv), dbot = f4_scale(ly, gv);
+            const int jl = left - px0, jr = right - px0;
+#pragma unroll
+            for (int j = 0; j < kGradRows; ++j) {
+              if (j != jl && j != jr) continue;  // warp-uniform
+              if (top == py) {
+                if (j == jl) f4_acc(acc[j], f4_scale(omx, dtop));
+                if (j == jr) f4_acc(acc[j], f4_scale(lx, dtop));
+              }
+              if (bot == py) {
+                if (j == jl) f4_acc(acc[j], f4_scale(omx, dbot));
+                if (j == jr) f4_acc(acc[j], f4_scale(lx, dbot));
+              }
+            }
+          }
+        }
+      }
+    }
+  }
+  // Fold (MirrorPadGrad): padded rows reach their un-padded row in ascending order -- one barrier-separated phase
+  // per rank inside the fold group (rank 2 only when H == 1); columns in ascending order inside a thread.  Only
+  // tiles some ROI reaches are written.
+  if (!__syncthreads_or(touched)) return;
+  const int sy = min(max(py - pad, 0), L.H - 1);
+  const int rank = py - (sy == 0 ? 0 : sy + pad);
+  float* grow = d.g.grad[lvl] + ((size_t)img * L.H + sy) * L.W * C + c;
+  for (int ph = 0; ph < 3; ++ph) {
+    if (row_live && grp_live && rank == ph) {
+#pragma unroll
+      for (int j = 0; j < kGradRows; ++j) {
+        if (px0 + j >= px1) break;
+        const int sx = min(max(px0 + j - pad, 0), L.W - 1);
+        D2B_BOUND((size_t)sy * L.W + sx, (size_t)L.H * L.W);
+        float4* q = reinterpret_cast<float4*>(grow + (size_t)sx * C);
+        float4 v = *q;
+        f4_acc(v, acc[j]);
+        *q = v;
+      }
+    }
+    __syncthreads();
+  }
+}
+
 template <typename TIn, typename TOut>
 int launch(const RoiAlignArgs& a, cudaStream_t st) {
   constexpr int E = Vec<TIn>::kElems;
@@ -503,9 +734,57 @@ extern "C" int d2b_roi_align_multilevel(const d2b_roi_align_params* p, void* /*w
   return launch<__nv_bfloat16, __nv_bfloat16>(a, st);
 }
 
-extern "C" size_t d2b_roi_align_backward_workspace_bytes(const d2b_roi_align_backward_params*) { return 0; }
+static size_t ws_align(size_t n) { return (n + 255) & ~(size_t)255; }
 
-extern "C" int d2b_roi_align_backward(const d2b_roi_align_backward_params* p, void*, size_t, d2b_stream_t stream) {
+// deterministic mode: key, rect, list, range and tap arrays, each 256-byte aligned; 0 when there is nothing to do
+extern "C" size_t d2b_roi_align_backward_workspace_bytes(const d2b_roi_align_backward_params* p) {
+  if (p == nullptr || !p->deterministic) return 0;
+  const d2b_roi_align_params& f = p->fwd;
+  if (f.num_rois <= 0 || f.num_levels < 1 || f.num_levels > D2B_MAX_LEVELS || f.num_images <= 0 ||
+      f.output_h <= 0 || f.output_w <= 0 || f.sampling_ratio < 0)
+    return 0;
+  const size_t M = (size_t)f.num_rois;
+  const size_t s1 = f.sampling_ratio > 0 ? (size_t)f.sampling_ratio : 1;
+  const size_t taps = s1 * ((size_t)f.output_h + (size_t)f.output_w);
+  return ws_align(M * sizeof(int)) + ws_align(M * sizeof(int4)) + ws_align(M * sizeof(int)) +
+         ws_align((size_t)f.num_levels * f.num_images * sizeof(int2)) + ws_align(M * taps * sizeof(GTap));
+}
+
+static int launch_backward_deterministic(const RoiAlignGradArgs& g, void* workspace, cudaStream_t st) {
+  const RoiAlignArgs& a = g.f;
+  GradDetArgs d;
+  d.g = g;
+  const size_t M = (size_t)a.M;
+  char* w = static_cast<char*>(workspace);
+  d.key = reinterpret_cast<int*>(w); w += ws_align(M * sizeof(int));
+  d.rect = reinterpret_cast<int4*>(w); w += ws_align(M * sizeof(int4));
+  d.list = reinterpret_cast<int*>(w); w += ws_align(M * sizeof(int));
+  d.range = reinterpret_cast<int2*>(w); w += ws_align((size_t)a.L * a.N * sizeof(int2));
+  d.taps = reinterpret_cast<GTap*>(w);
+  long long tiles = 0;
+  for (int l = 0; l < D2B_MAX_LEVELS; ++l) {
+    d.tile_start[l] = tiles;
+    d.tiles_y[l] = d.tiles_x[l] = 1;
+    if (l < a.L) {
+      d.tiles_y[l] = (a.lv[l].H + kGradTile - 1) / kGradTile;
+      d.tiles_x[l] = (a.lv[l].W + kGradTile - 1) / kGradTile;
+      tiles += (long long)a.N * d.tiles_y[l] * d.tiles_x[l];
+    }
+  }
+  d.tile_start[D2B_MAX_LEVELS] = tiles;
+  D2B_REQUIRE(tiles < (1ll << 31), "too many destination tiles (%lld)", tiles);
+  roi_align_grad_bin_kernel<<<(unsigned)((M + kBinThreads - 1) / kBinThreads), kBinThreads, 0, st>>>(d);
+  D2B_LAUNCH_CHECK();
+  roi_align_grad_partition_kernel<<<(unsigned)(a.L * a.N), kPartThreads, 0, st>>>(d);
+  D2B_LAUNCH_CHECK();
+  const dim3 grid((unsigned)tiles, (unsigned)((a.C + kGradChannels - 1) / kGradChannels));
+  roi_align_grad_accum_kernel<<<grid, kGradThreads, 0, st>>>(d);
+  D2B_LAUNCH_CHECK();
+  return D2B_OK;
+}
+
+extern "C" int d2b_roi_align_backward(const d2b_roi_align_backward_params* p, void* workspace, size_t workspace_bytes,
+                                      d2b_stream_t stream) {
   D2B_REQUIRE(p != nullptr, "params is NULL");
   RoiAlignGradArgs g;
   const int rc = fill_args(&p->fwd, g.f, true);
@@ -519,6 +798,14 @@ extern "C" int d2b_roi_align_backward(const d2b_roi_align_backward_params* p, vo
   g.grad_out = p->grad_out;
   g.f.level_counts = nullptr;
   g.f.level_out = nullptr;
+  if (p->deterministic) {
+    const size_t need = d2b_roi_align_backward_workspace_bytes(p);
+    if (workspace == nullptr || workspace_bytes < need) {
+      set_last_error("deterministic roi_align_backward needs %zu workspace bytes", need);
+      return D2B_EWORKSPACE;
+    }
+    return launch_backward_deterministic(g, workspace, static_cast<cudaStream_t>(stream));
+  }
   const dim3 grid((unsigned)g.f.M, (unsigned)((g.f.oh * g.f.ow + kBinsPerCta - 1) / kBinsPerCta));
   roi_align_backward_kernel<<<grid, kThreads, 0, static_cast<cudaStream_t>(stream)>>>(g);
   D2B_LAUNCH_CHECK();

@@ -537,6 +537,7 @@ REGISTER_OP("D2RoiAlignMultilevelGrad")
     .Attr("scales: list(float)")
     .Attr("canonical_box_size: int = 224")
     .Attr("canonical_level: int = 4")
+    .Attr("deterministic: bool = false")  // true: no atomics, bit-identical to the CPU kernel (CropAndResizeGradImage)
     .Output("grad_features: L * float")
     .SetShapeFn([](InferenceContext* c) {
       int L;
@@ -554,6 +555,7 @@ class D2RoiAlignMultilevelGradOp : public tf::OpKernel {
     OP_REQUIRES_OK(c, c->GetAttr("scales", &scales_));
     OP_REQUIRES_OK(c, c->GetAttr("canonical_box_size", &cbs_));
     OP_REQUIRES_OK(c, c->GetAttr("canonical_level", &cl_));
+    OP_REQUIRES_OK(c, c->GetAttr("deterministic", &deterministic_));
     OP_REQUIRES(c, static_cast<int>(scales_.size()) == L_ && L_ <= D2B_MAX_LEVELS,
                 tf::errors::InvalidArgument("len(scales) must equal L <= ", D2B_MAX_LEVELS));
   }
@@ -589,12 +591,13 @@ class D2RoiAlignMultilevelGradOp : public tf::OpKernel {
     f.min_level = static_cast<int>(std::lround(-std::log2(scales_[0])));
     f.canonical_box_size = cbs_; f.canonical_level = cl_;
     p.grad_out = g.flat<float>().data();
+    p.deterministic = deterministic_ ? 1 : 0;
     RunOp(ctx, p, d2b_roi_align_backward_workspace_bytes, d2b_roi_align_backward);
   }
 
  private:
   int L_, sr_, cbs_, cl_;
-  bool aligned_;
+  bool aligned_, deterministic_;
   std::vector<float> scales_;
 };
 REGISTER_KERNEL_BUILDER(Name("D2RoiAlignMultilevelGrad").Device(tf::DEVICE_GPU), D2RoiAlignMultilevelGradOp);

@@ -109,11 +109,12 @@ def crop_and_resize(image, boxes, box_ind, crop_size, aligned=True, method='bili
 
 def _roi_align_backward_call(grad_out, feature_shapes, scales, boxes, batch_idx, sampling_ratio, aligned,
                              pad_border=True, min_level=0, canonical_box_size=224, canonical_level=4,
-                             grad_features=None):
+                             grad_features=None, deterministic=False):
     """Launcher of d2b_roi_align_backward: gradient of `_roi_align_call` w.r.t. every level's NHWC map.
 
     `feature_shapes`: list of (N, H, W, C).  `grad_features` (optional list of fp32 tensors) is accumulated
-    into; when None, zero-initialised tensors are created."""
+    into; when None, zero-initialised tensors are created.  `deterministic`: sum without floating-point atomics,
+    in the CPU kernel's order (bit-identical to it and from run to run); the default is the faster atomic scatter."""
     dev = nv.device_of(grad_out, boxes)
     host = not grad_out.is_cuda
     g = nv.to_device(grad_out, dev, torch.float32)
@@ -146,6 +147,7 @@ def _roi_align_backward_call(grad_out, feature_shapes, scales, boxes, batch_idx,
     f.min_level = int(min_level)
     f.canonical_box_size, f.canonical_level = int(canonical_box_size), int(canonical_level)
     p.grad_out = g.data_ptr()
+    p.deterministic = int(bool(deterministic))
     nv.call("roi_align_backward", p, dev)
     if host:
         return [nv.to_host(t) for t in grad_features]

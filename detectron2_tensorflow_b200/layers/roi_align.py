@@ -26,12 +26,14 @@ class ROIAlign(Layer):
         return _roi_align_call([inputs], [self.spatial_scale], boxes, box_inds, 1, self.output_size,
                                self.sampling_ratio, self.aligned, True)
 
-    def backward(self, grad_output, input_shape, boxes, box_inds, grad_input=None):
+    def backward(self, grad_output, input_shape, boxes, box_inds, grad_input=None, deterministic=False):
         """Gradient of `call` w.r.t. `inputs` (what TF autodiff runs in training; boxes get none,
-        functional.py:120).  grad_output [B, oh, ow, C] -> [N, H, W, C]; accumulates into `grad_input` if given."""
+        functional.py:120).  grad_output [B, oh, ow, C] -> [N, H, W, C]; accumulates into `grad_input` if given.
+        deterministic=True sums without atomics in the CPU kernel's order: bit-identical to it and reproducible."""
         grads = _roi_align_backward_call(grad_output, [input_shape], [self.spatial_scale], boxes, box_inds,
                                          self.sampling_ratio, self.aligned,
-                                         grad_features=None if grad_input is None else [grad_input])
+                                         grad_features=None if grad_input is None else [grad_input],
+                                         deterministic=deterministic)
         return grads[0]
 
     def __repr__(self):

@@ -100,11 +100,14 @@ class ROIPooler(Layer):
         self.last_level_counts = counts
         return out
 
-    def backward(self, grad_output, x_shapes, instances, grad_x=None):
+    def backward(self, grad_output, x_shapes, instances, grad_x=None, deterministic=False):
         """Gradient of `call` w.r.t. the feature maps `x` (list of (N,H,W,C) shapes) -> list of NHWC tensors.
-        One kernel: each ROI scatters into the level `assign_boxes_to_levels` gave it."""
+        Each ROI's gradient goes to the level `assign_boxes_to_levels` gave it.  Default: one kernel of atomic
+        scatters (fastest; the last bits depend on scheduling).  deterministic=True: no floating-point atomics, the
+        CPU kernel's summation order -- bit-identical to it and from run to run."""
         assert len(x_shapes) == len(self.level_poolers)
         return _roi_align_backward_call(grad_output, x_shapes, self.scales, instances.data.boxes,
                                         instances.indices[:, 0].contiguous(), self.sampling_ratio, self.aligned,
                                         min_level=self.min_level, canonical_box_size=self.canonical_box_size,
-                                        canonical_level=self.canonical_level, grad_features=grad_x)
+                                        canonical_level=self.canonical_level, grad_features=grad_x,
+                                        deterministic=deterministic)

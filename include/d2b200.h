@@ -501,16 +501,28 @@ D2B_API int d2b_matcher(const d2b_matcher_params* p, void* workspace, size_t wor
  * ROIPooler / ROIAlign backward: gradient w.r.t. the feature maps (what TF
  * autodiff runs in training for poolers.py:134-180: AvgPoolGrad ->
  * CropAndResizeGradImage -> MirrorPadGrad -> per-level scatter).  Boxes get no
- * gradient (functional.py:120 stop_gradient).  One kernel: vector fp32
- * reductions (red.global.add.v4.f32) into grad_features, which are ACCUMULATED
+ * gradient (functional.py:120 stop_gradient).  grad_features are ACCUMULATED
  * into (zero them first unless summing with another consumer's gradient).
- * Summation order differs from the CPU kernel's => fp32 tolerance, not bit parity.
  * `fwd` describes the forward call; its features/out/level_* fields are ignored.
+ *
+ * deterministic == 0: one kernel, vector fp32 reductions (red.global.add.v4.f32).
+ *   The order of the additions depends on scheduling => fp32 tolerance against
+ *   the CPU kernel, and two calls may differ in the last bits.  No workspace.
+ * deterministic != 0: no floating-point atomics; BIT-IDENTICAL to the CPU kernel
+ *   (TF CropAndResizeGradImage + MirrorPadGrad) and to itself from run to run.
+ *   Per level and image, a zeroed padded gradient receives, ROI by ROI in input
+ *   order, crop row by crop row, column by column, each sample's TL, TR, BL, BR
+ *   products; then every padded pixel is added onto clamp(p - pad) in raster
+ *   order.  Only pixels of 8x8 tiles that some ROI reaches are written, so a
+ *   -0.0 in grad_features elsewhere stays -0.0 (the CPU kernel adds +0.0).
+ *   Needs d2b_roi_align_backward_workspace_bytes() of scratch (per-ROI level,
+ *   footprint and sample taps, and the ROI lists of each level and image).
  * ---------------------------------------------------------------------- */
 typedef struct {
   d2b_roi_align_params fwd;
   const float* grad_out;                 /* [num_rois, output_h, output_w, channels] fp32 */
   float* grad_features[D2B_MAX_LEVELS];  /* level l: [num_images, height[l], width[l], channels] fp32 */
+  int32_t deterministic;                 /* 0: atomic scatter (fastest); 1: bit-exact, reproducible order */
 } d2b_roi_align_backward_params;
 D2B_API size_t d2b_roi_align_backward_workspace_bytes(const d2b_roi_align_backward_params* p);
 D2B_API int d2b_roi_align_backward(const d2b_roi_align_backward_params* p, void* workspace,
