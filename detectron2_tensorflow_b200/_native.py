@@ -90,7 +90,8 @@ class MatrixNmsParams(C.Structure):
 
 class PasteMasksParams(C.Structure):
     _fields_ = [("box_masks", _vp), ("boxes", _vp), ("num_masks", _i64), ("mask_h", _i32), ("mask_w", _i32),
-                ("image_h", _i32), ("image_w", _i32), ("mask_threshold", _f32), ("out", _vp)]
+                ("image_h", _i32), ("image_w", _i32), ("mask_threshold", _f32), ("out", _vp),
+                ("out_rle", _vp), ("rle_capacity", _i64), ("out_rle_offsets", _vp)]
 
 
 class CropAndResizeParams(C.Structure):
@@ -186,7 +187,8 @@ class SoloSelectParams(C.Structure):
 class SoloUpsampleParams(C.Structure):
     _fields_ = [("packed_masks", _vp), ("batch", _i32), ("num_dets", _i32), ("mask_h", _i32), ("mask_w", _i32),
                 ("image_h", _i32), ("image_w", _i32), ("align_corners", _i32), ("mask_threshold", _f32),
-                ("out_masks", _vp), ("out_packed_masks", _vp), ("out_boxes", _vp)]
+                ("out_masks", _vp), ("out_packed_masks", _vp), ("out_boxes", _vp),
+                ("out_rle", _vp), ("rle_capacity", _i64), ("out_rle_offsets", _vp)]
 
 
 class RoiAlignBackwardParams(C.Structure):

@@ -9,7 +9,10 @@
 // rectangle of each box -- the index range the inverse of the affine crop_and_resize map gives, widened
 // by 2 -- and applies the exact per-pixel rule there, storing the ones.  A one-pass kernel that computed
 // every pixel wrote 2.3-2.5 TB/s on a B200 against 7.3 TB/s for the memset.
+// With out_rle_offsets the same rule (paste_row / paste_on) feeds the COCO run-length encoder of mask_rle.cuh over
+// the same rectangles, and the planes are written only when `out` is given too.
 #include "kernels.cuh"
+#include "mask_rle.cuh"
 
 namespace d2b {
 namespace {
@@ -63,47 +66,104 @@ __device__ __forceinline__ void axis_range(const Axis& ax, int n, float max_in, 
   hi = min(n - 1, (int)ceilf(b) + 2);
 }
 
-__global__ void __launch_bounds__(kPasteThreads) paste_boxes_kernel(PasteArgs a) {
-  extern __shared__ float s_mask[];
-  const long long m = blockIdx.y;
+// Mask m's sampling axes and the rectangle [y0, y1] x [x0, x1] outside which every pasted pixel is 0.
+struct PasteBox {
+  Axis ay, ax;
+  float ymax_in, xmax_in;
+  int y0, y1, x0, x1;
+};
+__device__ __forceinline__ PasteBox paste_box(const PasteArgs& a, long long m) {
+  PasteBox g;
   const float4 bx = __ldg(reinterpret_cast<const float4*>(a.boxes) + m);
   // to_normalized_coordinates: scale by 1/height, 1/width (box_list_ops.py:829-839)
   const float ys = 1.0f / (float)a.H, xs = 1.0f / (float)a.W;
-  const Axis ay = make_axis(ys * bx.x, ys * bx.z, a.H, a.mh);
-  const Axis ax = make_axis(xs * bx.y, xs * bx.w, a.W, a.mw);
-  const float ymax_in = (float)(a.mh - 1), xmax_in = (float)(a.mw - 1);
-  int y0, y1, x0, x1;
-  axis_range(ay, a.H, ymax_in, y0, y1);
-  axis_range(ax, a.W, xmax_in, x0, x1);
-  if (y0 + (int)blockIdx.x > y1 || x0 > x1) return;  // block-uniform
+  g.ay = make_axis(ys * bx.x, ys * bx.z, a.H, a.mh);
+  g.ax = make_axis(xs * bx.y, xs * bx.w, a.W, a.mw);
+  g.ymax_in = (float)(a.mh - 1); g.xmax_in = (float)(a.mw - 1);
+  axis_range(g.ay, a.H, g.ymax_in, g.y0, g.y1);
+  axis_range(g.ax, a.W, g.xmax_in, g.x0, g.x1);
+  return g;
+}
+
+// The per-pixel rule, split at the row so the plane kernel hoists the row part out of its column loop.
+struct PasteRow {
+  int top, bot;
+  float ly;
+};
+// false: row y samples outside the box mask (extrapolation value 0)
+__device__ __forceinline__ bool paste_row(const PasteBox& g, int y, PasteRow& r) {
+  const float in_y = g.ay.at(y);
+  if (!(in_y >= 0.0f && in_y <= g.ymax_in)) return false;
+  const float fy = floorf(in_y);
+  r.top = (int)fy; r.bot = (int)ceilf(in_y);
+  r.ly = in_y - fy;
+  return true;
+}
+__device__ __forceinline__ bool paste_on(const float* mk, int mw, float thr, const PasteBox& g, const PasteRow& r, int x) {
+  const float in_x = g.ax.at(x);
+  if (!(in_x >= 0.0f && in_x <= g.xmax_in)) return false;
+  const float f = floorf(in_x);
+  const int left = (int)f, right = (int)ceilf(in_x);
+  const float lx = in_x - f;
+  const float tl = mk[r.top * mw + left], tr = mk[r.top * mw + right];
+  const float bl = mk[r.bot * mw + left], br = mk[r.bot * mw + right];
+  float t = tr - tl; t = t * lx; t = tl + t;
+  float bb = br - bl; bb = bb * lx; bb = bl + bb;
+  float v = bb - t; v = v * r.ly; v = t + v;
+  return v > thr;
+}
+
+__device__ __forceinline__ const float* stage_mask(const PasteArgs& a, long long m, float* s_mask, int nthreads) {
   const float* mk = a.masks + (size_t)m * a.mh * a.mw;
-  if (a.smem_mask) {
-    for (int i = threadIdx.x; i < a.mh * a.mw; i += kPasteThreads) s_mask[i] = __ldg(mk + i);
-    __syncthreads();
-    mk = s_mask;
-  }
+  if (!a.smem_mask) return mk;
+  for (int i = threadIdx.x; i < a.mh * a.mw; i += nthreads) s_mask[i] = __ldg(mk + i);
+  __syncthreads();
+  return s_mask;
+}
+
+__global__ void __launch_bounds__(kPasteThreads) paste_boxes_kernel(PasteArgs a) {
+  extern __shared__ float s_mask[];
+  const long long m = blockIdx.y;
+  const PasteBox g = paste_box(a, m);
+  if (g.y0 + (int)blockIdx.x > g.y1 || g.x0 > g.x1) return;  // block-uniform
+  const float* mk = stage_mask(a, m, s_mask, kPasteThreads);
   uint8_t* o = a.out + (size_t)m * ((size_t)a.H * a.W);
-  for (int y = y0 + (int)blockIdx.x; y <= y1; y += kRectCtas) {
-    const float in_y = ay.at(y);
-    if (!(in_y >= 0.0f && in_y <= ymax_in)) continue;
-    const float fy = floorf(in_y);
-    const int top = (int)fy, bot = (int)ceilf(in_y);
-    const float ly = in_y - fy;
-    for (int x = x0 + (int)threadIdx.x; x <= x1; x += kPasteThreads) {
-      const float in_x = ax.at(x);
-      if (in_x >= 0.0f && in_x <= xmax_in) {
-        const float f = floorf(in_x);
-        const int left = (int)f, right = (int)ceilf(in_x);
-        const float lx = in_x - f;
-        const float tl = mk[top * a.mw + left], tr = mk[top * a.mw + right];
-        const float bl = mk[bot * a.mw + left], br = mk[bot * a.mw + right];
-        float t = tr - tl; t = t * lx; t = tl + t;
-        float bb = br - bl; bb = bb * lx; bb = bl + bb;
-        float r = bb - t; r = r * ly; r = t + r;
-        if (r > a.thr) o[(size_t)y * a.W + x] = 1;
-      }
-    }
+  for (int y = g.y0 + (int)blockIdx.x; y <= g.y1; y += kRectCtas) {
+    PasteRow r;
+    if (!paste_row(g, y, r)) continue;
+    for (int x = g.x0 + (int)threadIdx.x; x <= g.x1; x += kPasteThreads)
+      if (paste_on(mk, a.mw, a.thr, g, r, x)) o[(size_t)y * a.W + x] = 1;
   }
+}
+
+struct PastePixel {
+  const float* mk;
+  int mw, y0, y1;
+  float thr;
+  PasteBox g;
+  __device__ __forceinline__ bool operator()(int y, int x) const {  // x is inside [g.x0, g.x1]
+    PasteRow r;
+    return y >= y0 && y <= y1 && paste_row(g, y, r) && paste_on(mk, mw, thr, g, r, x);
+  }
+};
+
+// One CTA per mask: count pass (kWrite = false) or write pass over the rectangle of paste_boxes_kernel.
+template <bool kWrite>
+__global__ void __launch_bounds__(kRleThreads) paste_rle_kernel(PasteArgs a, RleOut o) {
+  extern __shared__ float s_mask[];
+  __shared__ RleShared sh;
+  const long long m = blockIdx.x;
+  long long beg = 0, end = 0;
+  if (kWrite) {
+    beg = o.offsets[m]; end = o.offsets[m + 1];
+    if (end > o.capacity) return;  // block-uniform: this string does not fit
+  }
+  const PasteBox g = paste_box(a, m);
+  PastePixel px;
+  px.mk = stage_mask(a, m, s_mask, kRleThreads);
+  px.mw = a.mw; px.y0 = g.y0; px.y1 = g.y1; px.thr = a.thr; px.g = g;
+  rle_encode_mask<kWrite>(px, rle_walk_of(a.H, a.W, g.y0, g.y1, g.x0, g.x1), sh, o.offsets + m + 1, o.chars + beg,
+                          end - beg);
 }
 
 }  // namespace
@@ -111,6 +171,7 @@ __global__ void __launch_bounds__(kPasteThreads) paste_boxes_kernel(PasteArgs a)
 
 using namespace d2b;
 
+// The RLE byte lengths are staged in out_rle_offsets itself: no workspace either way.
 extern "C" size_t d2b_paste_masks_workspace_bytes(const d2b_paste_masks_params*) { return 0; }
 
 extern "C" int d2b_paste_masks(const d2b_paste_masks_params* p, void*, size_t, d2b_stream_t stream) {
@@ -119,24 +180,48 @@ extern "C" int d2b_paste_masks(const d2b_paste_masks_params* p, void*, size_t, d
               (long long)p->num_masks);
   D2B_REQUIRE(p->mask_h >= 1 && p->mask_w >= 1 && p->image_h >= 1 && p->image_w >= 1, "paste_masks: bad sizes");
   D2B_REQUIRE((long long)p->image_h * p->image_w < (1ll << 31) - 65536, "paste_masks: image too large");
-  if (p->num_masks == 0) return D2B_OK;  // mask_ops.py:25-28: zeros [0, H, W]
-  D2B_REQUIRE(p->box_masks && p->boxes && p->out, "paste_masks: NULL pointer");
+  const bool rle = p->out_rle_offsets != nullptr;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (rle) {
+    const int rc = rle_check("paste_masks", p->out_rle, p->rle_capacity);
+    if (rc != D2B_OK) return rc;
+  }
+  if (p->num_masks == 0) {  // mask_ops.py:25-28: zeros [0, H, W]
+    if (rle) D2B_CUDA(cudaMemsetAsync(p->out_rle_offsets, 0, sizeof(int64_t), st));
+    return D2B_OK;
+  }
+  D2B_REQUIRE(p->box_masks && p->boxes && (p->out || rle), "paste_masks: NULL pointer");
   PasteArgs a;
   a.masks = p->box_masks; a.boxes = p->boxes; a.mh = p->mask_h; a.mw = p->mask_w;
   a.H = p->image_h; a.W = p->image_w; a.thr = p->mask_threshold;
   const long long plane = (long long)a.H * a.W;
   a.smem_mask = (a.mh * a.mw <= kMaxMaskSmem);
   const size_t smem = a.smem_mask ? sizeof(float) * a.mh * a.mw : 0;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  D2B_CUDA(cudaMemsetAsync(p->out, 0, (size_t)p->num_masks * (size_t)plane, st));
-  if (smem > 48 * 1024)
-    D2B_CUDA(cudaFuncSetAttribute(paste_boxes_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  for (long long m0 = 0; m0 < p->num_masks; m0 += 65535) {  // grid.y limit
-    const long long cnt = p->num_masks - m0 < 65535 ? p->num_masks - m0 : 65535;
-    a.masks = p->box_masks + (size_t)m0 * a.mh * a.mw;
-    a.boxes = p->boxes + 4 * m0;
-    a.out = p->out + (size_t)m0 * plane;
-    paste_boxes_kernel<<<dim3(kRectCtas, (unsigned)cnt), kPasteThreads, smem, st>>>(a);
+  if (p->out) {
+    D2B_CUDA(cudaMemsetAsync(p->out, 0, (size_t)p->num_masks * (size_t)plane, st));
+    if (smem > 48 * 1024)
+      D2B_CUDA(cudaFuncSetAttribute(paste_boxes_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    for (long long m0 = 0; m0 < p->num_masks; m0 += 65535) {  // grid.y limit
+      const long long cnt = p->num_masks - m0 < 65535 ? p->num_masks - m0 : 65535;
+      PasteArgs c = a;
+      c.masks = p->box_masks + (size_t)m0 * a.mh * a.mw;
+      c.boxes = p->boxes + 4 * m0;
+      c.out = p->out + (size_t)m0 * plane;
+      paste_boxes_kernel<<<dim3(kRectCtas, (unsigned)cnt), kPasteThreads, smem, st>>>(c);
+      D2B_LAUNCH_CHECK();
+    }
+  }
+  if (rle) {
+    RleOut o;
+    o.chars = p->out_rle; o.offsets = p->out_rle_offsets; o.capacity = p->rle_capacity;
+    a.out = nullptr;
+    D2B_CUDA(allow_dynamic_smem(paste_rle_kernel<false>, smem));
+    D2B_CUDA(allow_dynamic_smem(paste_rle_kernel<true>, smem));
+    paste_rle_kernel<false><<<(unsigned)p->num_masks, kRleThreads, smem, st>>>(a, o);
+    D2B_LAUNCH_CHECK();
+    rle_offsets_kernel<<<1, kRleThreads, 0, st>>>(o.offsets, p->num_masks);
+    D2B_LAUNCH_CHECK();
+    paste_rle_kernel<true><<<(unsigned)p->num_masks, kRleThreads, smem, st>>>(a, o);
     D2B_LAUNCH_CHECK();
   }
   return D2B_OK;

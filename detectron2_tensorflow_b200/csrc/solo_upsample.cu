@@ -10,9 +10,13 @@
 //     warp and accumulated with 64-bit atomics; a finalise kernel applies the reference's mean / where rule.
 // TF ResizeBilinear arithmetic in the reference's op order (no FMA), both coordinate conventions the reference can
 // end up with (functional.py:21-35): half-pixel centres (tf.compat.v2.image.resize) and align_corners=True.
+// With out_rle_offsets the same per-pixel rule (resize_tap / up_lerp) feeds the COCO run-length encoder of
+// mask_rle.cuh (solo_rle_kernel) over the rectangle the taps of the set source pixels can reach.
+#include <limits.h>
 #include <math.h>
 
 #include "kernels.cuh"
+#include "mask_rle.cuh"
 
 namespace d2b {
 namespace {
@@ -54,6 +58,14 @@ __device__ __forceinline__ void resize_tap(int i, int in_size, float scale, int 
   lo = max((int)f, 0);
   hi = min((int)ceilf(src), in_size - 1);
   lerp = src - f;
+}
+
+// bilinear value of one output pixel from its four source pixels (the reference's op order)
+__device__ __forceinline__ float up_lerp(float tl, float tr, float bl, float br, float lx, float ly) {
+  float top = tr - tl; top = top * lx; top = tl + top;
+  float bot = br - bl; bot = bot * lx; bot = bl + bot;
+  float v = bot - top; v = v * ly; v = top + v;
+  return v;
 }
 
 __global__ void up_init_stats(Stats* s, int n) {
@@ -188,11 +200,7 @@ __global__ void __launch_bounds__(kUpThreads) solo_upsample_kernel(const UpArgs 
           //  masks 0.81 -> 1.23 ms, noise 4.2 -> 7.6 ms)
           const bool empty = shortcuts && (s0.y < lo || s0.x > hi) && (s1.y < lo || s1.x > hi);
           if (!empty) {
-            const float tl = q0[lo], tr = q0[hi], bl = q1[lo], br = q1[hi];
-            float top = tr - tl; top = top * t.lerp; top = tl + top;
-            float bot = br - bl; bot = bot * t.lerp; bot = bl + bot;
-            float v = bot - top; v = v * yl; v = top + v;
-            on = v > a.thr;
+            on = up_lerp(q0[lo], q0[hi], q1[lo], q1[hi], t.lerp, yl) > a.thr;
             if (on) {
               row_cnt += 1; sum_x32 += (unsigned)x;
               if (x > 0) { min_x = min(min_x, x); max_x = max(max_x, x); }
@@ -269,6 +277,99 @@ __global__ void up_boxes_kernel(const Stats* stats, int n, float* boxes) {
   boxes[i * 4 + 3] = fmaxf(xmax, xmean);
 }
 
+struct SoloPixel {
+  const u64* src;  // packed source mask
+  int h, w, align_corners;
+  float scale_y, scale_x, thr;
+  int y0, y1;
+  __device__ __forceinline__ float bit(int y, int x) const {
+    const long long q = (long long)y * w + x;
+    return ((src[q >> 6] >> (q & 63)) & 1ull) ? 1.0f : 0.0f;
+  }
+  __device__ __forceinline__ bool operator()(int y, int x) const {
+    if (y < y0 || y > y1) return false;
+    int ylo, yhi, xlo, xhi;
+    float ly, lx;
+    resize_tap(y, h, scale_y, align_corners, ylo, yhi, ly);
+    resize_tap(x, w, scale_x, align_corners, xlo, xhi, lx);
+    return up_lerp(bit(ylo, xlo), bit(ylo, xhi), bit(yhi, xlo), bit(yhi, xhi), lx, ly) > thr;
+  }
+};
+
+// CTA-wide min of lo and max of hi (every thread calls it)
+__device__ __forceinline__ void block_min_max(int& lo, int& hi, int* s) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    lo = min(lo, __shfl_xor_sync(0xffffffffu, lo, o));
+    hi = max(hi, __shfl_xor_sync(0xffffffffu, hi, o));
+  }
+  if (threadIdx.x == 0) { s[0] = INT_MAX; s[1] = INT_MIN; }
+  __syncthreads();
+  if ((threadIdx.x & 31) == 0) { atomicMin(&s[0], lo); atomicMax(&s[1], hi); }
+  __syncthreads();
+  lo = s[0]; hi = s[1];
+  __syncthreads();
+}
+
+// One CTA per (image, detection): count pass (kWrite = false) or write pass of the COCO RLE of its image mask.
+// For 0 <= thr < 1 a pixel whose four source pixels are 0 is off, so only output rows / columns whose taps reach the
+// set source rows / columns are walked; an empty source mask (padding rows) walks nothing and encodes [H*W].
+template <bool kWrite>
+__global__ void __launch_bounds__(kRleThreads) solo_rle_kernel(const UpArgs a, RleOut o, int stage_src) {
+  extern __shared__ u64 s_src[];
+  __shared__ RleShared sh;
+  __shared__ int s_mm[2];
+  const long long m = (long long)blockIdx.y * a.D + blockIdx.x;
+  long long beg = 0, end = 0;
+  if (kWrite) {
+    beg = o.offsets[m]; end = o.offsets[m + 1];
+    if (end > o.capacity) return;  // block-uniform: this string does not fit
+  }
+  SoloPixel px;
+  px.src = a.packed + m * a.Wd_in;
+  if (stage_src) {
+    for (int i = threadIdx.x; i < a.Wd_in; i += kRleThreads) s_src[i] = __ldg(px.src + i);
+    __syncthreads();
+    px.src = s_src;
+  }
+  px.h = a.h; px.w = a.w; px.align_corners = a.align_corners;
+  px.scale_y = a.scale_y; px.scale_x = a.scale_x; px.thr = a.thr;
+  int y0 = 0, y1 = a.H - 1, x0 = 0, x1 = a.W - 1;
+  if (a.thr >= 0.0f && a.thr < 1.0f) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    int r0 = INT_MAX, r1 = INT_MIN, c0 = INT_MAX, c1 = INT_MIN;  // set source rows / columns
+    for (int r = warp; r < a.h; r += kRleWarps) {
+      for (int x = lane; x < a.w; x += 32) {
+        if (px.bit(r, x) != 0.0f) {
+          r0 = min(r0, r); r1 = max(r1, r);
+          c0 = min(c0, x); c1 = max(c1, x);
+        }
+      }
+    }
+    block_min_max(r0, r1, s_mm);
+    block_min_max(c0, c1, s_mm);
+    y0 = INT_MAX; y1 = INT_MIN; x0 = INT_MAX; x1 = INT_MIN;
+    if (r1 >= 0) {
+      for (int y = threadIdx.x; y < a.H; y += kRleThreads) {
+        int lo, hi;
+        float l;
+        resize_tap(y, a.h, a.scale_y, a.align_corners, lo, hi, l);
+        if (hi >= r0 && lo <= r1) { y0 = min(y0, y); y1 = max(y1, y); }
+      }
+      for (int x = threadIdx.x; x < a.W; x += kRleThreads) {
+        int lo, hi;
+        float l;
+        resize_tap(x, a.w, a.scale_x, a.align_corners, lo, hi, l);
+        if (hi >= c0 && lo <= c1) { x0 = min(x0, x); x1 = max(x1, x); }
+      }
+    }
+    block_min_max(y0, y1, s_mm);
+    block_min_max(x0, x1, s_mm);
+  }
+  px.y0 = y0; px.y1 = y1;
+  rle_encode_mask<kWrite>(px, rle_walk_of(a.H, a.W, y0, y1, x0, x1), sh, o.offsets + m + 1, o.chars + beg, end - beg);
+}
+
 struct UpPlan {
   int iters, rows_cap;
   size_t smem;
@@ -318,14 +419,22 @@ extern "C" int d2b_solo_upsample(const d2b_solo_upsample_params* p, void* worksp
   int rc = up_plan(p, pl);
   if (rc != D2B_OK) return rc;
   const int n = p->batch * p->num_dets;
-  if (n == 0) return D2B_OK;
+  const bool rle = p->out_rle_offsets != nullptr;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (rle) {
+    rc = rle_check("solo_upsample", p->out_rle, p->rle_capacity);
+    if (rc != D2B_OK) return rc;
+  }
+  if (n == 0) {
+    if (rle) D2B_CUDA(cudaMemsetAsync(p->out_rle_offsets, 0, sizeof(int64_t), st));
+    return D2B_OK;
+  }
   D2B_REQUIRE(p->packed_masks && p->out_boxes, "solo_upsample: NULL pointer");
   const size_t need = ws_slice(sizeof(Stats) * (size_t)n);
   if (workspace == nullptr || workspace_bytes < need) {
     set_last_error("solo_upsample needs %zu workspace bytes", need);
     return D2B_EWORKSPACE;
   }
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
   UpArgs a;
   a.packed = reinterpret_cast<const u64*>(p->packed_masks);
   a.B = p->batch; a.D = p->num_dets; a.h = p->mask_h; a.w = p->mask_w; a.H = p->image_h; a.W = p->image_w;
@@ -351,5 +460,21 @@ extern "C" int d2b_solo_upsample(const d2b_solo_upsample_params* p, void* worksp
   D2B_LAUNCH_CHECK();
   up_boxes_kernel<<<(n + 255) / 256, 256, 0, st>>>(a.stats, n, p->out_boxes);
   D2B_LAUNCH_CHECK();
+  if (rle) {
+    RleOut o;
+    o.chars = p->out_rle; o.offsets = p->out_rle_offsets; o.capacity = p->rle_capacity;
+    const size_t src_bytes = sizeof(u64) * (size_t)a.Wd_in;
+    const int stage = src_bytes <= 64 * 1024;  // 200 x 336 source masks: 8.4 KB
+    const size_t smem = stage ? src_bytes : 0;
+    D2B_CUDA(allow_dynamic_smem(solo_rle_kernel<false>, smem));
+    D2B_CUDA(allow_dynamic_smem(solo_rle_kernel<true>, smem));
+    const dim3 g((unsigned)p->num_dets, (unsigned)p->batch);
+    solo_rle_kernel<false><<<g, kRleThreads, smem, st>>>(a, o, stage);
+    D2B_LAUNCH_CHECK();
+    rle_offsets_kernel<<<1, kRleThreads, 0, st>>>(o.offsets, n);
+    D2B_LAUNCH_CHECK();
+    solo_rle_kernel<true><<<g, kRleThreads, smem, st>>>(a, o, stage);
+    D2B_LAUNCH_CHECK();
+  }
   return D2B_OK;
 }

@@ -2,6 +2,7 @@
 import torch
 
 from ... import _native as nv
+from ...structures.mask_ops import rle_call
 
 __all__ = ["point_nms", "solo_mask_encode", "solo_dynamic_masks", "solo_upsample_masks", "SOLOv2Inference"]
 
@@ -90,7 +91,7 @@ def solo_dynamic_masks(mask_features, mask_kernels, mask_threshold=0.5, counts=N
 
 
 def solo_upsample_masks(packed_masks, mask_hw, image_shape, mask_threshold=0.5, align_corners=False, return_masks=True,
-                        return_packed=False):
+                        return_packed=False, return_rle=False, rle_capacity=None):
     """The last stage of `MaskKernelBranch.inference` (solo_v2.py:599-627): bilinear `resize_images` of the kept masks
     to `image_shape`, threshold, boxes from masks -- from the bit-packed masks of `SOLOv2Inference.postprocess`.
 
@@ -98,7 +99,10 @@ def solo_upsample_masks(packed_masks, mask_hw, image_shape, mask_threshold=0.5, 
     align_corners=False is what `resize_images` does when `tf.compat.v2.image.resize` exists (functional.py:21-24: the
     align_corners kwarg is dropped, half-pixel centres); True is the TF 1.13 fall-back (:26-35).
     Returns dict(pred_masks uint8 [B, D, H, W] or None, packed_masks int64 [B, D, ceil(H*W/64)] or None,
-    boxes fp32 [B, D, 4] as (ymin, xmin, ymax, xmax))."""
+    boxes fp32 [B, D, 4] as (ymin, xmin, ymax, xmax)).
+    return_rle=True adds rle = (chars uint8 [capacity], offsets int64 [B*D + 1]) on the device: the COCO run-length
+    strings of the B*D image masks, encoded on the GPU (see `structures.mask_ops.reframe_box_masks_to_rle` for
+    rle_capacity and `rle_to_coco`); return_masks=False then skips the [B, D, H, W] planes altogether."""
     host = not packed_masks.is_cuda
     dev = nv.device_of(packed_masks)
     pk = nv.to_device(packed_masks, dev, torch.int64)
@@ -116,10 +120,23 @@ def solo_upsample_masks(packed_masks, mask_hw, image_shape, mask_threshold=0.5, 
     p.align_corners = 1 if align_corners else 0
     p.mask_threshold = float(mask_threshold)
     p.out_masks, p.out_packed_masks, p.out_boxes = nv.ptr(masks), nv.ptr(packed), boxes.data_ptr()
-    nv.call("solo_upsample", p, dev)
-    out = dict(pred_masks=masks, packed_masks=packed, boxes=boxes)
+    if not return_rle:
+        nv.call("solo_upsample", p, dev)
+        out = dict(pred_masks=masks, packed_masks=packed, boxes=boxes)
+        if host:
+            out = {k: (None if v is None else nv.to_host(v)) for k, v in out.items()}
+        return out
+    spare_boxes = torch.empty_like(boxes) if rle_capacity is None else None
+
+    def run(chars, cap, offsets, again):
+        if again:  # the exactly sized call after the sizing call: the planes and boxes are already written
+            p.out_masks = p.out_packed_masks = None
+            p.out_boxes = spare_boxes.data_ptr()
+        p.out_rle, p.rle_capacity, p.out_rle_offsets = chars, cap, offsets
+        nv.call("solo_upsample", p, dev)
+    out = dict(pred_masks=masks, packed_masks=packed, boxes=boxes, rle=rle_call(run, B * D, dev, rle_capacity))
     if host:
-        out = {k: (None if v is None else nv.to_host(v)) for k, v in out.items()}
+        out = {k: (v if v is None or k == "rle" else nv.to_host(v)) for k, v in out.items()}
     return out
 
 

@@ -315,7 +315,16 @@ typedef struct {
   int32_t mask_h, mask_w;
   int32_t image_h, image_w;
   float mask_threshold;
-  uint8_t* out;
+  uint8_t* out; /* [M, image_h, image_w]; optional when out_rle_offsets is set */
+  /* Optional COCO run-length encoding of every mask, equal to
+   * pycocotools.mask.encode(np.asfortranarray(mask))["counts"] (column-major runs starting with zeros, deltas of
+   * counts 3.. against the count two before, 5-bit groups + 48; no terminator; COCO size [image_h, image_w]).
+   * out_rle_offsets[0] = 0 and out_rle_offsets[i+1] = out_rle_offsets[i] + length of string i, always complete.
+   * String i is written to out_rle + out_rle_offsets[i] iff out_rle_offsets[i+1] <= rle_capacity; nothing is written
+   * at or past rle_capacity, so a call with rle_capacity 0 is the sizing query.  The planes are never staged. */
+  uint8_t* out_rle;         /* optional [rle_capacity] bytes: the strings of all masks, back to back */
+  int64_t rle_capacity;     /* bytes available at out_rle (0 allowed) */
+  int64_t* out_rle_offsets; /* optional [num_masks + 1]; non-NULL requests RLE */
 } d2b_paste_masks_params;
 D2B_API size_t d2b_paste_masks_workspace_bytes(const d2b_paste_masks_params* p);
 D2B_API int d2b_paste_masks(const d2b_paste_masks_params* p, void* workspace, size_t workspace_bytes,
@@ -723,6 +732,11 @@ typedef struct {
   uint8_t* out_masks;         /* optional [B, D, image_h, image_w] {0,1} */
   uint64_t* out_packed_masks; /* optional [B, D, ceil(image_h*image_w/64)] */
   float* out_boxes;           /* [B, D, 4] (ymin, xmin, ymax, xmax) */
+  /* optional COCO RLE of the B*D image masks (rows past the valid count encode as [image_h * image_w]);
+   * same format and contract as d2b_paste_masks_params.out_rle */
+  uint8_t* out_rle;         /* optional [rle_capacity] bytes */
+  int64_t rle_capacity;     /* bytes available at out_rle (0 allowed) */
+  int64_t* out_rle_offsets; /* optional [B*D + 1]; non-NULL requests RLE */
 } d2b_solo_upsample_params;
 D2B_API size_t d2b_solo_upsample_workspace_bytes(const d2b_solo_upsample_params* p);
 D2B_API int d2b_solo_upsample(const d2b_solo_upsample_params* p, void* workspace, size_t workspace_bytes,
