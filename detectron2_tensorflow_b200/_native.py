@@ -91,7 +91,9 @@ class MatrixNmsParams(C.Structure):
 class PasteMasksParams(C.Structure):
     _fields_ = [("box_masks", _vp), ("boxes", _vp), ("num_masks", _i64), ("mask_h", _i32), ("mask_w", _i32),
                 ("image_h", _i32), ("image_w", _i32), ("mask_threshold", _f32), ("out", _vp),
-                ("out_rle", _vp), ("rle_capacity", _i64), ("out_rle_offsets", _vp)]
+                ("out_rle", _vp), ("rle_capacity", _i64), ("out_rle_offsets", _vp),
+                ("num_images", _i32), ("dets_per_image", _i32), ("output_shapes", _vp), ("input_shapes", _vp),
+                ("valid", _vp)]
 
 
 class CropAndResizeParams(C.Structure):

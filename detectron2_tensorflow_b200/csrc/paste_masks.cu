@@ -10,7 +10,9 @@
 // by 2 -- and applies the exact per-pixel rule there, storing the ones.  A one-pass kernel that computed
 // every pixel wrote 2.3-2.5 TB/s on a B200 against 7.3 TB/s for the memset.
 // With out_rle_offsets the same rule (paste_row / paste_on) feeds the COCO run-length encoder of mask_rle.cuh over
-// the same rectangles, and the planes are written only when `out` is given too.
+// the same rectangles, and the planes are written only when `out` is given too.  The batched mode (num_images > 0)
+// encodes the dense [N, R] detection slots of a whole batch, each image at its own output size, in the same three
+// launches.
 #include "kernels.cuh"
 #include "mask_rle.cuh"
 
@@ -72,17 +74,20 @@ struct PasteBox {
   float ymax_in, xmax_in;
   int y0, y1, x0, x1;
 };
-__device__ __forceinline__ PasteBox paste_box(const PasteArgs& a, long long m) {
+// Box bx (yxyx in output-image pixels) of an H x W output image.
+__device__ __forceinline__ PasteBox paste_box_at(const float4 bx, int H, int W, int mh, int mw) {
   PasteBox g;
-  const float4 bx = __ldg(reinterpret_cast<const float4*>(a.boxes) + m);
   // to_normalized_coordinates: scale by 1/height, 1/width (box_list_ops.py:829-839)
-  const float ys = 1.0f / (float)a.H, xs = 1.0f / (float)a.W;
-  g.ay = make_axis(ys * bx.x, ys * bx.z, a.H, a.mh);
-  g.ax = make_axis(xs * bx.y, xs * bx.w, a.W, a.mw);
-  g.ymax_in = (float)(a.mh - 1); g.xmax_in = (float)(a.mw - 1);
-  axis_range(g.ay, a.H, g.ymax_in, g.y0, g.y1);
-  axis_range(g.ax, a.W, g.xmax_in, g.x0, g.x1);
+  const float ys = 1.0f / (float)H, xs = 1.0f / (float)W;
+  g.ay = make_axis(ys * bx.x, ys * bx.z, H, mh);
+  g.ax = make_axis(xs * bx.y, xs * bx.w, W, mw);
+  g.ymax_in = (float)(mh - 1); g.xmax_in = (float)(mw - 1);
+  axis_range(g.ay, H, g.ymax_in, g.y0, g.y1);
+  axis_range(g.ax, W, g.xmax_in, g.x0, g.x1);
   return g;
+}
+__device__ __forceinline__ PasteBox paste_box(const PasteArgs& a, long long m) {
+  return paste_box_at(__ldg(reinterpret_cast<const float4*>(a.boxes) + m), a.H, a.W, a.mh, a.mw);
 }
 
 // The per-pixel rule, split at the row so the plane kernel hoists the row part out of its column loop.
@@ -147,23 +152,72 @@ struct PastePixel {
   }
 };
 
-// One CTA per mask: count pass (kWrite = false) or write pass over the rectangle of paste_boxes_kernel.
-template <bool kWrite>
-__global__ void __launch_bounds__(kRleThreads) paste_rle_kernel(PasteArgs a, RleOut o) {
+// Per-image geometry of the batched mode (d2b_paste_masks_params.num_images > 0): mask m is slot m % R of image m / R.
+struct PasteBatch {
+  const int32_t* out_shapes;  // [N, 2] (h, w)
+  const int32_t* in_shapes;   // [N, 2] (h, w) or NULL: boxes as they are
+  const uint8_t* valid;       // [N * R] or NULL
+  int R;
+};
+
+constexpr long long kMaxPlane = (1ll << 31) - 65536;  // H * W below this keeps every column-major position an int
+
+// Mask m's output size and pasting box in the batched mode; false: the slot encodes as an empty string.
+__device__ __forceinline__ bool batch_slot(const PasteArgs& a, const PasteBatch& bt, long long m, int& H, int& W,
+                                           float4& bx) {
+  const long long n = m / bt.R;
+  H = __ldg(bt.out_shapes + 2 * n);
+  W = __ldg(bt.out_shapes + 2 * n + 1);
+  if (!(H >= 1 && W >= 1 && (long long)H * W < kMaxPlane)) return false;
+  if (bt.valid && !__ldg(bt.valid + m)) return false;
+  bx = __ldg(reinterpret_cast<const float4*>(a.boxes) + m);
+  if (bt.in_shapes) {  // postprocessing.py:36-43: scales = float32(float64(out) / float64(image_shape)), then boxes * scales
+    const float sy = __double2float_rn(__ddiv_rn((double)H, (double)__ldg(bt.in_shapes + 2 * n)));
+    const float sx = __double2float_rn(__ddiv_rn((double)W, (double)__ldg(bt.in_shapes + 2 * n + 1)));
+    bx.x = __fmul_rn(sy, bx.x); bx.y = __fmul_rn(sx, bx.y);
+    bx.z = __fmul_rn(sy, bx.z); bx.w = __fmul_rn(sx, bx.w);
+  }
+  return true;
+}
+
+// One CTA per mask: count pass (kWrite = false) or write pass over the rectangle of paste_boxes_kernel.  kBatched takes
+// the output size, the box scale and the validity from the mask's image (PasteBatch) instead of from PasteArgs.
+template <bool kWrite, bool kBatched>
+__global__ void __launch_bounds__(kRleThreads) paste_rle_kernel(PasteArgs a, RleOut o, PasteBatch bt) {
   extern __shared__ float s_mask[];
   __shared__ RleShared sh;
   const long long m = blockIdx.x;
+  int H = a.H, W = a.W;
+  float4 bx;
+  if (kBatched && !batch_slot(a, bt, m, H, W, bx)) {  // block-uniform: an empty string
+    if (!kWrite && threadIdx.x == 0) o.offsets[m + 1] = 0;
+    return;
+  }
   long long beg = 0, end = 0;
   if (kWrite) {
     beg = o.offsets[m]; end = o.offsets[m + 1];
     if (end > o.capacity) return;  // block-uniform: this string does not fit
   }
-  const PasteBox g = paste_box(a, m);
+  const PasteBox g = kBatched ? paste_box_at(bx, H, W, a.mh, a.mw) : paste_box(a, m);
   PastePixel px;
   px.mk = stage_mask(a, m, s_mask, kRleThreads);
   px.mw = a.mw; px.y0 = g.y0; px.y1 = g.y1; px.thr = a.thr; px.g = g;
-  rle_encode_mask<kWrite>(px, rle_walk_of(a.H, a.W, g.y0, g.y1, g.x0, g.x1), sh, o.offsets + m + 1, o.chars + beg,
+  rle_encode_mask<kWrite>(px, rle_walk_of(H, W, g.y0, g.y1, g.x0, g.x1), sh, o.offsets + m + 1, o.chars + beg,
                           end - beg);
+}
+
+template <bool kBatched>
+int paste_rle(const PasteArgs& a, const RleOut& o, const PasteBatch& bt, long long num_masks, size_t smem,
+              cudaStream_t st) {
+  D2B_CUDA(allow_dynamic_smem(paste_rle_kernel<false, kBatched>, smem));
+  D2B_CUDA(allow_dynamic_smem(paste_rle_kernel<true, kBatched>, smem));
+  paste_rle_kernel<false, kBatched><<<(unsigned)num_masks, kRleThreads, smem, st>>>(a, o, bt);
+  D2B_LAUNCH_CHECK();
+  rle_offsets_kernel<<<1, kRleThreads, 0, st>>>(o.offsets, num_masks);
+  D2B_LAUNCH_CHECK();
+  paste_rle_kernel<true, kBatched><<<(unsigned)num_masks, kRleThreads, smem, st>>>(a, o, bt);
+  D2B_LAUNCH_CHECK();
+  return D2B_OK;
 }
 
 }  // namespace
@@ -178,8 +232,21 @@ extern "C" int d2b_paste_masks(const d2b_paste_masks_params* p, void*, size_t, d
   D2B_REQUIRE(p != nullptr, "params is NULL");
   D2B_REQUIRE(p->num_masks >= 0 && p->num_masks <= 65535ll * 16, "paste_masks: num_masks=%lld out of range",
               (long long)p->num_masks);
-  D2B_REQUIRE(p->mask_h >= 1 && p->mask_w >= 1 && p->image_h >= 1 && p->image_w >= 1, "paste_masks: bad sizes");
-  D2B_REQUIRE((long long)p->image_h * p->image_w < (1ll << 31) - 65536, "paste_masks: image too large");
+  const bool batched = p->num_images > 0;
+  if (batched) {  // every image's size lives in device memory: the kernels check it per mask
+    D2B_REQUIRE(p->dets_per_image >= 0 && (long long)p->num_images * p->dets_per_image == p->num_masks,
+                "paste_masks: num_masks=%lld is not num_images=%d x dets_per_image=%d", (long long)p->num_masks,
+                (int)p->num_images, (int)p->dets_per_image);
+    D2B_REQUIRE(p->out == nullptr && p->out_rle_offsets != nullptr,
+                "paste_masks: the batched mode (num_images > 0) writes RLE only: out must be NULL, out_rle_offsets set");
+    D2B_REQUIRE(p->output_shapes != nullptr, "paste_masks: num_images > 0 with output_shapes NULL");
+    D2B_REQUIRE(p->mask_h >= 1 && p->mask_w >= 1, "paste_masks: bad sizes");
+  } else {
+    D2B_REQUIRE(p->num_images == 0 && p->dets_per_image == 0 && !p->output_shapes && !p->input_shapes && !p->valid,
+                "paste_masks: num_images=%d: the batched fields need num_images > 0", (int)p->num_images);
+    D2B_REQUIRE(p->mask_h >= 1 && p->mask_w >= 1 && p->image_h >= 1 && p->image_w >= 1, "paste_masks: bad sizes");
+    D2B_REQUIRE((long long)p->image_h * p->image_w < kMaxPlane, "paste_masks: image too large");
+  }
   const bool rle = p->out_rle_offsets != nullptr;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (rle) {
@@ -215,14 +282,10 @@ extern "C" int d2b_paste_masks(const d2b_paste_masks_params* p, void*, size_t, d
     RleOut o;
     o.chars = p->out_rle; o.offsets = p->out_rle_offsets; o.capacity = p->rle_capacity;
     a.out = nullptr;
-    D2B_CUDA(allow_dynamic_smem(paste_rle_kernel<false>, smem));
-    D2B_CUDA(allow_dynamic_smem(paste_rle_kernel<true>, smem));
-    paste_rle_kernel<false><<<(unsigned)p->num_masks, kRleThreads, smem, st>>>(a, o);
-    D2B_LAUNCH_CHECK();
-    rle_offsets_kernel<<<1, kRleThreads, 0, st>>>(o.offsets, p->num_masks);
-    D2B_LAUNCH_CHECK();
-    paste_rle_kernel<true><<<(unsigned)p->num_masks, kRleThreads, smem, st>>>(a, o);
-    D2B_LAUNCH_CHECK();
+    PasteBatch bt;
+    bt.out_shapes = p->output_shapes; bt.in_shapes = p->input_shapes; bt.valid = p->valid; bt.R = p->dets_per_image;
+    return batched ? paste_rle<true>(a, o, bt, p->num_masks, smem, st)
+                   : paste_rle<false>(a, o, bt, p->num_masks, smem, st);
   }
   return D2B_OK;
 }

@@ -1,5 +1,6 @@
 """Drop-in for lib/structures/mask_ops.py: `reframe_box_masks_to_image_masks` (:7-56), plus the COCO run-length
-encoding of the pasted masks on the GPU (`reframe_box_masks_to_rle`, `rle_to_coco`)."""
+encoding of the pasted masks on the GPU (`reframe_box_masks_to_rle`, `rle_to_coco`; the batched, per-image-size
+encoding of a whole batch's detections is `modeling.detector_postprocess_rle`)."""
 import torch
 
 from .. import _native as nv
@@ -74,14 +75,24 @@ def reframe_box_masks_to_rle(box_masks, boxes, image_shape, mask_threshold=0.5, 
     return rle_call(run, m.shape[0], dev, capacity)
 
 
-def rle_to_coco(chars, offsets, image_shape):
-    """(chars, offsets) of `reframe_box_masks_to_rle` / `solo_upsample_masks(return_rle=True)` -> host list of
-    {"size": [H, W], "counts": bytes}, the per-mask object pycocotools.mask.encode returns."""
+def rle_to_coco(chars, offsets, image_shape=None, sizes=None):
+    """(chars, offsets) of `reframe_box_masks_to_rle` / `solo_upsample_masks(return_rle=True)` /
+    `detector_postprocess_rle` -> host list of {"size": [H, W], "counts": bytes}, the per-mask object
+    pycocotools.mask.encode returns.  `image_shape` (H, W) is every mask's size; `sizes` [M, 2] gives mask i its own
+    (h, w) instead, e.g. np.repeat(output_shapes, R, 0) for the [N, R] slots of `detector_postprocess_rle`.  An empty
+    string (a slot without a detection; every real mask encodes to at least one count) gives None."""
     off = offsets.cpu().tolist()
     need = int(off[-1])
     if need > chars.numel():
         raise ValueError(f"the RLE strings need {need} bytes but the buffer holds {chars.numel()}: "
                          f"call again with capacity >= {need}")
     data = chars[:need].cpu().numpy().tobytes()
-    size = [int(image_shape[0]), int(image_shape[1])]
-    return [{"size": size, "counts": data[off[i]:off[i + 1]]} for i in range(len(off) - 1)]
+    M = len(off) - 1
+    if sizes is None:
+        assert image_shape is not None, "rle_to_coco needs image_shape or sizes"
+        sizes = [[int(image_shape[0]), int(image_shape[1])]] * M
+    else:
+        sizes = torch.as_tensor(sizes).reshape(-1, 2).tolist()
+        assert len(sizes) == M, f"{len(sizes)} sizes for {M} strings"
+    return [{"size": [int(sizes[i][0]), int(sizes[i][1])], "counts": data[off[i]:off[i + 1]]} if off[i + 1] > off[i]
+            else None for i in range(M)]

@@ -325,6 +325,20 @@ typedef struct {
   uint8_t* out_rle;         /* optional [rle_capacity] bytes: the strings of all masks, back to back */
   int64_t rle_capacity;     /* bytes available at out_rle (0 allowed) */
   int64_t* out_rle_offsets; /* optional [num_masks + 1]; non-NULL requests RLE */
+  /* Batched mode (num_images > 0): the num_masks = num_images * dets_per_image masks are the dense [N, R] detection
+   * slots of detector_postprocess, image-major (mask m belongs to image m / R), and each image's masks are pasted and
+   * encoded at that image's own output size.  Only RLE is produced: `out` must be NULL and out_rle_offsets non-NULL;
+   * image_h / image_w are ignored.  The capacity contract is the one above.  With input_shapes set the boxes are
+   * scaled as detector_postprocess "fixed" does it (per axis scale = (float)((double)out / (double)in), then one fp32
+   * multiply per coordinate); NULL takes them as they are ("conventional").  A slot that is not valid, and every slot
+   * of an image whose output size has h < 1, w < 1 or h * w >= 2^31 - 65536, encodes as an empty string
+   * (offsets[m + 1] == offsets[m]); no pasted mask does, since an all-zero mask is one count.
+   * Left 0 / NULL, the op is the single-size one above. */
+  int32_t num_images;           /* N; 0 = single-size mode */
+  int32_t dets_per_image;       /* R */
+  const int32_t* output_shapes; /* [N, 2] (h, w) device: the size of image n's masks and of its RLE `size` */
+  const int32_t* input_shapes;  /* optional [N, 2] (h, w) device: the image_shape the boxes refer to */
+  const uint8_t* valid;         /* optional [N, R] device: 0 = no detection in this slot */
 } d2b_paste_masks_params;
 D2B_API size_t d2b_paste_masks_workspace_bytes(const d2b_paste_masks_params* p);
 D2B_API int d2b_paste_masks(const d2b_paste_masks_params* p, void* workspace, size_t workspace_bytes,
