@@ -176,6 +176,11 @@ struct FrcnnFetch {
     cls = (int)(ci / (unsigned)Rmax);
     roi = (int)(ci - (unsigned)cls * (unsigned)Rmax);
     const int i = slot_map[(size_t)n * Rmax + roi];
+    if (i < 0) {  // a slot no index row fills: the zero row of SparseBoxList.to_dense (score_thresh < 0 only)
+      box = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+      score = 0.0f;
+      return;
+    }
     const float h = (float)shapes[2 * n], w = (float)shapes[2 * n + 1];
     box = d2b_clip(boxes.get(i, Kb == 1 ? 0 : cls, Kb), h, w);
     score = __ldg(scores + (size_t)i * (K + 1) + cls);
@@ -366,8 +371,10 @@ struct YoloFetch {
 };
 
 // One warp per box, lanes stride the K class probabilities (coalesced); the (value, ~class) composite makes the
-// warp maximum pick the FIRST maximal class like tf.argmax.  Boxes above the threshold append a (score, index)
-// key to their image's candidate list; the segment sort restores (score desc, index asc).
+// warp maximum pick the FIRST maximal class like tf.argmax (+0 and -0 are equal).  NaN ranks above every number:
+// TF's Max reduction propagates NaN, so a row holding one has score_max NaN and fails `> thresh` (:352-355).
+// Boxes above the threshold append a (score, index) key to their image's candidate list; the segment sort
+// restores (score desc, index asc).
 __global__ void yolo_prep_kernel(const float* probs, int n, int K, float thresh, int P, u64* keys, int32_t* count,
                                  float* cand_score, int32_t* cand_cls) {
   const int img = blockIdx.y;
@@ -377,7 +384,8 @@ __global__ void yolo_prep_kernel(const float* probs, int n, int K, float thresh,
   const float* pr = probs + ((size_t)img * n + i) * K;
   u64 best = 0ull;
   for (int k = lane; k < K; k += 32) {
-    const u64 c = ((u64)float_to_key(__ldg(pr + k)) << 32) | (u64)(0xffffffffu - (unsigned)k);
+    const float v = __ldg(pr + k);
+    const u64 c = ((u64)(v != v ? 0xffffffffu : float_to_key(v)) << 32) | (u64)(0xffffffffu - (unsigned)k);
     best = c > best ? c : best;
   }
 #pragma unroll
@@ -483,6 +491,17 @@ __global__ void frcnn_prep_kernel(const FrcnnBoxes boxes, const float* scores, c
       if (slot < P) keys[(size_t)n * P + slot] = make_key(s, (unsigned)(k * Rmax + (int)r));
     }
   }
+}
+
+// score_thresh < 0 only, after frcnn_prep_kernel: a slot that no index row fills (slot_map still -1) is a row of
+// zeros in SparseBoxList.to_dense (box_list.py:204-246), so each of its K classes scores 0 > thresh with a zero box
+// and is a candidate like any other (fast_rcnn.py:119-136).  One thread per (image, slot).
+__global__ void frcnn_absent_kernel(const int32_t* slot_map, int N, int Rmax, int K, int P, u64* keys, int32_t* count) {
+  const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= (long long)N * Rmax || slot_map[t] >= 0) return;
+  const int n = (int)(t / Rmax), r = (int)(t - (long long)n * Rmax);
+  const int base = atomicAdd(count + n, K);
+  for (int k = 0; k < K && base + k < P; ++k) keys[(size_t)n * P + base + k] = make_key(0.0f, (unsigned)(k * Rmax + r));
 }
 
 // ------------------------------------------------------------------ RetinaNet front
@@ -756,12 +775,21 @@ extern "C" int d2b_fast_rcnn_postprocess(const d2b_fast_rcnn_params* p, void* wo
   if (nms_in) D2B_CUDA(cudaMemsetAsync(nms_in, 0, sizeof(u64), st));
   D2B_CUDA(cudaMemsetAsync(count, 0, sizeof(int32_t) * N, st));
   D2B_CUDA(cudaMemsetAsync(max_coord, 0, sizeof(float) * N, st));  // clipped coords are >= 0; padding rows are 0
+  // a negative threshold passes the zero scores of the slots no index row fills: mark every slot absent first
+  const bool absent_cands = p->score_thresh < 0.0f && p->rmax > 0;
+  if (absent_cands) D2B_CUDA(cudaMemsetAsync(slot_map, 0xff, sizeof(int32_t) * N * (size_t)p->rmax, st));
   const long long MK = p->num_preds * p->num_classes;
   if (MK > 0) {
     D2B_CUDA(launch_pdl(frcnn_prep_kernel, dim3((unsigned)((MK + 255) / 256)), dim3(256), 0, st, 0,
         fb, p->scores, reinterpret_cast<const long long*>(p->indices),
         p->num_preds, N, p->rmax, p->num_bbox_reg_classes, p->num_classes, p->image_shapes, p->score_thresh, pl.P,
         keys, count, slot_map, reinterpret_cast<int*>(max_coord)));
+    D2B_LAUNCH_CHECK();
+  }
+  if (absent_cands) {
+    const long long NR = (long long)N * p->rmax;
+    frcnn_absent_kernel<<<(unsigned)((NR + 255) / 256), 256, 0, st>>>(slot_map, N, p->rmax, p->num_classes, pl.P, keys,
+                                                                      count);
     D2B_LAUNCH_CHECK();
   }
   rc = sort_segments_desc(keys, N, pl.P, count, st);

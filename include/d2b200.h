@@ -214,6 +214,10 @@ D2B_API int d2b_rpn_proposals(const d2b_rpn_proposals_params* p, void* workspace
  * Fused decode (FastRCNNOutputs.inference, fast_rcnn.py:359-369, 381-395): with boxes == NULL the predicted boxes are
  * Box2BoxTransform.apply_deltas(deltas [M, Kb*4], proposal_boxes [M, 4]) (box_regression.py:76-123) evaluated where a
  * box is needed -- value-identical to d2b_apply_deltas followed by this call, without the [M, Kb*4] round trip.
+ * Index rows may come in any order.  A row with n outside [0, N) or slot outside [0, Rmax) is dropped.  The result
+ * is undefined when two rows name the same (image, slot).  As SparseBoxList.to_dense, a slot that no row fills is a
+ * row of zeros: with score_thresh < 0 each of its K classes is a candidate with score 0, a zero box and
+ * out_roi_index = the slot; with score_thresh >= 0 it never is.
  * ---------------------------------------------------------------------- */
 typedef struct {
   const float* boxes;
@@ -559,6 +563,8 @@ D2B_API int d2b_roi_align_backward(const d2b_roi_align_backward_params* p, void*
  * YOLOv4Outputs.inference    lib/modeling/single_stage_heads/yolov4_outputs.py:331-390
  * boxes [N, n, 4], probs [N, n, K] -> per image: max/argmax over classes, score
  * threshold, ONE class-agnostic NMS capped at post_nms_topk, zero-padded outputs.
+ * The class is the FIRST maximal one (+0 and -0 compare equal) and the score is its probability.  NaN: TF's
+ * reduce_max propagates it, so a box with a NaN probability in any class is never kept, whatever score_thresh.
  * ---------------------------------------------------------------------- */
 typedef struct {
   const float* boxes;

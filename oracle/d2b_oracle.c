@@ -1146,9 +1146,11 @@ ORC_API void orc_yolo_inference(const float* boxes, const float* probs, int N, i
     int64_t total = 0;
     for (int64_t i = 0; i < n; ++i) {
       const float* pr = probs + ((size_t)im * n + i) * K;
-      float mx = pr[0]; int64_t am = 0;
-      for (int k = 1; k < K; ++k) if (pr[k] > mx) { mx = pr[k]; am = k; }
-      if (!(mx > score_thresh)) continue;
+      /* reduce_max propagates NaN (TF's Max kernel reduces with Eigen::PropagateNaN): a row holding a NaN has
+       * score_max NaN and is never kept, whatever the threshold; argmax then only sees NaN-free rows */
+      float mx = pr[0]; int64_t am = 0; int has_nan = pr[0] != pr[0];
+      for (int k = 1; k < K; ++k) { if (pr[k] != pr[k]) has_nan = 1; else if (pr[k] > mx) { mx = pr[k]; am = k; } }
+      if (has_nan || !(mx > score_thresh)) continue;
       memcpy(cb + 4 * total, boxes + ((size_t)im * n + i) * 4, 16);
       cs[total] = mx; cc[total] = am; ++total;
     }
