@@ -190,7 +190,8 @@ class SoloUpsampleParams(C.Structure):
     _fields_ = [("packed_masks", _vp), ("batch", _i32), ("num_dets", _i32), ("mask_h", _i32), ("mask_w", _i32),
                 ("image_h", _i32), ("image_w", _i32), ("align_corners", _i32), ("mask_threshold", _f32),
                 ("out_masks", _vp), ("out_packed_masks", _vp), ("out_boxes", _vp),
-                ("out_rle", _vp), ("rle_capacity", _i64), ("out_rle_offsets", _vp)]
+                ("out_rle", _vp), ("rle_capacity", _i64), ("out_rle_offsets", _vp),
+                ("output_shapes", _vp), ("mask_shapes", _vp), ("valid", _vp)]
 
 
 class RoiAlignBackwardParams(C.Structure):

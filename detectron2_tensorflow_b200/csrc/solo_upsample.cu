@@ -11,7 +11,9 @@
 // TF ResizeBilinear arithmetic in the reference's op order (no FMA), both coordinate conventions the reference can
 // end up with (functional.py:21-35): half-pixel centres (tf.compat.v2.image.resize) and align_corners=True.
 // With out_rle_offsets the same per-pixel rule (resize_tap / up_lerp) feeds the COCO run-length encoder of
-// mask_rle.cuh (solo_rle_kernel) over the rectangle the taps of the set source pixels can reach.
+// mask_rle.cuh (solo_rle_kernel) over the rectangle the taps of the set source pixels can reach.  The batched mode
+// (output_shapes set) encodes each image's masks at that image's own output size, from the top-left crop of its masks
+// that the image covers, in the same three launches; its boxes come from the count pass's own pixel decisions.
 #include <limits.h>
 #include <math.h>
 
@@ -44,6 +46,11 @@ struct UpArgs {
   u64* out_packed;
   Stats* stats;
 };
+
+// The scale of one axis of a resize from in_size to out_size (TF ResizeBilinear's, fp32), host and device.
+__host__ __device__ __forceinline__ float resize_scale(int in_size, int out_size, int align_corners) {
+  return (align_corners && out_size > 1) ? (float)(in_size - 1) / (float)(out_size - 1) : (float)in_size / (float)out_size;
+}
 
 __device__ __forceinline__ void resize_tap(int i, int in_size, float scale, int align_corners, int& lo, int& hi, float& lerp) {
   float src;
@@ -263,27 +270,32 @@ __global__ void __launch_bounds__(kUpThreads) solo_upsample_kernel(const UpArgs 
 }
 
 // solo_v2.py:606-625: mean = sum / (count + 1e-5); where(yy > 0, yy, mean); min / max over all pixels
-__global__ void up_boxes_kernel(const Stats* stats, int n, float* boxes) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  const Stats s = stats[i];
+__device__ __forceinline__ float4 up_box(const Stats s) {  // (ymin, xmin, ymax, xmax)
   const float den = (float)s.count + 1e-5f;
   const float ymean = (float)s.sum_y / den, xmean = (float)s.sum_x / den;
   const float ymin = s.max_y >= 0 ? (float)s.min_y : INFINITY, ymax = s.max_y >= 0 ? (float)s.max_y : -INFINITY;
   const float xmin = s.max_x >= 0 ? (float)s.min_x : INFINITY, xmax = s.max_x >= 0 ? (float)s.max_x : -INFINITY;
-  boxes[i * 4 + 0] = fminf(ymin, ymean);
-  boxes[i * 4 + 1] = fminf(xmin, xmean);
-  boxes[i * 4 + 2] = fmaxf(ymax, ymean);
-  boxes[i * 4 + 3] = fmaxf(xmax, xmean);
+  return make_float4(fminf(ymin, ymean), fminf(xmin, xmean), fmaxf(ymax, ymean), fmaxf(xmax, xmean));
+}
+
+__global__ void up_boxes_kernel(const Stats* stats, int n, float* boxes) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const float4 bx = up_box(stats[i]);
+  boxes[i * 4 + 0] = bx.x;
+  boxes[i * 4 + 1] = bx.y;
+  boxes[i * 4 + 2] = bx.z;
+  boxes[i * 4 + 3] = bx.w;
 }
 
 struct SoloPixel {
   const u64* src;  // packed source mask
-  int h, w, align_corners;
+  int h, w, align_corners;  // taps read rows 0..h-1, columns 0..w-1
+  int stride;               // bits from one source row to the next (w, or mask_w for a crop)
   float scale_y, scale_x, thr;
   int y0, y1;
   __device__ __forceinline__ float bit(int y, int x) const {
-    const long long q = (long long)y * w + x;
+    const long long q = (long long)y * stride + x;
     return ((src[q >> 6] >> (q & 63)) & 1ull) ? 1.0f : 0.0f;
   }
   __device__ __forceinline__ bool operator()(int y, int x) const {
@@ -311,15 +323,92 @@ __device__ __forceinline__ void block_min_max(int& lo, int& hi, int* s) {
   __syncthreads();
 }
 
+// The count pass of the batched mode: the pixel rule of SoloPixel, plus the exact integer box statistics of the pixels
+// it sets.  Every pixel the walk visits is evaluated exactly once per pass, and a pixel it does not visit is off.
+struct SoloStatsPixel {
+  SoloPixel px;
+  mutable Stats st;  // this thread's share
+  __device__ __forceinline__ bool operator()(int y, int x) const {
+    const bool on = px(y, x);
+    if (on) {
+      st.count += 1; st.sum_y += (u64)y; st.sum_x += (u64)x;
+      if (y > 0) { st.min_y = min(st.min_y, y); st.max_y = max(st.max_y, y); }
+      if (x > 0) { st.min_x = min(st.min_x, x); st.max_x = max(st.max_x, x); }
+    }
+    return on;
+  }
+};
+
+// CTA-wide sum / min / max of every thread's statistics, returned to thread 0 (every thread calls it).
+__device__ __forceinline__ Stats block_stats(Stats s, Stats* sw) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    s.count += __shfl_xor_sync(0xffffffffu, s.count, o);
+    s.sum_y += __shfl_xor_sync(0xffffffffu, s.sum_y, o);
+    s.sum_x += __shfl_xor_sync(0xffffffffu, s.sum_x, o);
+    s.min_y = min(s.min_y, __shfl_xor_sync(0xffffffffu, s.min_y, o));
+    s.max_y = max(s.max_y, __shfl_xor_sync(0xffffffffu, s.max_y, o));
+    s.min_x = min(s.min_x, __shfl_xor_sync(0xffffffffu, s.min_x, o));
+    s.max_x = max(s.max_x, __shfl_xor_sync(0xffffffffu, s.max_x, o));
+  }
+  if ((threadIdx.x & 31) == 0) sw[threadIdx.x >> 5] = s;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    for (int q = 1; q < kRleWarps; ++q) {
+      const Stats t = sw[q];
+      s.count += t.count; s.sum_y += t.sum_y; s.sum_x += t.sum_x;
+      s.min_y = min(s.min_y, t.min_y); s.max_y = max(s.max_y, t.max_y);
+      s.min_x = min(s.min_x, t.min_x); s.max_x = max(s.max_x, t.max_x);
+    }
+  }
+  return s;
+}
+
+// Per-image geometry of the batched mode (d2b_solo_upsample_params.output_shapes set): CTA (d, b) is slot b * D + d.
+struct UpBatch {
+  const int32_t* out_shapes;   // [B, 2] (h, w)
+  const int32_t* mask_shapes;  // [B, 2] (h, w) or NULL: the whole mask
+  const uint8_t* valid;        // [B * D] or NULL
+  float* boxes;                // [B * D, 4]
+};
+
+constexpr long long kMaxPlane = (1ll << 31) - 65536;  // H * W below this keeps every column-major position an int
+
 // One CTA per (image, detection): count pass (kWrite = false) or write pass of the COCO RLE of its image mask.
 // For 0 <= thr < 1 a pixel whose four source pixels are 0 is off, so only output rows / columns whose taps reach the
 // set source rows / columns are walked; an empty source mask (padding rows) walks nothing and encodes [H*W].
-template <bool kWrite>
-__global__ void __launch_bounds__(kRleThreads) solo_rle_kernel(const UpArgs a, RleOut o, int stage_src) {
+// kBatched takes the output size, the crop and the validity from the slot's image (UpBatch), and the count pass also
+// writes the slot's box.
+template <bool kWrite, bool kBatched>
+__global__ void __launch_bounds__(kRleThreads) solo_rle_kernel(const UpArgs a, RleOut o, int stage_src, UpBatch bt) {
   extern __shared__ u64 s_src[];
   __shared__ RleShared sh;
   __shared__ int s_mm[2];
   const long long m = (long long)blockIdx.y * a.D + blockIdx.x;
+  int h = a.h, w = a.w, H = a.H, W = a.W;
+  float scale_y = a.scale_y, scale_x = a.scale_x;
+  if (kBatched) {
+    const int b = blockIdx.y;
+    D2B_BOUND(m, (long long)a.B * a.D);
+    D2B_BOUND(2 * b + 1, 2 * a.B);
+    H = __ldg(bt.out_shapes + 2 * b);
+    W = __ldg(bt.out_shapes + 2 * b + 1);
+    if (bt.mask_shapes) {
+      h = __ldg(bt.mask_shapes + 2 * b);
+      w = __ldg(bt.mask_shapes + 2 * b + 1);
+    }
+    const bool live = H >= 1 && W >= 1 && (long long)H * W < kMaxPlane && h >= 1 && h <= a.h && w >= 1 && w <= a.w &&
+                      (bt.valid == nullptr || __ldg(bt.valid + m) != 0);
+    if (!live) {  // block-uniform: an empty string and a zero box
+      if (!kWrite && threadIdx.x < 4) {
+        if (threadIdx.x == 0) o.offsets[m + 1] = 0;
+        bt.boxes[4 * m + threadIdx.x] = 0.0f;
+      }
+      return;
+    }
+    scale_y = resize_scale(h, H, a.align_corners);
+    scale_x = resize_scale(w, W, a.align_corners);
+  }
   long long beg = 0, end = 0;
   if (kWrite) {
     beg = o.offsets[m]; end = o.offsets[m + 1];
@@ -332,14 +421,14 @@ __global__ void __launch_bounds__(kRleThreads) solo_rle_kernel(const UpArgs a, R
     __syncthreads();
     px.src = s_src;
   }
-  px.h = a.h; px.w = a.w; px.align_corners = a.align_corners;
-  px.scale_y = a.scale_y; px.scale_x = a.scale_x; px.thr = a.thr;
-  int y0 = 0, y1 = a.H - 1, x0 = 0, x1 = a.W - 1;
+  px.h = h; px.w = w; px.stride = a.w; px.align_corners = a.align_corners;
+  px.scale_y = scale_y; px.scale_x = scale_x; px.thr = a.thr;
+  int y0 = 0, y1 = H - 1, x0 = 0, x1 = W - 1;
   if (a.thr >= 0.0f && a.thr < 1.0f) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     int r0 = INT_MAX, r1 = INT_MIN, c0 = INT_MAX, c1 = INT_MIN;  // set source rows / columns
-    for (int r = warp; r < a.h; r += kRleWarps) {
-      for (int x = lane; x < a.w; x += 32) {
+    for (int r = warp; r < h; r += kRleWarps) {
+      for (int x = lane; x < w; x += 32) {
         if (px.bit(r, x) != 0.0f) {
           r0 = min(r0, r); r1 = max(r1, r);
           c0 = min(c0, x); c1 = max(c1, x);
@@ -350,16 +439,16 @@ __global__ void __launch_bounds__(kRleThreads) solo_rle_kernel(const UpArgs a, R
     block_min_max(c0, c1, s_mm);
     y0 = INT_MAX; y1 = INT_MIN; x0 = INT_MAX; x1 = INT_MIN;
     if (r1 >= 0) {
-      for (int y = threadIdx.x; y < a.H; y += kRleThreads) {
+      for (int y = threadIdx.x; y < H; y += kRleThreads) {
         int lo, hi;
         float l;
-        resize_tap(y, a.h, a.scale_y, a.align_corners, lo, hi, l);
+        resize_tap(y, h, scale_y, a.align_corners, lo, hi, l);
         if (hi >= r0 && lo <= r1) { y0 = min(y0, y); y1 = max(y1, y); }
       }
-      for (int x = threadIdx.x; x < a.W; x += kRleThreads) {
+      for (int x = threadIdx.x; x < W; x += kRleThreads) {
         int lo, hi;
         float l;
-        resize_tap(x, a.w, a.scale_x, a.align_corners, lo, hi, l);
+        resize_tap(x, w, scale_x, a.align_corners, lo, hi, l);
         if (hi >= c0 && lo <= c1) { x0 = min(x0, x); x1 = max(x1, x); }
       }
     }
@@ -367,7 +456,39 @@ __global__ void __launch_bounds__(kRleThreads) solo_rle_kernel(const UpArgs a, R
     block_min_max(x0, x1, s_mm);
   }
   px.y0 = y0; px.y1 = y1;
-  rle_encode_mask<kWrite>(px, rle_walk_of(a.H, a.W, y0, y1, x0, x1), sh, o.offsets + m + 1, o.chars + beg, end - beg);
+  const RleWalk wk = rle_walk_of(H, W, y0, y1, x0, x1);
+  if constexpr (kBatched && !kWrite) {
+    __shared__ Stats s_st[kRleWarps];
+    SoloStatsPixel sp;
+    sp.px = px;
+    sp.st.count = sp.st.sum_y = sp.st.sum_x = 0ull;
+    sp.st.min_y = sp.st.min_x = 0x7fffffff;
+    sp.st.max_y = sp.st.max_x = -1;
+    rle_encode_mask<false>(sp, wk, sh, o.offsets + m + 1, o.chars, 0);
+    const Stats st = block_stats(sp.st, s_st);
+    D2B_BOUND(4 * m + 3, 4ll * a.B * a.D);
+    if (threadIdx.x == 0) {
+      const float4 bx = up_box(st);
+      float* box = bt.boxes + 4 * m;
+      box[0] = bx.x; box[1] = bx.y; box[2] = bx.z; box[3] = bx.w;
+    }
+  } else {
+    rle_encode_mask<kWrite>(px, wk, sh, o.offsets + m + 1, o.chars + beg, end - beg);
+  }
+}
+
+template <bool kBatched>
+int solo_rle(const UpArgs& a, const RleOut& o, const UpBatch& bt, int stage, size_t smem, cudaStream_t st) {
+  D2B_CUDA(allow_dynamic_smem(solo_rle_kernel<false, kBatched>, smem));
+  D2B_CUDA(allow_dynamic_smem(solo_rle_kernel<true, kBatched>, smem));
+  const dim3 g((unsigned)a.D, (unsigned)a.B);
+  solo_rle_kernel<false, kBatched><<<g, kRleThreads, smem, st>>>(a, o, stage, bt);
+  D2B_LAUNCH_CHECK();
+  rle_offsets_kernel<<<1, kRleThreads, 0, st>>>(o.offsets, (long long)a.B * a.D);
+  D2B_LAUNCH_CHECK();
+  solo_rle_kernel<true, kBatched><<<g, kRleThreads, smem, st>>>(a, o, stage, bt);
+  D2B_LAUNCH_CHECK();
+  return D2B_OK;
 }
 
 struct UpPlan {
@@ -379,12 +500,24 @@ int up_plan(const d2b_solo_upsample_params* p, UpPlan& pl) {
   D2B_REQUIRE(p != nullptr, "params is NULL");
   D2B_REQUIRE(p->batch >= 0 && p->num_dets >= 0, "solo_upsample: negative sizes");
   D2B_REQUIRE(p->batch <= 65535 && p->num_dets <= 65535, "solo_upsample: batch / num_dets too large");
+  if (p->output_shapes) {  // batched mode: every image's sizes live in device memory; the kernels check them per slot
+    D2B_REQUIRE(p->mask_h >= 1 && p->mask_w >= 1 && p->mask_w <= 65535 && p->mask_h <= 65535,
+                "solo_upsample: bad mask_h / mask_w");
+    D2B_REQUIRE(p->out_masks == nullptr && p->out_packed_masks == nullptr,
+                "solo_upsample: the batched mode (output_shapes set) writes RLE and boxes only: no planes");
+    D2B_REQUIRE(p->out_rle_offsets != nullptr && (p->out_boxes != nullptr || (long long)p->batch * p->num_dets == 0),
+                "solo_upsample: the batched mode (output_shapes set) needs out_rle_offsets and out_boxes");
+    pl = UpPlan{};
+    return D2B_OK;
+  }
+  D2B_REQUIRE(p->mask_shapes == nullptr && p->valid == nullptr,
+              "solo_upsample: mask_shapes / valid are batched-mode fields: they need output_shapes");
   D2B_REQUIRE(p->mask_h >= 1 && p->mask_w >= 1 && p->image_h >= 1 && p->image_w >= 1, "solo_upsample: empty mask / image");
   D2B_REQUIRE(p->mask_w <= 65535 && p->mask_h <= 65535 && (long long)p->image_h * p->image_w < (1ll << 31),
               "solo_upsample: sizes out of range");
   const int ac = p->align_corners != 0;
-  pl.scale_y = (ac && p->image_h > 1) ? (float)(p->mask_h - 1) / (float)(p->image_h - 1) : (float)p->mask_h / (float)p->image_h;
-  pl.scale_x = (ac && p->image_w > 1) ? (float)(p->mask_w - 1) / (float)(p->image_w - 1) : (float)p->mask_w / (float)p->image_w;
+  pl.scale_y = resize_scale(p->mask_h, p->image_h, ac);
+  pl.scale_x = resize_scale(p->mask_w, p->image_w, ac);
   for (int iters = 8; iters >= 1; iters >>= 1) {
     const long long chunk = (long long)iters * kUpThreads * kRun;
     const long long out_rows = chunk / p->image_w + 2;
@@ -409,7 +542,7 @@ using namespace d2b;
 
 extern "C" size_t d2b_solo_upsample_workspace_bytes(const d2b_solo_upsample_params* p) {
   UpPlan pl;
-  if (up_plan(p, pl) != D2B_OK) return 0;
+  if (up_plan(p, pl) != D2B_OK || p->output_shapes) return 0;  // the batched mode reduces its boxes inside the CTA
   return ws_slice(sizeof(Stats) * (size_t)p->batch * (p->num_dets > 0 ? p->num_dets : 1));
 }
 
@@ -430,6 +563,22 @@ extern "C" int d2b_solo_upsample(const d2b_solo_upsample_params* p, void* worksp
     return D2B_OK;
   }
   D2B_REQUIRE(p->packed_masks && p->out_boxes, "solo_upsample: NULL pointer");
+  const int Wd_in = (int)(((long long)p->mask_h * p->mask_w + 63) / 64);
+  const size_t src_bytes = sizeof(u64) * (size_t)Wd_in;
+  const int stage = src_bytes <= 64 * 1024;  // 200 x 336 source masks: 8.4 KB
+  const size_t rle_smem = stage ? src_bytes : 0;
+  if (p->output_shapes) {
+    UpArgs a = {};
+    a.packed = reinterpret_cast<const u64*>(p->packed_masks);
+    a.B = p->batch; a.D = p->num_dets; a.h = p->mask_h; a.w = p->mask_w; a.Wd_in = Wd_in;
+    a.align_corners = p->align_corners != 0;
+    a.thr = p->mask_threshold;
+    RleOut o;
+    o.chars = p->out_rle; o.offsets = p->out_rle_offsets; o.capacity = p->rle_capacity;
+    UpBatch bt;
+    bt.out_shapes = p->output_shapes; bt.mask_shapes = p->mask_shapes; bt.valid = p->valid; bt.boxes = p->out_boxes;
+    return solo_rle<true>(a, o, bt, stage, rle_smem, st);
+  }
   const size_t need = ws_slice(sizeof(Stats) * (size_t)n);
   if (workspace == nullptr || workspace_bytes < need) {
     set_last_error("solo_upsample needs %zu workspace bytes", need);
@@ -438,7 +587,7 @@ extern "C" int d2b_solo_upsample(const d2b_solo_upsample_params* p, void* worksp
   UpArgs a;
   a.packed = reinterpret_cast<const u64*>(p->packed_masks);
   a.B = p->batch; a.D = p->num_dets; a.h = p->mask_h; a.w = p->mask_w; a.H = p->image_h; a.W = p->image_w;
-  a.Wd_in = (int)(((long long)p->mask_h * p->mask_w + 63) / 64);
+  a.Wd_in = Wd_in;
   a.Wd_out = (int)(((long long)p->image_h * p->image_w + 63) / 64);
   a.align_corners = p->align_corners != 0;
   a.scale_y = pl.scale_y; a.scale_x = pl.scale_x; a.thr = p->mask_threshold;
@@ -463,18 +612,7 @@ extern "C" int d2b_solo_upsample(const d2b_solo_upsample_params* p, void* worksp
   if (rle) {
     RleOut o;
     o.chars = p->out_rle; o.offsets = p->out_rle_offsets; o.capacity = p->rle_capacity;
-    const size_t src_bytes = sizeof(u64) * (size_t)a.Wd_in;
-    const int stage = src_bytes <= 64 * 1024;  // 200 x 336 source masks: 8.4 KB
-    const size_t smem = stage ? src_bytes : 0;
-    D2B_CUDA(allow_dynamic_smem(solo_rle_kernel<false>, smem));
-    D2B_CUDA(allow_dynamic_smem(solo_rle_kernel<true>, smem));
-    const dim3 g((unsigned)p->num_dets, (unsigned)p->batch);
-    solo_rle_kernel<false><<<g, kRleThreads, smem, st>>>(a, o, stage);
-    D2B_LAUNCH_CHECK();
-    rle_offsets_kernel<<<1, kRleThreads, 0, st>>>(o.offsets, n);
-    D2B_LAUNCH_CHECK();
-    solo_rle_kernel<true><<<g, kRleThreads, smem, st>>>(a, o, stage);
-    D2B_LAUNCH_CHECK();
+    return solo_rle<false>(a, o, UpBatch{}, stage, rle_smem, st);
   }
   return D2B_OK;
 }

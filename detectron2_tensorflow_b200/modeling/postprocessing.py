@@ -7,9 +7,7 @@ import torch
 
 from .. import _native as nv
 from ..structures.box_list import SparseBoxList
-from ..structures.mask_ops import _paste_params, reframe_box_masks_to_image_masks, rle_call
-
-MAX_PLANE = (1 << 31) - 65536  # d2b_paste_masks: an output image must have h * w below this
+from ..structures.mask_ops import _output_shapes, _paste_params, reframe_box_masks_to_image_masks, rle_call
 
 
 def _scale_boxes(boxes, scales):
@@ -50,24 +48,6 @@ def detector_postprocess(results, output_shape, mask_format, image_shapes=None, 
     else:
         raise ValueError(f"mask format '{mask_format}' is not recognized.")
     return results
-
-
-def _output_shapes(output_shapes, N):
-    """The per-image output sizes as an int32 [N, 2] tensor.  Host sizes are checked here, before any device work; a
-    CUDA tensor (the form a CUDA graph replays with new sizes) is taken as it is, and the kernel gives an image whose
-    size is out of range empty strings."""
-    if isinstance(output_shapes, torch.Tensor) and output_shapes.is_cuda:
-        assert output_shapes.numel() == 2 * N, f"output_shapes has {output_shapes.numel()} values for {N} images"
-        return output_shapes.to(torch.int32).reshape(N, 2)
-    host = np.asarray(output_shapes.cpu() if isinstance(output_shapes, torch.Tensor) else output_shapes, np.int64)
-    if host.size != 2 * N:
-        raise ValueError(f"output_shapes has {host.size} values for {N} images")
-    host = host.reshape(N, 2)
-    bad = (host[:, 0] < 1) | (host[:, 1] < 1) | (host[:, 0] * host[:, 1] >= MAX_PLANE)
-    if bad.any():
-        n = int(np.flatnonzero(bad)[0])
-        raise ValueError(f"output_shapes[{n}] = {host[n].tolist()}: each side must be >= 1 and h * w < {MAX_PLANE}")
-    return torch.from_numpy(host.astype(np.int32))
 
 
 def detector_postprocess_rle(results, output_shapes, mask_threshold=0.5, mask_format="fixed", capacity=None):

@@ -2,9 +2,11 @@
 import torch
 
 from ... import _native as nv
-from ...structures.mask_ops import rle_call
+from ...structures.box_list import BoxList
+from ...structures.mask_ops import _output_shapes, rle_call
 
-__all__ = ["point_nms", "solo_mask_encode", "solo_dynamic_masks", "solo_upsample_masks", "SOLOv2Inference"]
+__all__ = ["point_nms", "solo_mask_encode", "solo_dynamic_masks", "solo_upsample_masks", "solo_upsample_rle",
+           "SOLOv2Inference"]
 
 
 def point_nms(inputs, kernel_size=2, scope=None):
@@ -140,6 +142,49 @@ def solo_upsample_masks(packed_masks, mask_hw, image_shape, mask_threshold=0.5, 
     return out
 
 
+def solo_upsample_rle(packed_masks, mask_hw, output_shapes, mask_shapes=None, valid=None, mask_threshold=0.5,
+                      align_corners=False, capacity=None):
+    """`solo_upsample_masks` for a whole batch at once, each image at its own output size, as COCO run-length strings
+    encoded on the GPU (d2b_solo_upsample in its batched mode); no image plane is written.
+
+    packed_masks int64 [B, D, ceil(h*w/64)], mask_hw = (h, w): the masks of `SOLOv2Inference.postprocess`, which cover
+    the padded canvas of the batch.  Slot (b, d) is `resize_images(masks[b, d, :hb, :wb], output_shapes[b])` thresholded,
+    with (hb, wb) = mask_shapes[b] (the top-left part of the canvas image b fills; None: the whole mask).
+    output_shapes / mask_shapes: [B, 2] (h, w) -- host sequences / arrays / tensors (checked here, before any device
+    work), or CUDA int32 tensors, taken as they are, which is how a CUDA graph is given sizes it can replay with.
+    valid: optional [B, D] (bool or uint8); a slot that is not valid has an empty string and a zero box.
+    capacity: None sizes the strings exactly (one host sync); an int issues no sync and can be captured in a CUDA graph
+    (the contract of `structures.mask_ops.reframe_box_masks_to_rle`).
+
+    Returns ((chars uint8 [capacity], offsets int64 [B * D + 1]), boxes fp32 [B, D, 4]): slot m = b * D + d is
+    chars[offsets[m]:offsets[m + 1]], byte-identical to pycocotools.mask.encode of its mask at output_shapes[b], and
+    boxes[b, d] is the box from that mask (solo_v2.py:606-625) in image b's output pixels."""
+    assert packed_masks.dim() == 3
+    B, D, Wd = packed_masks.shape
+    h, w = int(mask_hw[0]), int(mask_hw[1])
+    assert Wd == (h * w + 63) // 64
+    shapes = _output_shapes(output_shapes, B)
+    crops = None if mask_shapes is None else _output_shapes(mask_shapes, B, "mask_shapes", (h, w))
+    dev = nv.device_of(packed_masks, shapes, crops)
+    pk = nv.to_device(packed_masks, dev, torch.int64)
+    shapes = nv.to_device(shapes, dev)
+    crops = None if crops is None else nv.to_device(crops, dev)
+    ok = None if valid is None else nv.to_device(valid, dev, torch.uint8).reshape(B * D)
+    boxes = torch.empty((B, D, 4), dtype=torch.float32, device=dev)
+    p = nv.SoloUpsampleParams()
+    p.packed_masks = pk.data_ptr()
+    p.batch, p.num_dets, p.mask_h, p.mask_w = B, D, h, w
+    p.align_corners = 1 if align_corners else 0
+    p.mask_threshold = float(mask_threshold)
+    p.out_boxes = boxes.data_ptr()
+    p.output_shapes, p.mask_shapes, p.valid = shapes.data_ptr(), nv.ptr(crops), nv.ptr(ok)
+
+    def run(chars, cap, offsets, again):  # the sizing call and the exactly sized one write the same boxes
+        p.out_rle, p.rle_capacity, p.out_rle_offsets = chars, cap, offsets
+        nv.call("solo_upsample", p, dev)
+    return rle_call(run, B * D, dev, capacity), boxes
+
+
 class SOLOv2Inference(object):
     """The tail of `SOLOv2Head.inference` after the dynamic convolution (solo_v2.py:507-558), batched: mask stage,
     `sum_masks > strides` filter, mask scoring, top-k, Matrix-NMS on bit-packed masks, score filter, pad / clip.
@@ -161,6 +206,7 @@ class SOLOv2Inference(object):
         self.nms_sigma = nms_sigma
         self.update_score_threshold = update_score_threshold
         self.max_detections_per_image = max_detections_per_image
+        self._cell_strides = {}  # device -> [G] stride of each grid cell, kept so that select_candidates copies nothing
 
     def postprocess(self, mask_logits, scores, classes, strides, counts=None, return_masks=True, mask_features=None,
                     mask_kernels=None):
@@ -224,8 +270,11 @@ class SOLOv2Inference(object):
         B, G, K = sc.shape
         E = kn.shape[2]
         assert kn.shape[:2] == (B, G) and G == sum(g * g for g in self.num_grids)
-        cell = torch.cat([torch.full((g * g,), float(s_), dtype=torch.float32) for g, s_ in zip(self.num_grids, self.strides)])
-        cell = cell.to(dev)
+        cell = self._cell_strides.get(dev)
+        if cell is None:
+            cell = torch.cat([torch.full((g * g,), float(s_), dtype=torch.float32)
+                              for g, s_ in zip(self.num_grids, self.strides)]).to(dev)
+            self._cell_strides[dev] = cell
         n = self.max_candidates
         o_sc = torch.empty((B, n), dtype=torch.float32, device=dev)
         o_cl = torch.empty((B, n), dtype=torch.int64, device=dev)
@@ -250,6 +299,42 @@ class SOLOv2Inference(object):
         Returns dict(pred_classes int64 [B, D], pred_masks uint8 [B, D, H_img, W_img], scores [B, D], is_valid [B, D],
         boxes fp32 [B, D, 4], num [B], num_candidates [B])."""
         host = not pred_mask_features.is_cuda
+        feat, cand, tail = self._tail(pred_probs, pred_kernels, pred_mask_features)
+        up = solo_upsample_masks(tail["packed_masks"], feat.shape[1:3], image_shape, self.mask_threshold, self.align_corners)
+        out = dict(pred_classes=tail["pred_classes"], pred_masks=up["pred_masks"], scores=tail["scores"],
+                   is_valid=tail["is_valid"], boxes=up["boxes"], num=tail["num"], num_candidates=cand["total"])
+        if host:
+            out = {k: nv.to_host(v) for k, v in out.items()}
+        return out
+
+    def inference_rle(self, pred_probs, pred_kernels, pred_mask_features, output_shapes, mask_shapes=None,
+                      capacity=None):
+        """`inference` for COCO results: each image's masks at its own output size, as COCO run-length strings
+        (`solo_upsample_rle` on the masks of the tail, with `is_valid` as the slot validity).
+        output_shapes [B, 2]: each image's output size; mask_shapes [B, 2] or None: the top-left part of the mask
+        features that image b fills (ImageList pads bottom and right), e.g. ceil(image size in the canvas / 4).  Both
+        may be CUDA int32 tensors; with an int capacity the whole chain issues no host sync and can be captured in a
+        CUDA graph.
+        Returns (results, rle): results is a dense BoxList [B, D] with the boxes from the masks (in output pixels) and
+        `scores`, `pred_classes`, `is_valid`; rle = (chars, offsets) as `solo_upsample_rle` returns them.
+        `modeling.coco_results(results, rle, results.boxes, output_shapes, image_ids, category_ids)` makes the COCO
+        results list of the batch."""
+        B = pred_mask_features.shape[0]
+        hw = pred_mask_features.shape[1:3]
+        output_shapes = _output_shapes(output_shapes, B)  # host sizes are refused before any device work
+        if mask_shapes is not None:
+            mask_shapes = _output_shapes(mask_shapes, B, "mask_shapes", hw)
+        feat, _, tail = self._tail(pred_probs, pred_kernels, pred_mask_features)
+        rle, boxes = solo_upsample_rle(tail["packed_masks"], hw, output_shapes, mask_shapes, tail["is_valid"],
+                                       self.mask_threshold, self.align_corners, capacity)
+        results = BoxList(boxes)
+        results.add_field("scores", tail["scores"])
+        results.add_field("pred_classes", tail["pred_classes"])
+        results.add_field("is_valid", tail["is_valid"])
+        return results, rle
+
+    def _tail(self, pred_probs, pred_kernels, pred_mask_features):
+        """Candidate selection -> dynamic conv + mask stage -> tail, on the device: (features, candidates, tail)."""
         dev = nv.device_of(pred_mask_features)
         feat = nv.to_device(pred_mask_features, dev, torch.float32)
         B = feat.shape[0]
@@ -258,9 +343,4 @@ class SOLOv2Inference(object):
         cand = self.select_candidates(sc.contiguous(), kn.contiguous())
         tail = self.postprocess(None, cand["scores"], cand["classes"], cand["strides"], cand["counts"], return_masks=False,
                                 mask_features=feat, mask_kernels=cand["kernels"])
-        up = solo_upsample_masks(tail["packed_masks"], feat.shape[1:3], image_shape, self.mask_threshold, self.align_corners)
-        out = dict(pred_classes=tail["pred_classes"], pred_masks=up["pred_masks"], scores=tail["scores"],
-                   is_valid=tail["is_valid"], boxes=up["boxes"], num=tail["num"], num_candidates=cand["total"])
-        if host:
-            out = {k: nv.to_host(v) for k, v in out.items()}
-        return out
+        return feat, cand, tail

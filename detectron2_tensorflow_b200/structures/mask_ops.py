@@ -1,9 +1,12 @@
 """Drop-in for lib/structures/mask_ops.py: `reframe_box_masks_to_image_masks` (:7-56), plus the COCO run-length
 encoding of the pasted masks on the GPU (`reframe_box_masks_to_rle`, `rle_to_coco`; the batched, per-image-size
 encoding of a whole batch's detections is `modeling.detector_postprocess_rle`)."""
+import numpy as np
 import torch
 
 from .. import _native as nv
+
+MAX_PLANE = (1 << 31) - 65536  # the batched RLE modes: an output image must have h * w below this
 
 
 def reframe_box_masks_to_image_masks(box_masks, boxes, image_shape, mask_threshold=0.5, scope=None):
@@ -51,6 +54,28 @@ def rle_call(run, num_masks, device, capacity):
     chars = torch.empty(capacity, dtype=torch.uint8, device=device)
     run(chars.data_ptr() if capacity else None, capacity, offsets.data_ptr(), again)
     return chars, offsets
+
+
+def _output_shapes(shapes, N, name="output_shapes", max_hw=None):
+    """Per-image (h, w) sizes as an int32 [N, 2] tensor.  Host sizes are checked here, before any device work: each
+    side >= 1, h * w < MAX_PLANE and, with max_hw, h <= max_hw[0] and w <= max_hw[1].  A CUDA tensor (the form a CUDA
+    graph replays with new sizes) is taken as it is, and the kernel gives an image whose size is out of range empty
+    strings."""
+    if isinstance(shapes, torch.Tensor) and shapes.is_cuda:
+        assert shapes.numel() == 2 * N, f"{name} has {shapes.numel()} values for {N} images"
+        return shapes.to(torch.int32).reshape(N, 2)
+    host = np.asarray(shapes.cpu() if isinstance(shapes, torch.Tensor) else shapes, np.int64)
+    if host.size != 2 * N:
+        raise ValueError(f"{name} has {host.size} values for {N} images")
+    host = host.reshape(N, 2)
+    bad = (host[:, 0] < 1) | (host[:, 1] < 1) | (host[:, 0] * host[:, 1] >= MAX_PLANE)
+    if max_hw is not None:
+        bad |= (host[:, 0] > max_hw[0]) | (host[:, 1] > max_hw[1])
+    if bad.any():
+        n = int(np.flatnonzero(bad)[0])
+        limit = "" if max_hw is None else f", h <= {int(max_hw[0])}, w <= {int(max_hw[1])}"
+        raise ValueError(f"{name}[{n}] = {host[n].tolist()}: each side must be >= 1{limit} and h * w < {MAX_PLANE}")
+    return torch.from_numpy(host.astype(np.int32))
 
 
 def reframe_box_masks_to_rle(box_masks, boxes, image_shape, mask_threshold=0.5, capacity=None):

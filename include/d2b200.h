@@ -757,6 +757,20 @@ typedef struct {
   uint8_t* out_rle;         /* optional [rle_capacity] bytes */
   int64_t rle_capacity;     /* bytes available at out_rle (0 allowed) */
   int64_t* out_rle_offsets; /* optional [B*D + 1]; non-NULL requests RLE */
+  /* Batched mode (output_shapes non-NULL): slot m = b * D + d is the mask
+   *   resize_images(pred_masks[b, d, :hb, :wb], output_shapes[b]) > mask_threshold
+   * and its box from that mask, with the per-pixel and box rules above; (hb, wb) = mask_shapes[b], or (mask_h, mask_w)
+   * when mask_shapes is NULL (each image fills only the top-left part of the padded canvas the mask features cover).
+   * The resize scale of each axis is the single-size one with the crop as the input size.  Only RLE and boxes are
+   * produced: out_masks and out_packed_masks must be NULL, out_rle_offsets and out_boxes set; image_h / image_w are
+   * ignored and no workspace is needed.  The capacity contract is the one above, and string m's COCO `size` is
+   * output_shapes[b]; out_boxes[b, d] is in image b's output pixels.  A slot that is not valid, every slot of an image
+   * whose output size has h < 1, w < 1 or h * w >= 2^31 - 65536, and every slot of an image whose crop is outside
+   * [1, mask_h] x [1, mask_w], encodes as an empty string (offsets[m + 1] == offsets[m]) with box (0, 0, 0, 0); a
+   * valid slot is never empty, since an all-zero mask is one count.  Left NULL, the op is the single-size one above. */
+  const int32_t* output_shapes; /* [B, 2] (h, w) device; non-NULL selects the batched mode */
+  const int32_t* mask_shapes;   /* optional [B, 2] (h, w) device: the top-left region of image b's masks to resize */
+  const uint8_t* valid;         /* optional [B, D] device: 0 = no detection in this slot */
 } d2b_solo_upsample_params;
 D2B_API size_t d2b_solo_upsample_workspace_bytes(const d2b_solo_upsample_params* p);
 D2B_API int d2b_solo_upsample(const d2b_solo_upsample_params* p, void* workspace, size_t workspace_bytes,
